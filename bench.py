@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU forward (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's output as DIR/*.npy
 
 A step = one forward of the model over one batch of synthetic images (BASELINE.json configs[1]: ViT-B/16 augreg 224,
 197 tokens, GLOBAL batch 1024, random-init weights). With N GPUs the batch is sharded (1024 / N images per GPU,
@@ -161,6 +162,25 @@ def bind_to_gpu_numa_node(index: int) -> dict:
     return info
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, y: torch.Tensor, rank: int, world: int) -> None:
+    """Writes `y`, the forward's output in the last timed step, as float32 .npy. Weights and images are seeded, so the
+    same arguments give the same inputs on every run. Above 64 MB in all (e.g. the Whisper encoder's 64 x 1500 x 1280
+    tokens) a fixed, seeded subset of the samples is written, in batch order; the same subset on every run."""
+    import numpy as np
+
+    limit = DUMP_BYTES // world
+    keep = max(1, min(y.shape[0], limit // max(4 * y[0].numel(), 1)))
+    if keep < y.shape[0]:
+        idx = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        y = y[idx.to(y.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    name = "embeddings" if world == 1 else f"embeddings_rank{rank}"
+    np.save(os.path.join(out_dir, f"{name}.npy"), y.float().cpu().numpy())
+
+
 def committed_traffic(config: str, per_gpu_batch: int) -> dict | None:
     """DRAM bytes per launch (dram__bytes_read.sum + dram__bytes_write.sum) from the committed `ncu --set full`
     capture of this configuration: profiles/r02/ncu_traffic.json, written by scripts/ncu_summary.py from the .ncu-rep
@@ -257,7 +277,12 @@ def main() -> None:
                          "clocks of a cold GPU while the legs after them run power-capped")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output of the last one as DIR/embeddings.npy (float32; "
+                         "DIR/embeddings_rank<r>.npy per rank under torchrun) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference_arm(args, cfg)
@@ -353,6 +378,8 @@ def main() -> None:
             torch.cuda.profiler.stop()
         del xp
     ms_step, launches, clocks, y, x_dev = device_rate(B, steps, 1, True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y, rank, world)
     launches_per_step = launches // steps
     value = world * B / (ms_step * 1e-3)
 

@@ -285,3 +285,21 @@ def test_clock_sampler_windows_its_samples_to_the_timed_region():
     assert inside["window"] == "timed region" and inside["power_w_max"] == 950.0
     short = s.stop(3.0, 3.01)
     assert short["samples"] == 3 and short["window"].startswith("warm-up + timed region")
+
+
+def test_bench_dump_outputs_is_float32_bounded_and_seeded(tmp_path, monkeypatch):
+    """bench.dump_outputs: a small output is written whole as float32; a larger one is cut to the same seeded subset of
+    samples, in batch order, on every call, within the byte limit."""
+    import bench
+
+    y = torch.arange(6 * 3 * 4, dtype=torch.bfloat16).reshape(6, 3, 4)
+    bench.dump_outputs(str(tmp_path / "whole"), y, 0, 1)
+    got = np.load(tmp_path / "whole" / "embeddings.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, y.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * 3 * 4 * 4)  # room for two samples
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), y, 0, 1)
+    a, b = np.load(tmp_path / "a" / "embeddings.npy"), np.load(tmp_path / "b" / "embeddings.npy")
+    assert a.shape == (2, 3, 4) and np.array_equal(a, b)
+    rows = [int(r[0, 0]) // 12 for r in a]
+    assert rows == sorted(rows) and all(np.array_equal(r, y[i].float().numpy()) for r, i in zip(a, rows))
