@@ -1,17 +1,13 @@
 // C-ABI entry point for the attention core (see include/b200enc.h).
-#include <cstdlib>
-
 #include "../../include/b200enc.h"
-#include "attention.cuh"
 #include "attention_short.cuh"
-#include "attention_short_split.cuh"
-#include "attention_v6.cuh"
+#include "attention_stream.cuh"
 #include "host_util.h"
 
 using namespace b200;
 
 #ifdef ATT_TRACE
-// debug builds only (scripts/gpu_trace_attention.sh): event trace buffer of CTA 0, see ATT_EV in attention.cuh
+// debug builds only (make ../b200enc_trace): event trace buffer of CTA 0, see ATT_EV in attention_common.cuh
 static long long* g_attention_trace = nullptr;
 extern "C" void b200enc_debug_attention_trace(long long* buf) { g_attention_trace = buf; }
 #endif
@@ -21,6 +17,7 @@ namespace {
 template <typename Kern, typename Params>
 int launch_pdl(Kern kern, int grid, int threads, int smem, cudaStream_t s, const CUtensorMap& tq, const CUtensorMap& tk,
                const CUtensorMap& tv, const CUtensorMap& to, const Params& p) {
+  if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem)) return rc;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(threads);
@@ -34,114 +31,10 @@ int launch_pdl(Kern kern, int grid, int threads, int smem, cudaStream_t s, const
   B200_CUDA(cudaLaunchKernelEx(&cfg, kern, tq, tk, tv, to, p));
   return 0;
 }
-
-// The streaming kernel: attention_v6.cuh (separate P columns, scores issued a block ahead); the previous kernel
-// (attention.cuh) stays reachable with B200ENC_ATTN_V5=1 for same-box A/B runs and its self-tests.
-template <typename P>
-void fill_params(P& p, int B, int H, int Lq, int Lkv, float scale, void* out, long long out_batch_stride, int ldo, int flags,
-                 const float* bias, long long bias_b_stride, long long bias_h_stride, long long bias_row_stride,
-                 long long* trace) {
-  p.B = B;
-  p.H = H;
-  p.Lq = Lq;
-  p.Lkv = Lkv;
-  p.n_qp = (Lq + 2 * ATT_BQ - 1) / (2 * ATT_BQ);
-  p.n_items = B * H * p.n_qp;
-  p.scale_log2e = scale * 1.4426950408889634f;
-  p.out = reinterpret_cast<__nv_bfloat16*>(out);
-  p.out_batch_stride = out_batch_stride;
-  p.ldo = ldo;
-  p.causal = (flags & B200ENC_ATTN_CAUSAL) ? 1 : 0;
-  p.bias = bias;
-  p.bias_b_stride = bias_b_stride;
-  p.bias_h_stride = bias_h_stride;
-  p.bias_row_stride = bias_row_stride;
-  p.abort_word = abort_word();
-  p.debug_fault = (flags >> 16) & 1;  // selftest only (B200ENC_ATTN_DEBUG_FAULT)
-  p.trace = trace;
-}
-
-template <typename KernT, typename KernF, typename P>
-int launch_streaming(KernT kern_bias, KernF kern_plain, int threads, int smem, const CUtensorMap& tq, const CUtensorMap& tk,
-                     const CUtensorMap& tv, const CUtensorMap& to, const P& p, cudaStream_t s) {
-  const int grid = p.n_items < sm_count() ? p.n_items : sm_count();
-  if (p.bias != nullptr) {
-    if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern_bias), smem)) return rc;
-    return launch_pdl(kern_bias, grid, threads, smem, s, tq, tk, tv, to, p);
-  }
-  if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern_plain), smem)) return rc;
-  return launch_pdl(kern_plain, grid, threads, smem, s, tq, tk, tv, to, p);
-}
-
-bool use_v5() {
-  static const bool v = [] {
-    const char* e = getenv("B200ENC_ATTN_V5");
-    return e != nullptr && e[0] == '1';
-  }();
-  return v;
-}
 }  // namespace
 
-// Lkv <= 256, no mask: the single-pass kernel of attention_short.cuh. TMEM layout (see its header): private columns
-// for S and O where 512 columns allow it, otherwise O_t over the upper columns of S_t.
-static int attention_short_impl(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
-                                long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride, int ldo,
-                                int B, int H, int Lq, int Lkv, float scale, int flags, void* stream) {
-  AttnShortParams p;
-  p.nk16 = (Lkv + 15) & ~15;
-  CUtensorMap tq, tk, tv, to;
-  int rc;
-  const long long qbs = B > 1 ? q_batch_stride : (long long)Lq * ldq;
-  const long long kbs = B > 1 ? kv_batch_stride : (long long)Lkv * ldkv;
-  const long long obs = B > 1 ? out_batch_stride : (long long)Lq * ldo;
-  if ((rc = make_tmap_bf16(&tq, q, uint64_t(H) * ATT_HD, Lq, B, ldq, qbs, ATT_HD, ATT_BQ, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tk, k, uint64_t(H) * ATT_HD, Lkv, B, ldkv, kbs, ATT_HD, p.nk16, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tv, v, uint64_t(H) * ATT_HD, Lkv, B, ldkv, kbs, ATT_HD, p.nk16, 128))) return rc;
-  if ((rc = make_tmap_bf16(&to, out, uint64_t(H) * ATT_HD, Lq, B, ldo, obs, ATT_HD, 32, 128))) return rc;
-  p.B = B;
-  p.H = H;
-  p.Lq = Lq;
-  p.Lkv = Lkv;
-  p.n_qp = (Lq + 2 * ATT_BQ - 1) / (2 * ATT_BQ);
-  p.n_items = B * H * p.n_qp;
-  p.scale_log2e = scale * 1.4426950408889634f;
-  if (p.nk16 <= 176) {  // everything has its own columns: S_t 176 | O_t 64 | l_t 16
-    p.tm_s0 = 0, p.tm_o0 = 176, p.tm_l0 = 240, p.tm_s1 = 256, p.tm_o1 = 432, p.tm_l1 = 496, p.alias0 = p.alias1 = 0;
-  } else if (p.nk16 <= 208) {  // S0 208 | l0 16 | S1 208 | l1 16 | O0 64; O1 over the upper columns of S1
-    p.tm_s0 = 0, p.tm_l0 = 208, p.tm_s1 = 224, p.tm_l1 = 432, p.tm_o0 = 448, p.tm_o1 = 224 + 128, p.alias0 = 0, p.alias1 = 1;
-  } else if (p.nk16 <= 240) {  // both O_t over S_t; l_t behind the scores
-    p.tm_s0 = 0, p.tm_o0 = 128, p.tm_l0 = 240, p.tm_s1 = 256, p.tm_o1 = 256 + 128, p.tm_l1 = 496, p.alias0 = p.alias1 = 1;
-  } else {  // the scores fill all 256 columns of a tile: O_t and l_t both lie over them
-    p.tm_s0 = 0, p.tm_o0 = 128, p.tm_l0 = 192, p.tm_s1 = 256, p.tm_o1 = 256 + 128, p.tm_l1 = 256 + 192, p.alias0 = p.alias1 = 1;
-  }
-  p.abort_word = abort_word();
-  p.debug_fault = (flags >> 16) & 1;
-#ifdef ATT_TRACE
-  p.trace = g_attention_trace;
-#else
-  p.trace = nullptr;
-#endif
-  const int grid = p.n_items < sm_count() ? p.n_items : sm_count();
-  // the row length of ViT at 224 px (197 tokens -> 13 halves of 16 columns) has its own instantiation
-  // The two-threads-per-row instantiation for 197 keys (attention_short_split.cuh) is an experiment: correct (same
-  // self-tests) but 6 % slower than one thread per row at b = 1024 (0.269 vs 0.252 ms), so it only runs when asked for.
-  static const bool use_split = [] {
-    const char* e = getenv("B200ENC_ATTN_SPLIT");
-    return e != nullptr && e[0] == '1';
-  }();
-  if (Lkv == ASP_LKV && use_split) {
-    CUtensorMap to2;
-    if ((rc = make_tmap_bf16(&to2, out, uint64_t(H) * ATT_HD, Lq, B, ldo, obs, 32, 32, 64))) return rc;
-    p.tm_o1 = p.tm_s1 + 8 * ASP_A;  // the hole between the two pieces of P (attention_short_split.cuh)
-    if ((rc = ensure_dynamic_smem(reinterpret_cast<const void*>(attention_short197_kernel), ATS_SMEM_BYTES))) return rc;
-    return launch_pdl(attention_short197_kernel, grid, ASP_THREADS, ATS_SMEM_BYTES, reinterpret_cast<cudaStream_t>(stream), tq, tk,
-                      tv, to2, p);
-  }
-  auto kern = p.nk16 == 208 ? attention_short_kernel<13> : attention_short_kernel<0>;
-  if ((rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), ATS_SMEM_BYTES))) return rc;
-  return launch_pdl(kern, grid, ATT_THREADS, ATS_SMEM_BYTES, reinterpret_cast<cudaStream_t>(stream), tq, tk, tv, to, p);
-}
-
+// Two kernels: Lkv <= 256 without a mask runs the single-pass kernel of attention_short.cuh, everything else (longer
+// rows, causal, biased, or B200ENC_ATTN_GENERAL) the streaming kernel of attention_stream.cuh.
 static int attention_impl(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
                           long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride, int ldo, int B,
                           int H, int Lq, int Lkv, int head_dim, float scale, int flags, const float* bias,
@@ -155,36 +48,82 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
                  "b200enc_attention: leading dimension smaller than H*64");
   B200_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 15u) == 0 && ldo % 8 == 0 && out_batch_stride % 8 == 0,
                  "b200enc_attention: output rows must be 16-byte aligned");
-  CUtensorMap tq, tk, tv, to;
-  int rc;
-  if (Lkv <= ATS_MAX_KV && bias == nullptr && !(flags & (B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL)))
-    return attention_short_impl(q, q_batch_stride, ldq, k, v, kv_batch_stride, ldkv, out, out_batch_stride, ldo, B, H, Lq,
-                                Lkv, scale, flags, stream);
+  const bool short_kv = Lkv <= ATS_MAX_KV && bias == nullptr && !(flags & (B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL));
+  // K/V boxes: the whole row rounded up to 16 for the short kernel (N of its score MMA), 128-row blocks otherwise
+  const int nk16 = (Lkv + 15) & ~15;
+  const int kv_box = short_kv ? nk16 : ATT_BKV;
   const long long qbs = B > 1 ? q_batch_stride : (long long)Lq * ldq;
   const long long kbs = B > 1 ? kv_batch_stride : (long long)Lkv * ldkv;
-  if ((rc = make_tmap_bf16(&tq, q, uint64_t(H) * ATT_HD, Lq, B, ldq, qbs, ATT_HD, ATT_BQ, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tk, k, uint64_t(H) * ATT_HD, Lkv, B, ldkv, kbs, ATT_HD, ATT_BKV, 128))) return rc;
-  if ((rc = make_tmap_bf16(&tv, v, uint64_t(H) * ATT_HD, Lkv, B, ldkv, kbs, ATT_HD, ATT_BKV, 128))) return rc;
-  // output: one TMA store of 32 rows x 64 columns per softmax warp; rows >= Lq of a batch are clipped by the map
   const long long obs = B > 1 ? out_batch_stride : (long long)Lq * ldo;
+  CUtensorMap tq, tk, tv, to;
+  int rc;
+  if ((rc = make_tmap_bf16(&tq, q, uint64_t(H) * ATT_HD, Lq, B, ldq, qbs, ATT_HD, ATT_BQ, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tk, k, uint64_t(H) * ATT_HD, Lkv, B, ldkv, kbs, ATT_HD, kv_box, 128))) return rc;
+  if ((rc = make_tmap_bf16(&tv, v, uint64_t(H) * ATT_HD, Lkv, B, ldkv, kbs, ATT_HD, kv_box, 128))) return rc;
+  // output: one TMA store of 32 rows x 64 columns per softmax warp; rows >= Lq of a batch are clipped by the map
   if ((rc = make_tmap_bf16(&to, out, uint64_t(H) * ATT_HD, Lq, B, ldo, obs, ATT_HD, 32, 128))) return rc;
+  const int n_qp = (Lq + 2 * ATT_BQ - 1) / (2 * ATT_BQ);
+  const int n_items = B * H * n_qp;
+  const int grid = n_items < sm_count() ? n_items : sm_count();
+  const float scale_log2e = scale * 1.4426950408889634f;
+  const int debug_fault = (flags >> 16) & 1;  // selftest only (B200ENC_ATTN_DEBUG_FAULT)
 #ifdef ATT_TRACE
   long long* const trace = g_attention_trace;
 #else
   long long* const trace = nullptr;
 #endif
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  if (use_v5()) {
-    AttnParams p;
-    fill_params(p, B, H, Lq, Lkv, scale, out, out_batch_stride, ldo, flags, bias, bias_b_stride, bias_h_stride,
-                bias_row_stride, trace);
-    return launch_streaming(attention_kernel<true>, attention_kernel<false>, ATT_THREADS, ATT_SMEM_BYTES, tq, tk, tv, to, p, s);
+
+  if (short_kv) {
+    AttnShortParams p;
+    p.B = B;
+    p.H = H;
+    p.Lq = Lq;
+    p.Lkv = Lkv;
+    p.nk16 = nk16;
+    p.n_qp = n_qp;
+    p.n_items = n_items;
+    p.scale_log2e = scale_log2e;
+    // TMEM layout (see attention_short.cuh): private columns for S and O where 512 columns allow it, otherwise O_t
+    // over the upper columns of S_t
+    if (nk16 <= 176) {  // everything has its own columns: S_t 176 | O_t 64 | l_t 16
+      p.tm_s0 = 0, p.tm_o0 = 176, p.tm_l0 = 240, p.tm_s1 = 256, p.tm_o1 = 432, p.tm_l1 = 496, p.alias0 = p.alias1 = 0;
+    } else if (nk16 <= 208) {  // S0 208 | l0 16 | S1 208 | l1 16 | O0 64; O1 over the upper columns of S1
+      p.tm_s0 = 0, p.tm_l0 = 208, p.tm_s1 = 224, p.tm_l1 = 432, p.tm_o0 = 448, p.tm_o1 = 224 + 128, p.alias0 = 0, p.alias1 = 1;
+    } else if (nk16 <= 240) {  // both O_t over S_t; l_t behind the scores
+      p.tm_s0 = 0, p.tm_o0 = 128, p.tm_l0 = 240, p.tm_s1 = 256, p.tm_o1 = 256 + 128, p.tm_l1 = 496, p.alias0 = p.alias1 = 1;
+    } else {  // the scores fill all 256 columns of a tile: O_t and l_t both lie over them
+      p.tm_s0 = 0, p.tm_o0 = 128, p.tm_l0 = 192, p.tm_s1 = 256, p.tm_o1 = 256 + 128, p.tm_l1 = 256 + 192, p.alias0 = p.alias1 = 1;
+    }
+    p.abort_word = abort_word();
+    p.debug_fault = debug_fault;
+    p.trace = trace;
+    // the row length of ViT at 224 px (197 tokens -> 13 halves of 16 columns) has its own instantiation
+    const auto kern = nk16 == 208 ? attention_short_kernel<13> : attention_short_kernel<0>;
+    return launch_pdl(kern, grid, ATT_THREADS, ATS_SMEM_BYTES, s, tq, tk, tv, to, p);
   }
-  v6::AttnParams p;
-  fill_params(p, B, H, Lq, Lkv, scale, out, out_batch_stride, ldo, flags, bias, bias_b_stride, bias_h_stride,
-              bias_row_stride, trace);
-  return launch_streaming(v6::attention_kernel<true>, v6::attention_kernel<false>, v6::ATT_THREADS, v6::ATT_SMEM_BYTES, tq,
-                          tk, tv, to, p, s);
+
+  AttnParams p;
+  p.B = B;
+  p.H = H;
+  p.Lq = Lq;
+  p.Lkv = Lkv;
+  p.n_qp = n_qp;
+  p.n_items = n_items;
+  p.scale_log2e = scale_log2e;
+  p.out = reinterpret_cast<__nv_bfloat16*>(out);
+  p.out_batch_stride = out_batch_stride;
+  p.ldo = ldo;
+  p.causal = (flags & B200ENC_ATTN_CAUSAL) ? 1 : 0;
+  p.bias = bias;
+  p.bias_b_stride = bias_b_stride;
+  p.bias_h_stride = bias_h_stride;
+  p.bias_row_stride = bias_row_stride;
+  p.abort_word = abort_word();
+  p.debug_fault = debug_fault;
+  p.trace = trace;
+  const auto kern = bias != nullptr ? attention_kernel<true> : attention_kernel<false>;
+  return launch_pdl(kern, grid, ATT_THREADS, ATT_SMEM_BYTES, s, tq, tk, tv, to, p);
 }
 
 extern "C" int b200enc_attention(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,

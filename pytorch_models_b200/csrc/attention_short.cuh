@@ -1,7 +1,7 @@
 // Attention for SHORT key/value sequences (Lkv <= 256, head_dim 64, no mask) on sm_100a: the whole score row of a
 // query fits in tensor memory, so the softmax is exact and single-pass (reference: F.scaled_dot_product_attention at
 // pytorch_models/transformer.py:52 with attn_mask=None, is_causal=False — ViT-B/16 at 224 px has 197 tokens, the
-// configuration the headline metric is quoted on; longer, causal or biased calls use attention.cuh).
+// configuration the headline metric is quoted on; longer, causal or biased calls use attention_stream.cuh).
 //
 // Why a second kernel: with two 128-key blocks per item the general kernel pays its per-block fixed costs (barrier
 // round trips S_FULL -> P_FULL -> O_FULL, the rescale bookkeeping of the online softmax, an item boundary every
@@ -12,7 +12,7 @@
 //   warp 1      : tcgen05.mma issuer:  S_t = Q_t K^T  as ONE group of 4 MMAs with N = nk16 (up to 256 columns of
 //                 TMEM), O_t = P_t V as nk16/16 MMAs with P as the TMEM A operand. Order per item:
 //                 PV0(n) QK0(n+1) PV1(n) QK1(n+1)
-//   warp 2      : watchdog (same contract as attention.cuh: no unbounded wait can hang the GPU)
+//   warp 2      : watchdog (attention_common.cuh: no unbounded wait can hang the GPU)
 //   warps 4..7  : softmax of tile 0, warps 8..11 of tile 1; one thread per query row. Pass 1 streams the row out of
 //                 TMEM in 32-column chunks for the exact maximum (FMNMX3), pass 2 streams it again, takes the
 //                 exponentials and writes P back over S as packed bf16 (chunk c of P lands on columns of S that
@@ -24,20 +24,12 @@
 // complete, and QK1(n+1) waits (T_FREE) until the epilogue has pulled O1(n) into registers. Above 224 both tiles
 // alias. The host picks the layout (api_attention.cu).
 // The normalised output leaves through one TMA store per warp, Q/K/V are read straight out of the fused QKV
-// activation through strided tensor maps — as in attention.cuh.
+// activation through strided tensor maps (attention_common.cuh). Every role waits with mbar_wait_parked: a waiting
+// warp issues almost nothing and leaves its sub-partition's issue slots to the warps that compute.
 #pragma once
-#include "attention.cuh"
+#include "attention_common.cuh"
 
 namespace b200 {
-
-#ifndef ATS_PARKED_WAITS
-#define ATS_PARKED_WAITS 1
-#endif
-#if ATS_PARKED_WAITS
-#define ATS_WAIT(bar, parity) mbar_wait_parked(bar, parity)
-#else
-#define ATS_WAIT(bar, parity) mbar_wait_plain(bar, parity)
-#endif
 
 constexpr int ATS_MAX_KV = 256;
 constexpr int ATS_KV_BYTES = ATS_MAX_KV * 128;                         // 32 KB: up to 256 rows x 64 bf16
@@ -62,15 +54,6 @@ struct AttnShortParams {
   int debug_fault;
   long long* trace;
 };
-
-#ifndef ATS_FUSED_ISSUE
-#define ATS_FUSED_ISSUE 0  // 1: P.V(n) + row sums + Q.K(n+1) of tile 0 as one run behind the P_FULL wait (measured 6 % SLOWER at L = 197: 0.267 vs 0.251 ms)
-#endif
-__device__ __forceinline__ float fmax3(float a, float b, float c) {
-  float d;
-  asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
-  return d;
-}
 
 // kNH: number of 16-column halves of the score row (nk16 / 16) as a compile-time constant, 0 = read it from the
 // parameters. With a constant every chunk guard folds away: no taken branches over skipped code (ncu: `no_inst`
@@ -144,7 +127,7 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       const int b = bh / p.H;
       const bool two = two_of(item);
       const uint32_t s = uint32_t(n) & 1u;
-      ATS_WAIT(bar(EMPTY + s), ((uint32_t(n) >> 1) & 1u) ^ 1u);
+      mbar_wait_parked(bar(EMPTY + s), ((uint32_t(n) >> 1) & 1u) ^ 1u);
       if (elect_one()) {
         const uint32_t st = sbase + s * ATS_STAGE_BYTES;
         mbar_expect_tx(bar(FULL + s), (two ? 2 : 1) * ATT_TILE_BYTES + 2 * p.nk16 * 128);
@@ -169,7 +152,7 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     auto issue_qk = [&](int n, int t) {
       const uint32_t st = sbase + (uint32_t(n) & 1u) * ATS_STAGE_BYTES;
       if ((t == 0 ? p.alias0 : p.alias1) && nq[t] > 0) {  // the epilogue has pulled the previous O_t out of the columns S_t covers
-        ATS_WAIT(bar(T_FREE + t), (nq[t] - 1) & 1u);
+        mbar_wait_parked(bar(T_FREE + t), (nq[t] - 1) & 1u);
         tc_fence_after();
       }
       const uint64_t dq = make_smem_desc_sw128(st + t * ATT_TILE_BYTES, 16, 1024);
@@ -189,7 +172,7 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     };
     auto issue_pv = [&](int n, int t) {
       const uint32_t st = sbase + (uint32_t(n) & 1u) * ATS_STAGE_BYTES;
-      ATS_WAIT(bar(P_FULL + t), npv[t] & 1u);
+      mbar_wait_parked(bar(P_FULL + t), npv[t] & 1u);
       if (lane == 0) ATT_EV(110 + t);
       tc_fence_after();
       const uint64_t dv0 = make_smem_desc_sw128(st + ATS_OFF_V, 16, 1024);
@@ -211,56 +194,19 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       if (lane == 0) ATT_EV(120 + t);
     };
     if (n_my > 0) {
-      ATS_WAIT(bar(FULL + 0), 0u);
+      mbar_wait_parked(bar(FULL + 0), 0u);
       tc_fence_after();
       issue_qk(0, 0);
       if (two_of(item_of(0))) issue_qk(0, 1);
       for (int n = 0; n < n_my; ++n) {
         const bool two = two_of(item_of(n));
         const bool more = n + 1 < n_my;
-#if ATS_FUSED_ISSUE
-        // Tile 0 with private O columns (no T_FREE hand-shake): when the next item's operands have already landed —
-        // probed BEFORE the P_FULL wait — P.V(n), the row sums and Q.K(n+1) leave as one run of MMAs from one elected
-        // region, with every descriptor built ahead of the wake-up (the trace showed more clocks in this warp's
-        // serial work between the groups than in the MMA issue itself; same change as in attention.cuh).
-        const uint32_t fb = bar(FULL + ((uint32_t(n) + 1u) & 1u)), fpar = ((uint32_t(n) + 1u) >> 1) & 1u;
-        const bool fuse0 = more && !p.alias0 && __all_sync(0xffffffffu, mbar_try_wait(fb, fpar));
-        if (fuse0) {
-          const uint32_t st = sbase + (uint32_t(n) & 1u) * ATS_STAGE_BYTES;
-          const uint32_t stn = sbase + ((uint32_t(n) + 1u) & 1u) * ATS_STAGE_BYTES;
-          const uint64_t dv0 = make_smem_desc_sw128(st + ATS_OFF_V, 16, 1024);
-          const uint64_t dq = make_smem_desc_sw128(stn, 16, 1024);
-          const uint64_t dk = make_smem_desc_sw128(stn + ATS_OFF_K, 16, 1024);
-          const uint32_t pa0 = tmem_base + p.tm_s0, d_o = tmem_base + p.tm_o0, d_l = tmem_base + p.tm_l0;
-          ATS_WAIT(bar(P_FULL + 0), npv[0] & 1u);
-          if (lane == 0) ATT_EV(110);
+        issue_pv(n, 0);
+        if (more) {
+          mbar_wait_parked(bar(FULL + ((uint32_t(n) + 1u) & 1u)), ((uint32_t(n) + 1u) >> 1) & 1u);
+          if (lane == 0) ATT_EV(130);
           tc_fence_after();
-          if (elect_one()) {
-#pragma unroll
-            for (int k = 0; k < ATS_MAX_KV / 16; ++k)
-              if (k < ksteps) umma_ts(d_o, pa0 + 8u * k, dv0 + 128u * k, idesc_o, k != 0 ? 1u : 0u);
-#pragma unroll
-            for (int k = 0; k < ATS_MAX_KV / 16; ++k)
-              if (k < ksteps) umma_ts(d_l, pa0 + 8u * k, d_ones + 2u * (k & 3), idesc_l, k != 0 ? 1u : 0u);
-            umma_commit(bar(O_FULL + 0));
-#pragma unroll
-            for (int k = 0; k < ATT_HD / 16; ++k) umma_ss(pa0, dq + 2u * k, dk + 2u * k, idesc_s, k != 0 ? 1u : 0u);
-            umma_commit(bar(S_FULL + 0));
-          }
-          __syncwarp();
-          ++npv[0];
-          ++nq[0];
-          if (lane == 0) ATT_EV(100);
-        } else
-#endif
-        {
-          issue_pv(n, 0);
-          if (more) {
-            ATS_WAIT(bar(FULL + ((uint32_t(n) + 1u) & 1u)), ((uint32_t(n) + 1u) >> 1) & 1u);
-            if (lane == 0) ATT_EV(130);
-            tc_fence_after();
-            issue_qk(n + 1, 0);
-          }
+          issue_qk(n + 1, 0);
         }
         if (two) issue_pv(n, 1);
         if (elect_one()) umma_commit(bar(EMPTY + (uint32_t(n) & 1u)));  // every MMA reading this stage has been issued
@@ -271,7 +217,7 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     }
     if (lane == 0) mbar_arrive(bar(DONE));
   } else if (warp == 2) {
-    // ------------------------------------------------------------ watchdog (see attention.cuh)
+    // ------------------------------------------------------------ watchdog (input: the issuer's item counter)
     if (abw != nullptr) {
       uint32_t last = 0xFFFFFFFFu;
       uint64_t t_last = 0;
@@ -321,7 +267,7 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       const int row0 = qp * 256 + t * ATT_BQ;
       if (row0 >= p.Lq) continue;  // tile absent (same rule as the issuer)
       const bool warp_live = row0 + qd * 32 < p.Lq;
-      ATS_WAIT(bar(S_FULL + t), g & 1u);
+      mbar_wait_parked(bar(S_FULL + t), g & 1u);
       if (lane == 0 && qd == 0) ATT_EV(200 + t);
       tc_fence_after();
       if (warp_live) {
@@ -431,7 +377,7 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       __syncwarp();
       if (lane == 0) mbar_arrive(bar(P_FULL + t));
       if (lane == 0 && qd == 0) ATT_EV(210 + t);
-      ATS_WAIT(bar(O_FULL + t), g & 1u);
+      mbar_wait_parked(bar(O_FULL + t), g & 1u);
       tc_fence_after();
       if (lane == 0 && qd == 0) ATT_EV(220 + t);
       if (warp_live) {

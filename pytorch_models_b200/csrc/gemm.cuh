@@ -159,7 +159,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       smem + SM::kRing + SM::kStg + GEMM_SMEM_COLVEC + 8 * (2 * kStages + 4));
 
   // Role index, not the hardware warp id: the sub-partition's arbiter serves the HIGHEST warp id first (measured,
-  // B300_MICROARCH.md; attention.cuh does the same), so the two control roles (TMA producer, MMA issuer: a handful of
+  // B300_MICROARCH.md; attention_stream.cuh too), so the two control roles (TMA producer, MMA issuer: a handful of
   // instructions per K block, but every one of them on the tensor core's critical path) sit in hardware warps 8 and 9,
   // above the epilogue warps whose GELU / LayerNorm-fold arithmetic keeps the issue slots ~45 % busy; the epilogue
   // roles 2..9 are hardware warps 0..7. TMEM lane quarters follow the hardware warp id.

@@ -64,18 +64,6 @@ __device__ __forceinline__ bool mbar_try_wait_hint(uint32_t bar, uint32_t parity
       : "memory");
   return ok != 0;
 }
-// Non-blocking probe (no hardware suspend): has the phase with this parity completed?
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
 // Bounded wait. A protocol slip (or a fault in another role) must not hang the GPU: a wait that has lasted
 // B200_WAIT_LIMIT_NS raises the library's abort word (mapped host memory, see host_util.cu) and returns; once the word
 // is set, every wait that has lasted B200_WAIT_WATCH_NS (far longer than any wait of a healthy kernel, which are
@@ -187,9 +175,6 @@ __device__ __forceinline__ void tc_fence_before() {
 }
 __device__ __forceinline__ void tc_fence_after() {
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
 // ---------------------------------------------------------------- TMA
@@ -425,15 +410,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
       : "r"(taddr)
       : "memory");
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-}
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
@@ -463,15 +439,6 @@ __device__ __forceinline__ uint32_t tmem_ld1(uint32_t taddr) {
   uint32_t r;
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r) : "r"(taddr) : "memory");
   return r;
-}
-__device__ __forceinline__ uint32_t tmem_ld1_sync(uint32_t taddr) {  // load + wait
-  uint32_t r;
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];\n\ttcgen05.wait::ld.sync.aligned;"
-               : "=r"(r) : "r"(taddr) : "memory");
-  return r;
-}
-__device__ __forceinline__ void tmem_st1(uint32_t taddr, uint32_t r) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x1.b32 [%0], {%1};" ::"r"(taddr), "r"(r) : "memory");
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }

@@ -320,29 +320,14 @@ def test_bad_arguments_raise():
 
 
 @pytest.mark.parametrize("case", ["linear:tails_tma", "linear:embed_like", "linear:fold_gelu", "linear:fold_gelu_tanh", "linear:relu", "linear:fold_silu",
-                                  "attn:l197_tmem", "attn:cross_q1", "attn:causal_l448", "attn:causal_many", "rows:all"])
+                                  "attn:l197_tmem", "attn:cross_q1", "attn:causal_l448", "attn:causal_many", "attn:l576_tmem",
+                                  "attn:l1370_tmem", "attn:l1500_wide", "attn:fault", "rows:all"])
 def test_native_selftest(case):
     """The stand-alone C++ harness (fp64 CPU check inside the binary) on its edge-case shapes."""
     exe = os.path.join(ROOT, "pytorch_models_b200", "b200enc_selftest")
     if not os.path.exists(exe):
         pytest.skip("self-test binary not built")
     r = subprocess.run([exe, case], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-
-
-@pytest.mark.parametrize("case", ["attn:l576_tmem", "attn:l1370_tmem", "attn:causal_l448", "attn:l1500_wide", "attn:fault"])
-@pytest.mark.parametrize("kernel", ["v6", "v5"])
-def test_both_streaming_attention_kernels(case, kernel):
-    """The shipped streaming kernel (attention_v6.cuh) and the previous one (attention.cuh, B200ENC_ATTN_V5=1, kept for
-    same-box A/B runs) pass the same stand-alone cases, the watchdog's fault-injection run included."""
-    exe = os.path.join(ROOT, "pytorch_models_b200", "b200enc_selftest")
-    if not os.path.exists(exe):
-        pytest.skip("self-test binary not built")
-    env = dict(os.environ)
-    env.pop("B200ENC_ATTN_V5", None)
-    if kernel == "v5":
-        env["B200ENC_ATTN_V5"] = "1"
-    r = subprocess.run([exe, case], capture_output=True, text=True, timeout=300, env=env)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
 
 
