@@ -119,16 +119,17 @@ int b200enc_patch_embed16(const b200enc_linear_args* args, int img_h, int img_w,
 #define B200ENC_ATTN_DEBUG_FAULT 65536 /* self-test only: one CTA drops a barrier commit so that the watchdog path runs */
 
 /*
- * out[b][i][64h + :] = softmax_j( q[b][i][64h + :] . k[b][j][64h + :] * scale ) v[b][j][64h + :]
+ * out[b][i][hd*h + :] = softmax_j( q[b][i][hd*h + :] . k[b][j][hd*h + :] * scale ) v[b][j][hd*h + :],  hd = head_dim
  *
  * Replaces F.scaled_dot_product_attention(q, k, v, attn_mask=None, dropout_p=0, is_causal=False) at
  * transformer.py:52 together with the head split/merge views at :47-49 and :53: q, k, v are column slices of the
- * projection output (row strides ldq / ldkv, head h at columns [64h, 64h+64)), the result is head-interleaved
- * [B, Lq, H*64] ready for out_proj. head_dim must be 64 (every BASELINE config). Lq != Lkv is allowed
- * (the 1-query MAP pooling head, image/vit.py:41). K/V stream in blocks of 128 rows with an online
- * softmax. With B200ENC_ATTN_CAUSAL the K/V blocks above the diagonal are skipped entirely.
- * Unmasked calls with Lkv <= 256 (ViT-B/16 at 224 px: 197 tokens) take a single-pass kernel instead: the whole score
- * row of a query lives in tensor memory, exact maximum, no rescaling (csrc/attention_short.cuh).
+ * projection output (row strides ldq / ldkv, head h at columns [hd*h, hd*h + hd)), the result is head-interleaved
+ * [B, Lq, H*hd] ready for out_proj. head_dim is 64 (every BASELINE config) or 80, 96, 112, 128 (ViT-H/14: 80); any
+ * other value is refused. Lq != Lkv is allowed (the 1-query MAP pooling head, image/vit.py:41). K/V stream in blocks
+ * of 128 rows with an online softmax. With B200ENC_ATTN_CAUSAL the K/V blocks above the diagonal are skipped entirely.
+ * head_dim 64: unmasked calls with Lkv <= 256 (ViT-B/16 at 224 px: 197 tokens) take a single-pass kernel instead: the
+ * whole score row of a query lives in tensor memory, exact maximum, no rescaling (csrc/attention_short.cuh).
+ * head_dim 80-128 run one streaming kernel for every shape, mask and bias (csrc/attention_wide.cuh).
  */
 int b200enc_attention(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
                       long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride, int ldo, int B,

@@ -2,6 +2,7 @@
 #include "../../include/b200enc.h"
 #include "attention_short.cuh"
 #include "attention_stream.cuh"
+#include "attention_wide.cuh"
 #include "host_util.h"
 
 using namespace b200;
@@ -33,28 +34,73 @@ int launch_pdl(Kern kern, int grid, int threads, int smem, cudaStream_t s, const
 }
 }  // namespace
 
-// Two kernels: Lkv <= 256 without a mask runs the single-pass kernel of attention_short.cuh, everything else (longer
-// rows, causal, biased, or B200ENC_ATTN_GENERAL) the streaming kernel of attention_stream.cuh.
+// head_dim 64 has two kernels: Lkv <= 256 without a mask runs the single-pass kernel of attention_short.cuh, everything
+// else (longer rows, causal, biased, or B200ENC_ATTN_GENERAL) the streaming kernel of attention_stream.cuh.
+// head_dim 80, 96, 112 and 128 run the kernel of attention_wide.cuh for every Lkv, mask and bias.
+static int attention_wide(const void* q, long long qbs, int ldq, const void* k, const void* v, long long kbs, int ldkv,
+                          void* out, long long obs, int ldo, int B, int H, int Lq, int Lkv, int head_dim,
+                          float scale_log2e, int flags, const float* bias, long long bias_b_stride,
+                          long long bias_h_stride, long long bias_row_stride, cudaStream_t s) {
+  // 4-D maps (head_dim columns, H heads, L rows, B): a tile is two 64-column boxes; the columns >= head_dim of the
+  // second box are zero-filled on load and clipped on store. Output: 32 rows x 64 columns per softmax warp and store.
+  auto map = [&](CUtensorMap* m, const void* base, int L, int ld, long long bs, uint32_t box_rows) {
+    const uint64_t dims[4] = {uint64_t(head_dim), uint64_t(H), uint64_t(L), uint64_t(B)};
+    const uint64_t strides[3] = {uint64_t(head_dim) * 2, uint64_t(ld) * 2, uint64_t(bs) * 2};
+    const uint32_t box[4] = {64, 1, box_rows, 1};
+    return make_tmap_bf16_nd(m, base, 4, dims, strides, box, 128);
+  };
+  CUtensorMap tq, tk, tv, to;
+  int rc;
+  if ((rc = map(&tq, q, Lq, ldq, qbs, ATT_BQ))) return rc;
+  if ((rc = map(&tk, k, Lkv, ldkv, kbs, ATT_BKV))) return rc;
+  if ((rc = map(&tv, v, Lkv, ldkv, kbs, ATT_BKV))) return rc;
+  if ((rc = map(&to, out, Lq, ldo, obs, 32))) return rc;
+  AttnWideParams p;
+  p.B = B;
+  p.H = H;
+  p.Lq = Lq;
+  p.Lkv = Lkv;
+  p.head_dim = head_dim;
+  p.n_qp = (Lq + 2 * ATT_BQ - 1) / (2 * ATT_BQ);
+  p.n_items = B * H * p.n_qp;
+  p.scale_log2e = scale_log2e;
+  p.causal = (flags & B200ENC_ATTN_CAUSAL) ? 1 : 0;
+  p.bias = bias;
+  p.bias_b_stride = bias_b_stride;
+  p.bias_h_stride = bias_h_stride;
+  p.bias_row_stride = bias_row_stride;
+  p.abort_word = abort_word();
+  const int grid = p.n_items < sm_count() ? p.n_items : sm_count();
+  const auto kern = bias != nullptr ? attention_wide_kernel<true> : attention_wide_kernel<false>;
+  return launch_pdl(kern, grid, ATT_THREADS, ATW_SMEM_BYTES, s, tq, tk, tv, to, p);
+}
+
 static int attention_impl(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
                           long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride, int ldo, int B,
                           int H, int Lq, int Lkv, int head_dim, float scale, int flags, const float* bias,
                           long long bias_b_stride, long long bias_h_stride, long long bias_row_stride, void* stream) {
   if (int rc0 = check_abort("b200enc_attention")) return rc0;
   B200_CHECK_ARG(q && k && v && out, "b200enc_attention: null tensor pointer");
-  B200_CHECK_ARG(head_dim == ATT_HD, "b200enc_attention: head_dim=%d is not supported (only 64)", head_dim);
+  B200_CHECK_ARG(head_dim == ATT_HD || (head_dim > ATT_HD && head_dim <= ATW_MAX_HD && head_dim % 16 == 0),
+                 "b200enc_attention: head_dim=%d is not supported (64, 80, 96, 112 or 128)", head_dim);
   B200_CHECK_ARG(B >= 1 && H >= 1 && Lq >= 1 && Lkv >= 1, "b200enc_attention: bad shape B=%d H=%d Lq=%d Lkv=%d", B, H,
                  Lq, Lkv);
-  B200_CHECK_ARG(ldq >= H * ATT_HD && ldkv >= H * ATT_HD && ldo >= H * ATT_HD,
-                 "b200enc_attention: leading dimension smaller than H*64");
+  B200_CHECK_ARG(ldq >= H * head_dim && ldkv >= H * head_dim && ldo >= H * head_dim,
+                 "b200enc_attention: leading dimension smaller than H*head_dim");
   B200_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 15u) == 0 && ldo % 8 == 0 && out_batch_stride % 8 == 0,
                  "b200enc_attention: output rows must be 16-byte aligned");
+  const long long qbs = B > 1 ? q_batch_stride : (long long)Lq * ldq;
+  const long long kbs = B > 1 ? kv_batch_stride : (long long)Lkv * ldkv;
+  const long long obs = B > 1 ? out_batch_stride : (long long)Lq * ldo;
+  const float scale_log2e = scale * 1.4426950408889634f;
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  if (head_dim != ATT_HD)
+    return attention_wide(q, qbs, ldq, k, v, kbs, ldkv, out, obs, ldo, B, H, Lq, Lkv, head_dim, scale_log2e, flags,
+                          bias, bias_b_stride, bias_h_stride, bias_row_stride, s);
   const bool short_kv = Lkv <= ATS_MAX_KV && bias == nullptr && !(flags & (B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL));
   // K/V boxes: the whole row rounded up to 16 for the short kernel (N of its score MMA), 128-row blocks otherwise
   const int nk16 = (Lkv + 15) & ~15;
   const int kv_box = short_kv ? nk16 : ATT_BKV;
-  const long long qbs = B > 1 ? q_batch_stride : (long long)Lq * ldq;
-  const long long kbs = B > 1 ? kv_batch_stride : (long long)Lkv * ldkv;
-  const long long obs = B > 1 ? out_batch_stride : (long long)Lq * ldo;
   CUtensorMap tq, tk, tv, to;
   int rc;
   if ((rc = make_tmap_bf16(&tq, q, uint64_t(H) * ATT_HD, Lq, B, ldq, qbs, ATT_HD, ATT_BQ, 128))) return rc;
@@ -65,14 +111,12 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
   const int n_qp = (Lq + 2 * ATT_BQ - 1) / (2 * ATT_BQ);
   const int n_items = B * H * n_qp;
   const int grid = n_items < sm_count() ? n_items : sm_count();
-  const float scale_log2e = scale * 1.4426950408889634f;
   const int debug_fault = (flags >> 16) & 1;  // selftest only (B200ENC_ATTN_DEBUG_FAULT)
 #ifdef ATT_TRACE
   long long* const trace = g_attention_trace;
 #else
   long long* const trace = nullptr;
 #endif
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
 
   if (short_kv) {
     AttnShortParams p;

@@ -225,6 +225,12 @@ __device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, uint32_t src,
                "r"(src), "r"(c0), "r"(c1), "r"(c2)
                : "memory");
 }
+__device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2, int c3) {
+  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
+                   reinterpret_cast<uint64_t>(m)),
+               "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+               : "memory");
+}
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void tma_store_wait_read() {

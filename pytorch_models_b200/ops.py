@@ -198,13 +198,15 @@ def linear_fp8(x8: Tensor, w8: Tensor, acc_scale: Tensor, bias: Tensor | None, o
 
 def attention(q: Tensor, k: Tensor, v: Tensor, out: Tensor, n_heads: int, scale: float, causal: bool = False,
               bias: Tensor | None = None, streaming: bool = False) -> Tensor:
-    """q: (B, Lq, H*64) view, k/v: (B, Lkv, H*64) views sharing strides, out: (B, Lq, H*64).
+    """q: (B, Lq, H*hd) view, k/v: (B, Lkv, H*hd) views sharing strides, out: (B, Lq, H*hd), with head_dim
+    hd = D // n_heads in {64, 80, 96, 112, 128}.
 
     ``causal``: query i sees keys 0..i (top-left aligned like ``F.scaled_dot_product_attention(is_causal=True)``).
     ``bias``: fp32 (B, H, Lq, Lkv) view added to the scaled scores (``attn_mask`` of SDPA); broadcast dimensions may
     have stride 0 (``Tensor.expand``), the last stride must be 1.
-    Unmasked calls with Lkv <= 256 run the single-pass kernel (csrc/attention_short.cuh); ``streaming=True`` forces the
-    online-softmax kernel there too (A/B measurements and tests)."""
+    head_dim 64: unmasked calls with Lkv <= 256 run the single-pass kernel (csrc/attention_short.cuh); ``streaming=True``
+    forces the online-softmax kernel there too (A/B measurements and tests). Wider heads run csrc/attention_wide.cuh
+    for every shape, mask and bias (``streaming`` has nothing to select there)."""
     dev = _need_cuda(q, k, v, out, bias)
     for name, t in (("q", q), ("k", k), ("v", v), ("out", out)):
         _need(t, torch.bfloat16, name)

@@ -8,7 +8,7 @@ hand-written sm_100a kernels from ``libb200enc.so``:
     pre-norm layer (transformer.py:125-126), 5 launches (+1 row_stats for the first layer of a stack whose input
     did not come with statistics; ViT's patch-embedding GEMM provides them)
         linear [3·inner, d], LayerNorm folded -> fused q|k|v                  (transformer.py:87,47-49)
-        attention                             -> softmax(q kᵀ/√64) v          (transformer.py:52)
+        attention                             -> softmax(q kᵀ/√head_dim) v    (transformer.py:52)
         linear out_proj + bias + residual     -> x1 (+ partial LN statistics) (transformer.py:53,125)
         linear1, LayerNorm folded, erf-GELU   -> hidden                       (transformer.py:93,59-61)
         linear2 + bias + residual             -> x2 (+ partial LN statistics) (transformer.py:66,126)
@@ -17,8 +17,8 @@ hand-written sm_100a kernels from ``libb200enc.so``:
     its input (per-128-column (mean, M2) partials, combined in a fixed order by the consumer), so no separate pass
     over the residual stream is needed after the first layer.
 
-Only what the kernels implement is accepted (self/cross attention, optionally causal and/or with attn_bias; head_dim 64;
-GELU (erf / tanh), ReLU, SiLU; eval mode);
+Only what the kernels implement is accepted (self/cross attention, optionally causal and/or with attn_bias; head_dim 64,
+80, 96, 112 or 128; GELU (erf / tanh), ReLU, SiLU; eval mode);
 anything else raises ``NotImplementedError`` — there is no PyTorch fallback.
 """
 from __future__ import annotations
@@ -32,7 +32,7 @@ from torch import Tensor, nn
 from . import ops, plans
 from .compile import compilable, compilable_module
 
-_SUPPORTED_HEAD_DIM = 64
+_SUPPORTED_HEAD_DIMS = (64, 80, 96, 112, 128)  # 64: attention_stream / attention_short, wider: attention_wide
 _MAX_STAT_PARTS = 12  # libb200enc combines at most 12 partial statistics per row (d <= 1536)
 
 
@@ -169,8 +169,9 @@ class MHA(nn.Module):
         return self._packs[name].get(params, lambda: pack_plain(linears))
 
     def check_supported(self, attn_bias: Tensor | None = None, causal: bool = False) -> None:
-        if self.head_dim != _SUPPORTED_HEAD_DIM:
-            raise NotImplementedError(f"head_dim={self.head_dim}: the sm_100a attention kernel is specialised on 64")
+        if self.head_dim not in _SUPPORTED_HEAD_DIMS:
+            raise NotImplementedError(
+                f"head_dim={self.head_dim}: the sm_100a attention kernels take head_dim 64, 80, 96, 112 or 128")
         if self.training and self.dropout > 0.0:
             raise NotImplementedError("attention dropout (training mode) is not supported; call .eval()")
 
