@@ -41,9 +41,7 @@ void b200enc_tensor_map_cache_stats(unsigned long long* hits, unsigned long long
 #define B200ENC_LINEAR_RELU 4          /* nn.ReLU, transformer.py:63 (no residual) */
 #define B200ENC_LINEAR_SILU 8          /* nn.SiLU, transformer.py:64 (no residual) */
 #define B200ENC_LINEAR_FP8 16           /* OPTIONAL variant, never the default: x and w are e4m3 bytes, see acc_scale below */
-#define B200ENC_LINEAR_DIRECT_STORE 256 /* debug: per-thread st.global epilogue without the smem transpose */
-#define B200ENC_LINEAR_ONE_CTA 512      /* debug: 128-row tiles on single CTAs instead of 256-row tiles on CTA pairs */
-#define B200ENC_LINEAR_TWO_CTA 1024     /* debug: CTA pairs even where the wave-quantisation model prefers 128-row tiles */
+/* any other flag bit is refused (-1) */
 
 /*
  * out[b][m][n] = epi( sum_k x[b][m][k] * w[n][k] )   for b < batches, m < M, n < N      (tcgen05 GEMM)
@@ -115,8 +113,9 @@ int b200enc_patch_embed16(const b200enc_linear_args* args, int img_h, int img_w,
 
 /* flags for b200enc_attention */
 #define B200ENC_ATTN_CAUSAL 1 /* key j only visible to queries i >= j (is_causal=True of SDPA: DecoderLayer, transformer.py:97) */
-#define B200ENC_ATTN_GENERAL 131072 /* debug / A-B: use the streaming (online-softmax) kernel even where the short-sequence kernel applies */
-#define B200ENC_ATTN_DEBUG_FAULT 65536 /* self-test only: one CTA drops a barrier commit so that the watchdog path runs */
+#define B200ENC_ATTN_GENERAL 131072 /* use the streaming (online-softmax) kernel even where the short-sequence kernel
+                                       applies: the reference the tests check the short kernel against */
+/* any other flag bit is refused (-1) */
 
 /*
  * out[b][i][hd*h + :] = softmax_j( q[b][i][hd*h + :] . k[b][j][hd*h + :] * scale ) v[b][j][hd*h + :],  hd = head_dim

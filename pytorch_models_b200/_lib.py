@@ -21,7 +21,6 @@ LINEAR_SILU = 8
 ATTN_CAUSAL = 1
 ATTN_GENERAL = 131072
 LINEAR_FP8 = 16
-LINEAR_DIRECT_STORE = 256
 DTYPE_BF16 = 0
 DTYPE_F32 = 1
 

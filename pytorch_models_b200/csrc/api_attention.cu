@@ -89,6 +89,9 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
                  "b200enc_attention: leading dimension smaller than H*head_dim");
   B200_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 15u) == 0 && ldo % 8 == 0 && out_batch_stride % 8 == 0,
                  "b200enc_attention: output rows must be 16-byte aligned");
+  constexpr int kAttnFlags = B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL;
+  B200_CHECK_ARG((flags & ~kAttnFlags) == 0, "b200enc_attention: flags=%d has bits outside the documented set (0x%x)",
+                 flags, kAttnFlags);
   const long long qbs = B > 1 ? q_batch_stride : (long long)Lq * ldq;
   const long long kbs = B > 1 ? kv_batch_stride : (long long)Lkv * ldkv;
   const long long obs = B > 1 ? out_batch_stride : (long long)Lq * ldo;
@@ -111,7 +114,6 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
   const int n_qp = (Lq + 2 * ATT_BQ - 1) / (2 * ATT_BQ);
   const int n_items = B * H * n_qp;
   const int grid = n_items < sm_count() ? n_items : sm_count();
-  const int debug_fault = (flags >> 16) & 1;  // selftest only (B200ENC_ATTN_DEBUG_FAULT)
 #ifdef ATT_TRACE
   long long* const trace = g_attention_trace;
 #else
@@ -140,7 +142,6 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
       p.tm_s0 = 0, p.tm_o0 = 128, p.tm_l0 = 192, p.tm_s1 = 256, p.tm_o1 = 256 + 128, p.tm_l1 = 256 + 192, p.alias0 = p.alias1 = 1;
     }
     p.abort_word = abort_word();
-    p.debug_fault = debug_fault;
     p.trace = trace;
     // the row length of ViT at 224 px (197 tokens -> 13 halves of 16 columns) has its own instantiation
     const auto kern = nk16 == 208 ? attention_short_kernel<13> : attention_short_kernel<0>;
@@ -164,7 +165,6 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
   p.bias_h_stride = bias_h_stride;
   p.bias_row_stride = bias_row_stride;
   p.abort_word = abort_word();
-  p.debug_fault = debug_fault;
   p.trace = trace;
   const auto kern = bias != nullptr ? attention_kernel<true> : attention_kernel<false>;
   return launch_pdl(kern, grid, ATT_THREADS, ATT_SMEM_BYTES, s, tq, tk, tv, to, p);

@@ -7,10 +7,10 @@ using namespace b200;
 
 namespace {
 
-template <int kCtas, bool kFold, int kAct, bool kRes, bool kTma, bool kStats, bool kF8 = false, bool kPatch = false>
+template <int kCtas, bool kFold, int kAct, bool kRes, bool kStats, bool kF8 = false, bool kPatch = false>
 int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const GemmParams& p, int grid,
                 cudaStream_t stream) {
-  auto kern = gemm_bf16_kernel<kCtas, kFold, kAct, kRes, kTma, kStats, kF8, kPatch>;
+  auto kern = gemm_bf16_kernel<kCtas, kFold, kAct, kRes, kStats, kF8, kPatch>;
   constexpr int kSmem = GemmSmem<kCtas, kRes>::kBytes;
   if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), kSmem)) return rc;
   cudaLaunchConfig_t cfg = {};
@@ -32,16 +32,13 @@ int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap&
 }
 
 template <int kCtas, bool kFold, int kAct, bool kRes>
-int dispatch_store(bool tma, bool stats, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
-                   const GemmParams& p, int grid, cudaStream_t s) {
+int dispatch_store(bool stats, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const GemmParams& p,
+                   int grid, cudaStream_t s) {
   if constexpr (kRes && !kFold) {
-    if (stats && tma) return launch_gemm<kCtas, kFold, kAct, kRes, true, true>(ta, tb, tc, p, grid, s);
+    if (stats) return launch_gemm<kCtas, kFold, kAct, kRes, true>(ta, tb, tc, p, grid, s);
   }
-  if (stats) return set_error(-1, "b200enc_linear: stats_out needs a residual, non-folded, TMA-store epilogue");
-  if constexpr (kCtas == 1) {
-    if (!tma) return launch_gemm<1, kFold, kAct, kRes, false, false>(ta, tb, tc, p, grid, s);
-  }
-  return launch_gemm<kCtas, kFold, kAct, kRes, true, false>(ta, tb, tc, p, grid, s);
+  if (stats) return set_error(-1, "b200enc_linear: stats_out needs a residual, non-folded epilogue");
+  return launch_gemm<kCtas, kFold, kAct, kRes, false>(ta, tb, tc, p, grid, s);
 }
 
 // The FP8 variant: bias [+ erf-GELU] [+ residual], TMA store
@@ -49,29 +46,29 @@ template <int kCtas>
 int dispatch_fp8(bool gelu, bool res, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const GemmParams& p,
                  int grid, cudaStream_t s) {
   if (gelu && res) return set_error(-1, "b200enc_linear: FP8 variant: GELU and residual cannot be combined");
-  if (gelu) return launch_gemm<kCtas, false, 1, false, true, false, true>(ta, tb, tc, p, grid, s);
-  if (res) return launch_gemm<kCtas, false, 0, true, true, false, true>(ta, tb, tc, p, grid, s);
-  return launch_gemm<kCtas, false, 0, false, true, false, true>(ta, tb, tc, p, grid, s);
+  if (gelu) return launch_gemm<kCtas, false, 1, false, false, true>(ta, tb, tc, p, grid, s);
+  if (res) return launch_gemm<kCtas, false, 0, true, false, true>(ta, tb, tc, p, grid, s);
+  return launch_gemm<kCtas, false, 0, false, false, true>(ta, tb, tc, p, grid, s);
 }
 
 template <int kCtas>
-int dispatch_epilogue(int sel, bool tma, bool stats, const CUtensorMap& ta, const CUtensorMap& tb,
+int dispatch_epilogue(int sel, bool stats, const CUtensorMap& ta, const CUtensorMap& tb,
                       const CUtensorMap& tc, const GemmParams& p, int grid, cudaStream_t s) {
   switch (sel) {
-    case 0: return dispatch_store<kCtas, false, 0, false>(tma, stats, ta, tb, tc, p, grid, s);
-    case 1: return dispatch_store<kCtas, false, 0, true>(tma, stats, ta, tb, tc, p, grid, s);
-    case 2: return dispatch_store<kCtas, false, 1, false>(tma, stats, ta, tb, tc, p, grid, s);
-    case 3: return dispatch_store<kCtas, false, 1, true>(tma, stats, ta, tb, tc, p, grid, s);
-    case 4: return dispatch_store<kCtas, true, 0, false>(tma, stats, ta, tb, tc, p, grid, s);
-    case 5: return dispatch_store<kCtas, true, 0, true>(tma, stats, ta, tb, tc, p, grid, s);
-    case 6: return dispatch_store<kCtas, true, 1, false>(tma, stats, ta, tb, tc, p, grid, s);
-    case 7: return dispatch_store<kCtas, true, 1, true>(tma, stats, ta, tb, tc, p, grid, s);
-    case 8: return dispatch_store<kCtas, false, 2, false>(tma, stats, ta, tb, tc, p, grid, s);   // tanh-GELU
-    case 12: return dispatch_store<kCtas, true, 2, false>(tma, stats, ta, tb, tc, p, grid, s);   // LN fold + tanh-GELU
-    case 16: return dispatch_store<kCtas, false, 3, false>(tma, stats, ta, tb, tc, p, grid, s);  // ReLU
-    case 20: return dispatch_store<kCtas, true, 3, false>(tma, stats, ta, tb, tc, p, grid, s);
-    case 32: return dispatch_store<kCtas, false, 4, false>(tma, stats, ta, tb, tc, p, grid, s);  // SiLU
-    case 36: return dispatch_store<kCtas, true, 4, false>(tma, stats, ta, tb, tc, p, grid, s);
+    case 0: return dispatch_store<kCtas, false, 0, false>(stats, ta, tb, tc, p, grid, s);
+    case 1: return dispatch_store<kCtas, false, 0, true>(stats, ta, tb, tc, p, grid, s);
+    case 2: return dispatch_store<kCtas, false, 1, false>(stats, ta, tb, tc, p, grid, s);
+    case 3: return dispatch_store<kCtas, false, 1, true>(stats, ta, tb, tc, p, grid, s);
+    case 4: return dispatch_store<kCtas, true, 0, false>(stats, ta, tb, tc, p, grid, s);
+    case 5: return dispatch_store<kCtas, true, 0, true>(stats, ta, tb, tc, p, grid, s);
+    case 6: return dispatch_store<kCtas, true, 1, false>(stats, ta, tb, tc, p, grid, s);
+    case 7: return dispatch_store<kCtas, true, 1, true>(stats, ta, tb, tc, p, grid, s);
+    case 8: return dispatch_store<kCtas, false, 2, false>(stats, ta, tb, tc, p, grid, s);   // tanh-GELU
+    case 12: return dispatch_store<kCtas, true, 2, false>(stats, ta, tb, tc, p, grid, s);   // LN fold + tanh-GELU
+    case 16: return dispatch_store<kCtas, false, 3, false>(stats, ta, tb, tc, p, grid, s);  // ReLU
+    case 20: return dispatch_store<kCtas, true, 3, false>(stats, ta, tb, tc, p, grid, s);
+    case 32: return dispatch_store<kCtas, false, 4, false>(stats, ta, tb, tc, p, grid, s);  // SiLU
+    case 36: return dispatch_store<kCtas, true, 4, false>(stats, ta, tb, tc, p, grid, s);
     default: return set_error(-1, "b200enc_linear: tanh-GELU / ReLU / SiLU cannot be combined with a residual");
   }
 }
@@ -95,19 +92,11 @@ extern "C" int b200enc_patch_embed16(const b200enc_linear_args* a, int img_h, in
   B200_CHECK_ARG((long long)n * 3 * hp < (1ll << 31), "b200enc_patch_embed16: too many image planes");
   CUtensorMap ta, tb;
   int rc;
-  // see the kPatch comment in gemm.cuh (5-D no-swizzle form kept for A/B: -DGEMM_PATCH_SW32=0)
-  const uint64_t dims[5] = {8, uint64_t(n) * 3 * hp, 2, 16, uint64_t(wp)};
-  const uint64_t strides[4] = {uint64_t(16) * img_w * 2, 16, uint64_t(img_w) * 2, 32};
-  const uint32_t box[5] = {8, 8, 2, 4, 16};
-#if GEMM_PATCH_SW32
-  const uint64_t dims4[4] = {16, uint64_t(n) * 3 * hp, 16, uint64_t(wp)};
-  const uint64_t strides4[3] = {uint64_t(16) * img_w * 2, uint64_t(img_w) * 2, 32};
-  const uint32_t box4[4] = {16, 8, 4, 16};
-  (void)dims, (void)strides, (void)box;
-  if ((rc = make_tmap_bf16_nd(&ta, a->x, 4, dims4, strides4, box4, 32))) return rc;
-#else
-  if ((rc = make_tmap_bf16_nd(&ta, a->x, 5, dims, strides, box, 0))) return rc;
-#endif
+  // see the kPatch comment in gemm.cuh
+  const uint64_t dims[4] = {16, uint64_t(n) * 3 * hp, 16, uint64_t(wp)};
+  const uint64_t strides[3] = {uint64_t(16) * img_w * 2, uint64_t(img_w) * 2, 32};
+  const uint32_t box[4] = {16, 8, 4, 16};
+  if ((rc = make_tmap_bf16_nd(&ta, a->x, 4, dims, strides, box, 32))) return rc;
   if ((rc = make_tmap_bf16(&tb, a->w, 768, N, 0, a->ldw, 0, GEMM_BK, GEMM_BN, 128))) return rc;
   GemmParams p = {};
   p.M = P;
@@ -136,8 +125,8 @@ extern "C" int b200enc_patch_embed16(const b200enc_linear_args* a, int img_h, in
   const long long total = (long long)p.tiles_m * p.tiles_n * n;
   const int grid = int(total < sm_count() ? total : sm_count());
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  if (a->stats_out != nullptr) return launch_gemm<1, false, 0, true, false, true, false, true>(ta, tb, tb, p, grid, s);
-  return launch_gemm<1, false, 0, true, false, false, false, true>(ta, tb, tb, p, grid, s);
+  if (a->stats_out != nullptr) return launch_gemm<1, false, 0, true, true, false, true>(ta, tb, tb, p, grid, s);
+  return launch_gemm<1, false, 0, true, false, false, true>(ta, tb, tb, p, grid, s);
 }
 
 extern "C" int b200enc_linear(const b200enc_linear_args* a, void* stream) {
@@ -154,8 +143,7 @@ extern "C" int b200enc_linear(const b200enc_linear_args* a, void* stream) {
                    "b200enc_linear: FP8 variant needs K, ldx, ldw and the batch stride to be multiples of 16 bytes");
     B200_CHECK_ARG(a->acc_scale != nullptr && a->colsum == nullptr && a->stats_out == nullptr,
                    "b200enc_linear: FP8 variant needs acc_scale and supports neither the LayerNorm fold nor stats_out");
-    B200_CHECK_ARG((a->flags & (B200ENC_LINEAR_GELU_TANH | B200ENC_LINEAR_RELU | B200ENC_LINEAR_SILU |
-                                B200ENC_LINEAR_DIRECT_STORE)) == 0,
+    B200_CHECK_ARG((a->flags & (B200ENC_LINEAR_GELU_TANH | B200ENC_LINEAR_RELU | B200ENC_LINEAR_SILU)) == 0,
                    "b200enc_linear: FP8 variant supports bias, erf-GELU and residual epilogues only");
   }
   // ldx < K is allowed on purpose: overlapping rows express a strided 1-D convolution as a GEMM (whisper stem).
@@ -182,22 +170,24 @@ extern "C" int b200enc_linear(const b200enc_linear_args* a, void* stream) {
   const bool silu = (a->flags & B200ENC_LINEAR_SILU) != 0;
   B200_CHECK_ARG(int(gelu) + int(gelu_tanh) + int(relu) + int(silu) <= 1,
                  "b200enc_linear: at most one activation flag may be set");
+  constexpr int kLinearFlags =
+      B200ENC_LINEAR_GELU | B200ENC_LINEAR_GELU_TANH | B200ENC_LINEAR_RELU | B200ENC_LINEAR_SILU | B200ENC_LINEAR_FP8;
+  B200_CHECK_ARG((a->flags & ~kLinearFlags) == 0, "b200enc_linear: flags=%d has bits outside the documented set (0x%x)",
+                 a->flags, kLinearFlags);
   const bool res = a->residual != nullptr;
-  const bool tma_store = (a->flags & B200ENC_LINEAR_DIRECT_STORE) == 0;
   const bool stats = a->stats_out != nullptr;
 
-  // CTA pairs (256-row tiles) unless the problem has at most one 128-row tile per batch or the caller forbids it — or
-  // unless wave quantisation says otherwise (SURVEY §7 hard part 3): the kernel is persistent, so its time is
-  // ceil(tiles / slots) tile-times. At the strong-scaled ViT-B/16 shard (M = 25 216 = 98.5 x 256) the N = 768 GEMMs
-  // have 99 x 3 = 297 pair-tiles on 74 pairs = 4.01 -> 5 waves, the last one a single tile (20 % lost), while
-  // 128-row tiles give 197 x 3 = 591 tiles on 148 CTAs = 3.99 -> 4 waves. A 128-row tile costs about 1.15x half a
-  // pair-tile (3-stage ring, no operand sharing: round-1 A/B), which the model below charges.
-  const bool direct = (a->flags & B200ENC_LINEAR_DIRECT_STORE) != 0;
-  int ctas = (M > GEMM_BM && !(a->flags & B200ENC_LINEAR_ONE_CTA) && !direct) ? 2 : 1;
+  // CTA pairs (256-row tiles) unless the problem has at most one 128-row tile per batch — or unless wave quantisation
+  // says otherwise (SURVEY §7 hard part 3): the kernel is persistent, so its time is ceil(tiles / slots) tile-times.
+  // At the strong-scaled ViT-B/16 shard (M = 25 216 = 98.5 x 256) the N = 768 GEMMs have 99 x 3 = 297 pair-tiles on
+  // 74 pairs = 4.01 -> 5 waves, the last one a single tile (20 % lost), while 128-row tiles give 197 x 3 = 591 tiles
+  // on 148 CTAs = 3.99 -> 4 waves. A 128-row tile costs about 1.15x half a pair-tile (3-stage ring, no operand
+  // sharing: round-1 A/B), which the model below charges.
+  int ctas = M > GEMM_BM ? 2 : 1;
   // (Measured at M = 25 216, round 2: out_proj 0.036 vs 0.037 ms in favour of 128-row tiles, FC2 (K = 3072) 0.101 vs
   // 0.099 ms in favour of pairs — the longer main loop amortises the lone tile of the last wave — so the switch is
   // limited to K <= 1024.)
-  if (ctas == 2 && K <= 1024 && !(a->flags & B200ENC_LINEAR_TWO_CTA)) {
+  if (ctas == 2 && K <= 1024) {
     const long long tn = (N + GEMM_BN - 1) / GEMM_BN;
     const long long t2 = (long long)((M + 2 * GEMM_BM - 1) / (2 * GEMM_BM)) * tn * batches;
     const long long t1 = (long long)((M + GEMM_BM - 1) / GEMM_BM) * tn * batches;
@@ -222,12 +212,8 @@ extern "C" int b200enc_linear(const b200enc_linear_args* a, void* stream) {
   if ((rc = make_tmap_bf16(&tc, a->out, N, M, batches, a->ldo,
                            batches > 1 ? a->out_batch_stride : (long long)M * a->ldo, 64, 32, 128)))
     return rc;
-  if (!tma_store) {
-    B200_CHECK_ARG((reinterpret_cast<uintptr_t>(a->out) & 15u) == 0 && a->ldo % 8 == 0 && a->out_batch_stride % 8 == 0,
-                   "b200enc_linear: direct-store path needs 16-byte aligned rows");
-  }
 
-  GemmParams p;
+  GemmParams p = {};
   p.M = M;
   p.N = N;
   p.K = K;
@@ -248,11 +234,7 @@ extern "C" int b200enc_linear(const b200enc_linear_args* a, void* stream) {
   p.res = reinterpret_cast<const __nv_bfloat16*>(a->residual);
   p.res_batch_stride = a->res_batch_stride;
   p.ldr = a->ldr;
-  p.out = reinterpret_cast<__nv_bfloat16*>(a->out);
-  p.out_batch_stride = a->out_batch_stride;
-  p.ldo = a->ldo;
   p.acc_scale = a->acc_scale;
-  p.debug = (a->flags >> 16) & 3;
   p.abort_word = abort_word();
 
   const long long total = (long long)p.tiles_m * p.tiles_n * batches;
@@ -264,6 +246,6 @@ extern "C" int b200enc_linear(const b200enc_linear_args* a, void* stream) {
     return dispatch_fp8<1>(gelu, res, ta, tb, tc, p, grid, s);
   }
   const int sel = (silu ? 32 : 0) | (relu ? 16 : 0) | (gelu_tanh ? 8 : 0) | (fold ? 4 : 0) | (gelu ? 2 : 0) | (res ? 1 : 0);
-  if (ctas == 2) return dispatch_epilogue<2>(sel, tma_store, stats, ta, tb, tc, p, grid, s);
-  return dispatch_epilogue<1>(sel, tma_store, stats, ta, tb, tc, p, grid, s);
+  if (ctas == 2) return dispatch_epilogue<2>(sel, stats, ta, tb, tc, p, grid, s);
+  return dispatch_epilogue<1>(sel, stats, ta, tb, tc, p, grid, s);
 }

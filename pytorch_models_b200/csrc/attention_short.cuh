@@ -51,7 +51,6 @@ struct AttnShortParams {
   int tm_l0, tm_l1;                // 16 TMEM columns per tile that receive the row sums l = P . 1 (all 16 equal)
   int alias0, alias1;              // 1: O_t overlaps S_t, the next score MMA of the tile waits for the epilogue's read of O_t
   unsigned int* abort_word;
-  int debug_fault;
   long long* trace;
 };
 
@@ -157,14 +156,13 @@ attention_short_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       }
       const uint64_t dq = make_smem_desc_sw128(st + t * ATT_TILE_BYTES, 16, 1024);
       const uint64_t dk = make_smem_desc_sw128(st + ATS_OFF_K, 16, 1024);
-      const bool drop_commit = p.debug_fault == 1 && blockIdx.x == 0 && n == 0 && t == 0;
       if (elect_one()) {
         {
 #pragma unroll
           for (int k = 0; k < ATT_HD / 16; ++k)
             umma_ss(tmem_base + (t == 0 ? p.tm_s0 : p.tm_s1), dq + 2u * k, dk + 2u * k, idesc_s, k != 0 ? 1u : 0u);
         }
-        if (!drop_commit) umma_commit(bar(S_FULL + t));
+        umma_commit(bar(S_FULL + t));
       }
       __syncwarp();
       ++nq[t];

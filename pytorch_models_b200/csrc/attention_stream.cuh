@@ -55,7 +55,6 @@ struct AttnParams {
   long long bias_b_stride, bias_h_stride, bias_row_stride;
   long long* trace;   // debug only: (event, clock) records of CTA 0 (nullptr in production)
   unsigned int* abort_word;  // raised by the watchdog warp when the CTA stops making progress; may be nullptr
-  int debug_fault;           // selftest only: 1 = CTA 0 drops one S_FULL commit (a protocol slip) to exercise the watchdog
 };
 
 // One 128-column block of the online softmax for one query row (= one thread = one TMEM lane).
@@ -325,12 +324,11 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         const uint64_t dq = make_smem_desc_sw128(sq, 16, 1024);
         const uint64_t dk = make_smem_desc_sw128(sbase + ATT_SMEM_K + bl.stage * ATT_TILE_BYTES, 16, 1024);
         const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, n_mma_of(bl.j), 0, 0);
-        const bool drop_commit = p.debug_fault == 1 && blockIdx.x == 0 && bl.it == 0 && bl.j == 0 && t == 0;
         if (elect_one()) {
 #pragma unroll
           for (int k = 0; k < ATT_HD / 16; ++k)
             umma_ss(tmem_base + t * ATT_TM_TILE, dq + 2u * k, dk + 2u * k, idesc_s, k != 0 ? 1u : 0u);
-          if (!drop_commit) umma_commit(bar(S_FULL + t));
+          umma_commit(bar(S_FULL + t));
         }
         __syncwarp();
         ++nqk[t];

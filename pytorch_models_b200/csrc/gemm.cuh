@@ -19,14 +19,6 @@
 
 namespace b200 {
 
-// kPatch A operand: 1 = 4-D tensor map + 32-byte swizzle (32-byte TMA rows: 0.368 ms for the C2 patch embedding),
-// 0 = 5-D map + no swizzle (16-byte rows: 0.457 ms); both parity-green (b200enc_selftest patch:all)
-#ifndef GEMM_PATCH_SW32
-#define GEMM_PATCH_SW32 1
-#endif
-#ifndef GEMM_ROLES_HI
-#define GEMM_ROLES_HI 1  // 1: producer / MMA issuer in the highest hardware warps (issue priority), 0: warps 0 and 1
-#endif
 constexpr int GEMM_BM = 128;
 constexpr int GEMM_BN = 256;
 constexpr int GEMM_BK = 64;
@@ -77,14 +69,13 @@ struct GemmParams {
   const __nv_bfloat16* res;  // residual / positional table, nullptr if unused
   long long res_batch_stride;  // elements; 0 => same table for every batch (positional embedding)
   int ldr;                     // residual row stride (elements)
-  __nv_bfloat16* out;          // used by the direct-store path only
+  __nv_bfloat16* out;          // kPatch only (per-thread store of the token rows)
   long long out_batch_stride;
   int ldo;
   const float* acc_scale;  // kF8 only: device scalar, dequantisation scale of the accumulator
   // kPatch only (im2col-free patch embedding, p = 16): patch grid of one image and the tiling of its rows. An M tile is
   // 8 patch rows x 16 patch columns: tile row r <-> patch (ph0 + r % 8, pw0 + r / 8), tiles_m = pt_nph8 * pt_nw16.
   int pt_hp, pt_wp, pt_nw16;
-  int debug;  // timing experiments only: bit0 = skip the output store, bit1 = skip the whole epilogue body
   unsigned int* abort_word;  // raised by a bounded barrier wait that ran out (ptx.cuh: mbar_wait); may be nullptr
 };
 
@@ -134,8 +125,8 @@ __device__ __forceinline__ float2 silu_fast2(float2 x) {
 // 8-row x 32-byte atom of a K-major SWIZZLE_32B operand, one MMA K step wide (256 B between K steps, 1024 B between
 // 8-row groups). The 128-byte swizzle of the other GEMMs cannot be produced from NCHW: a 32-byte inner box is padded to
 // 128-byte rows there (csrc/probe_im2col_tma.cu). Rows of a tile are patches in (pw, ph % 8) order, so the epilogue maps
-// tile row -> token row and stores per thread (kTmaStore = false); patches outside the grid are zero-filled / skipped.
-template <int kCtas, bool kFold, int kAct, bool kRes, bool kTmaStore, bool kStats, bool kF8 = false, bool kPatch = false>
+// tile row -> token row and stores per thread instead of through tmC; patches outside the grid are zero-filled / skipped.
+template <int kCtas, bool kFold, int kAct, bool kRes, bool kStats, bool kF8 = false, bool kPatch = false>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmC, const GemmParams p) {
@@ -150,6 +141,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   constexpr int kBRows = SM::kBRows;
   constexpr int kStageBytes = SM::kStageBytes;
   constexpr int kTileM = GEMM_BM * kCtas;
+  constexpr bool kTmaOut = !kPatch;  // output tiles leave through tmC (TMA store); kPatch stores per thread
   // barrier slots (8 bytes each): full[kStages] empty[kStages] tfull[2] tempty[2]; then the TMEM base address word.
   auto full_bar = [&](int s) { return bars + 8u * s; };
   auto empty_bar = [&](int s) { return bars + 8u * (kStages + s); };
@@ -164,11 +156,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   // above the epilogue warps whose GELU / LayerNorm-fold arithmetic keeps the issue slots ~45 % busy; the epilogue
   // roles 2..9 are hardware warps 0..7. TMEM lane quarters follow the hardware warp id.
   const int hw_warp = threadIdx.x >> 5;
-#if GEMM_ROLES_HI
   const int warp = (hw_warp + 2) % (GEMM_THREADS / 32);
-#else
-  const int warp = hw_warp;
-#endif
   const int lane = threadIdx.x & 31;
   const uint32_t cta_rank = kCtas == 2 ? cluster_ctarank() : 0u;  // 0 = leader (issues the MMAs)
 
@@ -189,7 +177,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     fence_mbar_init();
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if (kTmaStore) tma_prefetch_desc(&tmC);
+    if (kTmaOut) tma_prefetch_desc(&tmC);
   }
   if (warp == 1) {
     if (kCtas == 2) {
@@ -237,13 +225,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           } else if (kPatch) {
             const int tm = r / p.tiles_n;
             mbar_expect_tx(full_bar(stage), kStageBytes);
-#if GEMM_PATCH_SW32
             tma_load_4d(&tmA, full_bar(stage), sa, 0, (b * 3 + (kb >> 2)) * p.pt_hp + 8 * (tm / p.pt_nw16), (kb & 3) * 4,
                         16 * (tm % p.pt_nw16));
-#else
-            tma_load_5d(&tmA, full_bar(stage), sa, 0, (b * 3 + (kb >> 2)) * p.pt_hp + 8 * (tm / p.pt_nw16), 0, (kb & 3) * 4,
-                        16 * (tm % p.pt_nw16));
-#endif
             tma_load_2d(&tmB, full_bar(stage), sa + GEMM_A_BYTES, kb * kBKe, n0);
           } else {
             mbar_expect_tx(full_bar(stage), kStageBytes);
@@ -271,11 +254,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           mbar_wait(full_bar(stage), phase, wctx);
           tc_fence_after();
           const uint32_t sa = ring + stage * kStageBytes;
-#if GEMM_PATCH_SW32
           const uint64_t da = kPatch ? make_smem_desc_sw32(sa, 256, 1024) : make_smem_desc_sw128(sa, 16, 1024);
-#else
-          const uint64_t da = kPatch ? make_smem_desc_nosw(sa, 128, 1024) : make_smem_desc_sw128(sa, 16, 1024);
-#endif
           constexpr uint32_t kAStep = kPatch ? 16u : 2u;  // 16 K elements further: two 128-byte core matrices / 32 bytes in the swizzle atom
           const uint64_t db = make_smem_desc_sw128(sa + GEMM_A_BYTES, 16, 1024);
           if (elect_one()) {
@@ -419,7 +398,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 #pragma unroll
       for (int cc = 0; cc < 2; ++cc) {
         const int nc = nh + cc * 64;
-        if (nc >= p.N || (p.debug & 2)) break;
+        if (nc >= p.N) break;
         uint32_t v0[32], v1[32];
         tmem_ld32(taddr + cc * 64, v0);
         tmem_ld32(taddr + cc * 64 + 32, v1);
@@ -437,7 +416,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         uint4 own[8];  // this lane's row of the residual chunk (kRes only)
         if (kRes) {
           constexpr int kBufOffR = SM::kStgBufs == 2 ? GEMM_STG_BYTES : 0;
-          if (kTmaStore) {  // the TMA store that last used this staging buffer has finished reading it
+          if (kTmaOut) {  // the TMA store that last used this staging buffer has finished reading it
             if (elect_one()) tma_store_wait_read<SM::kStgBufs - 1>();
             __syncwarp();
           }
@@ -498,8 +477,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           }
         }
 
-        if (p.debug & 1) continue;
-        if (kTmaStore) {
+        // A warp whose 32 rows all lie past M has nothing to store (the TMA store would clip every row). The branch
+        // also gives the chunk loop a join point before the store: without it ptxas duplicates the chunk's math for
+        // the one-chunk and two-chunk paths (+640 instructions in the residual + statistics epilogue).
+        if (kTmaOut && m0 + q * 32 >= p.M) continue;
+        if (kTmaOut) {
           // with two buffers the store that last used this one was issued a whole tile ago: no drain on the critical path
           constexpr int kBufOff = SM::kStgBufs == 2 ? GEMM_STG_BYTES : 0;
           if (!kRes) {  // (with a residual the buffer was already claimed for the transposition above)
@@ -538,7 +520,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         p.stats_out[((long long)b * p.stats_rows + p.stats_off + row) * n_slices + nh / GEMM_STAT_SLICE] =
             make_float2(mean_t, m2_t);
       }
-      if (!released) {  // warp owned no valid columns in this tile (N tail) or the epilogue body was skipped
+      if (!released) {  // warp owned no valid columns in this tile (N tail)
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
@@ -548,7 +530,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       acc ^= 1u;
       if (acc == 0) acc_phase ^= 1u;
     }
-    if (kTmaStore && elect_one()) tma_store_wait_all<0>();
+    if (kTmaOut && elect_one()) tma_store_wait_all<0>();
   }
 
   tc_fence_before();

@@ -194,14 +194,6 @@ __device__ __forceinline__ void tma_load_3d(const CUtensorMap* m, uint32_t bar, 
       "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_5d(const CUtensorMap* m, uint32_t bar, uint32_t dst, int c0, int c1, int c2, int c3,
-                                            int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(
-          dst),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
 // cta_group::2 variants: data lands in this CTA's smem, the transaction bytes are signalled on `bar_cluster`
 // (a shared::cluster address — the leader CTA's barrier).
 __device__ __forceinline__ void tma_load_2d_2cta(const CUtensorMap* m, uint32_t bar_cluster, uint32_t dst, int c0, int c1) {
@@ -369,17 +361,6 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr, uin
   d |= uint64_t((sbo_bytes >> 4) & 0x3FFFu) << 32;
   d |= uint64_t(1) << 46;
   d |= uint64_t(2) << 61;
-  return d;
-}
-
-// The same descriptor without swizzle (layout 0): a K-major operand made of 8-row x 16-byte core matrices, each 128
-// contiguous bytes; lbo = byte distance between core matrices adjacent in K, sbo = between 8-row groups (M / N).
-__device__ __forceinline__ uint64_t make_smem_desc_nosw(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= uint64_t((smem_addr & 0x3FFFFu) >> 4);
-  d |= uint64_t((lbo_bytes >> 4) & 0x3FFFu) << 16;
-  d |= uint64_t((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= uint64_t(1) << 46;
   return d;
 }
 

@@ -127,15 +127,15 @@ struct LinearCase {
   int batches, M, N, K;
   bool fold;
   int gelu;  // activation: 0 none, 1 erf-GELU, 2 tanh-GELU, 3 ReLU, 4 SiLU
-  bool res, res_bcast, direct, ints;
+  bool res, res_bcast, ints;
   int out_row_off;  // output rows shifted by this inside a (M + off)-row batch (patch-embed layout)
   int check_rows;   // rows per batch checked on the CPU (0 = all)
   int time_iters;
 };
 
 static bool run_linear(const LinearCase& c) {
-  printf("linear %s: batches=%d M=%d N=%d K=%d fold=%d gelu=%d res=%d bcast=%d direct=%d\n", c.name, c.batches, c.M,
-         c.N, c.K, c.fold, c.gelu, c.res, c.res_bcast, c.direct);
+  printf("linear %s: batches=%d M=%d N=%d K=%d fold=%d gelu=%d res=%d bcast=%d\n", c.name, c.batches, c.M, c.N, c.K,
+         c.fold, c.gelu, c.res, c.res_bcast);
   fflush(stdout);
   const int B = c.batches, M = c.M, N = c.N, K = c.K;
   const int Mo = M + c.out_row_off;
@@ -168,11 +168,9 @@ static bool run_linear(const LinearCase& c) {
   CK(cudaMemcpy(dr.p, hr.data(), hr.size() * 2, cudaMemcpyHostToDevice));
   CK(cudaMemset(dout.p, 0x7f, dout.bytes));  // sentinel 0x7f7f = 3.39e38 in bf16
 
-  const int dbg = getenv("B200_DEBUG_FLAGS") ? atoi(getenv("B200_DEBUG_FLAGS")) : 0;  // timing experiments only
-  const int extra_flags = getenv("B200_LINEAR_FLAGS") ? atoi(getenv("B200_LINEAR_FLAGS")) : 0;  // A/B: 512 one CTA, 1024 pairs
-  const int flags = extra_flags | (c.gelu == 1 ? B200ENC_LINEAR_GELU : c.gelu == 2 ? B200ENC_LINEAR_GELU_TANH : c.gelu == 3 ? B200ENC_LINEAR_RELU : c.gelu == 4 ? B200ENC_LINEAR_SILU : 0) | (c.direct ? B200ENC_LINEAR_DIRECT_STORE : 0) | (dbg << 16);
+  const int flags = c.gelu == 1 ? B200ENC_LINEAR_GELU : c.gelu == 2 ? B200ENC_LINEAR_GELU_TANH : c.gelu == 3 ? B200ENC_LINEAR_RELU : c.gelu == 4 ? B200ENC_LINEAR_SILU : 0;
   const int n_slices = (N + 127) / 128;
-  const bool want_stats = c.res && !c.fold && !c.direct;
+  const bool want_stats = c.res && !c.fold;
   GuardedBuf gso(size_t(B) * M * n_slices * 8);
   struct { void* p; } dso = {gso.p()};
   auto call = [&]() {
@@ -263,7 +261,7 @@ static bool run_linear(const LinearCase& c) {
   }
   ok = gso.intact("stats_out") && ok;
 
-  if ((ok || dbg) && c.time_iters > 0) {
+  if (ok && c.time_iters > 0) {
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));
@@ -284,34 +282,30 @@ static bool run_linear(const LinearCase& c) {
 }
 
 static const LinearCase kLinearCases[] = {
-    //  name            B   M      N     K    fold   gelu   res    bcast  direct ints  off rows iters
-    {"min_direct", 1, 128, 256, 64, false, false, false, false, true, true, 0, 0, 0},
-    {"min_tma", 1, 128, 256, 64, false, false, false, false, false, true, 0, 0, 0},
-    {"k256_direct", 1, 128, 256, 256, false, false, false, false, true, true, 0, 0, 0},
-    {"k256_tma", 1, 128, 256, 256, false, false, false, false, false, true, 0, 0, 0},
-    {"multi_tile", 1, 512, 768, 768, false, false, false, false, false, false, 0, 0, 0},
-    {"tails_direct", 1, 300, 576, 192, false, false, false, false, true, false, 0, 0, 0},
-    {"tails_tma", 1, 300, 576, 192, false, false, false, false, false, false, 0, 0, 0},
-    {"many_tiles", 1, 19000, 768, 768, false, false, false, false, false, false, 0, 40, 0},
-    {"embed_like", 3, 196, 768, 768, false, false, true, true, false, false, 1, 0, 0},
-    {"fold_gelu", 1, 1000, 3072, 768, true, true, false, false, false, false, 0, 60, 0},
-    {"fold_gelu_tanh", 1, 1000, 3072, 768, true, 2, false, false, false, false, 0, 60, 0},
-    {"gelu_tanh", 2, 300, 512, 256, false, 2, false, false, false, false, 0, 60, 0},
-    {"relu", 2, 300, 512, 256, false, 3, false, false, false, false, 0, 60, 0},
-    {"fold_silu", 1, 1000, 1024, 512, true, 4, false, false, false, false, 0, 60, 0},
-    {"residual", 1, 1000, 768, 3072, false, false, true, false, false, false, 0, 60, 0},
-    {"fold_qkv", 1, 1000, 2304, 768, true, false, false, false, false, false, 0, 60, 0},
-    {"perf_qkv", 1, 25216, 2304, 768, true, false, false, false, false, false, 0, 16, 20},
-    {"perf_out", 1, 25216, 768, 768, false, false, true, false, false, false, 0, 16, 20},
-    {"perf_fc1", 1, 25216, 3072, 768, true, true, false, false, false, false, 0, 16, 20},
-    {"perf_fc2", 1, 25216, 768, 3072, false, false, true, false, false, false, 0, 16, 20},
-    {"perf_qkv_direct", 1, 25216, 2304, 768, true, false, false, false, true, false, 0, 16, 20},
-    {"perf_qkv_l2fit", 1, 8192, 2304, 768, true, false, false, false, false, false, 0, 16, 60},
-    {"perf_qkv_big", 1, 201728, 2304, 768, true, false, false, false, false, false, 0, 8, 10},
-    {"perf_out_big", 1, 201728, 768, 768, false, false, true, false, false, false, 0, 8, 10},
-    {"perf_fc2_big", 1, 201728, 768, 3072, false, false, true, false, false, false, 0, 8, 10},
-    {"perf_fc1_big", 1, 201728, 3072, 768, true, true, false, false, false, false, 0, 8, 10},
-    {"perf_k4096", 1, 25216, 2304, 4096, false, false, false, false, false, false, 0, 8, 10},
+    //  name            B   M      N     K    fold   gelu   res    bcast  ints  off rows iters
+    {"min_tma", 1, 128, 256, 64, false, false, false, false, true, 0, 0, 0},
+    {"k256_tma", 1, 128, 256, 256, false, false, false, false, true, 0, 0, 0},
+    {"multi_tile", 1, 512, 768, 768, false, false, false, false, false, 0, 0, 0},
+    {"tails_tma", 1, 300, 576, 192, false, false, false, false, false, 0, 0, 0},
+    {"many_tiles", 1, 19000, 768, 768, false, false, false, false, false, 0, 40, 0},
+    {"embed_like", 3, 196, 768, 768, false, false, true, true, false, 1, 0, 0},
+    {"fold_gelu", 1, 1000, 3072, 768, true, true, false, false, false, 0, 60, 0},
+    {"fold_gelu_tanh", 1, 1000, 3072, 768, true, 2, false, false, false, 0, 60, 0},
+    {"gelu_tanh", 2, 300, 512, 256, false, 2, false, false, false, 0, 60, 0},
+    {"relu", 2, 300, 512, 256, false, 3, false, false, false, 0, 60, 0},
+    {"fold_silu", 1, 1000, 1024, 512, true, 4, false, false, false, 0, 60, 0},
+    {"residual", 1, 1000, 768, 3072, false, false, true, false, false, 0, 60, 0},
+    {"fold_qkv", 1, 1000, 2304, 768, true, false, false, false, false, 0, 60, 0},
+    {"perf_qkv", 1, 25216, 2304, 768, true, false, false, false, false, 0, 16, 20},
+    {"perf_out", 1, 25216, 768, 768, false, false, true, false, false, 0, 16, 20},
+    {"perf_fc1", 1, 25216, 3072, 768, true, true, false, false, false, 0, 16, 20},
+    {"perf_fc2", 1, 25216, 768, 3072, false, false, true, false, false, 0, 16, 20},
+    {"perf_qkv_l2fit", 1, 8192, 2304, 768, true, false, false, false, false, 0, 16, 60},
+    {"perf_qkv_big", 1, 201728, 2304, 768, true, false, false, false, false, 0, 8, 10},
+    {"perf_out_big", 1, 201728, 768, 768, false, false, true, false, false, 0, 8, 10},
+    {"perf_fc2_big", 1, 201728, 768, 3072, false, false, true, false, false, 0, 8, 10},
+    {"perf_fc1_big", 1, 201728, 3072, 768, true, true, false, false, false, 0, 8, 10},
+    {"perf_k4096", 1, 25216, 2304, 4096, false, false, false, false, false, 0, 8, 10},
 };
 
 
@@ -356,11 +350,10 @@ static bool run_attn(const AttnCase& c) {
   const uint16_t* kvbase_h = c.self_qkv ? hq.data() : hkv.data();
   uint16_t* kvbase_d = (uint16_t*)(c.self_qkv ? dq.p : dkv.p);
   const float scale = 0.125f;
-  const int attn_extra_flags = getenv("B200_ATTN_FLAGS") ? atoi(getenv("B200_ATTN_FLAGS")) : 0;  // A/B: 131072 = general kernel
   auto call = [&]() {
     return b200enc_attention(dq.p, (long long)Lq * ldq, ldq, kvbase_d + koff, kvbase_d + voff, (long long)Lkv * ldkv,
                              ldkv, dout.p, (long long)Lq * D, D, B, H, Lq, Lkv, 64, scale,
-                             (c.causal ? B200ENC_ATTN_CAUSAL : 0) | attn_extra_flags, nullptr);
+                             c.causal ? B200ENC_ATTN_CAUSAL : 0, nullptr);
   };
   int rc = call();
   if (rc) {
@@ -407,7 +400,7 @@ static bool run_attn(const AttnCase& c) {
   }
   bool ok = report(c.name, st);
   ok = gout.intact(c.name) && ok;
-  if ((ok || getenv("B200_DEBUG_FLAGS")) && c.time_iters > 0) {
+  if (ok && c.time_iters > 0) {
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
     CK(cudaEventCreate(&e1));
@@ -429,12 +422,11 @@ static bool run_attn(const AttnCase& c) {
 }
 
 static const AttnCase kAttnCases[] = {
-    // name        B   H   Lq    Lkv   self  psmem mag  bh iters
-    {"l64_smem", 1, 1, 64, 64, true, true, 1.0f, 0, 0},
+    // name        B   H   Lq    Lkv   self  causal mag  bh iters
+    {"causal_l64", 1, 1, 64, 64, true, true, 1.0f, 0, 0},
     {"l64_tmem", 1, 1, 64, 64, true, false, 1.0f, 0, 0},
-    {"l128_smem", 2, 2, 128, 128, true, true, 1.0f, 0, 0},
+    {"causal_l128", 2, 2, 128, 128, true, true, 1.0f, 0, 0},
     {"l128_tmem", 2, 2, 128, 128, true, false, 1.0f, 0, 0},
-    {"l197_smem", 2, 3, 197, 197, true, true, 2.0f, 0, 0},
     {"l197_tmem", 2, 3, 197, 197, true, false, 2.0f, 0, 0},
     {"l576_tmem", 1, 2, 576, 576, true, false, 2.0f, 0, 0},
     {"l1370_tmem", 1, 2, 1370, 1370, true, false, 3.0f, 1, 0},
@@ -453,7 +445,7 @@ static const AttnCase kAttnCases[] = {
     {"many_short", 150, 4, 197, 197, true, false, 2.0f, 10, 0},
     {"many_items", 40, 12, 197, 197, true, false, 2.0f, 6, 0},
     {"perf_vitb", 128, 12, 197, 197, true, false, 1.0f, 2, 20},
-    {"perf_vitb_smem", 128, 12, 197, 197, true, true, 1.0f, 2, 20},
+    {"perf_vitb_causal", 128, 12, 197, 197, true, true, 1.0f, 2, 20},
     {"perf_whisper", 8, 20, 1500, 1500, true, false, 1.0f, 1, 10},
     {"perf_siglip", 32, 16, 576, 576, true, false, 1.0f, 1, 10},
     // full-batch shapes of BASELINE configs C2..C5 (one GPU): what one attention launch of the bench processes
@@ -477,49 +469,6 @@ static const AttnCase kAttnCases[] = {
     {"many_short_q300", 200, 2, 300, 200, false, false, 2.0f, 20, 0},
     {"causal_l1100", 2, 2, 1100, 1100, true, true, 3.0f, 0, 0},
 };
-
-// Watchdog path: one CTA drops a barrier commit (B200ENC_ATTN_DEBUG_FAULT); the kernel must still terminate (within the
-// wait limit, 4 s), the status word must be raised, every entry point must refuse work until it is acknowledged, and a
-// normal launch afterwards must be correct again.
-static bool run_attn_fault() {
-  printf("attention fault injection: dropped S_FULL commit in CTA 0\n");
-  fflush(stdout);
-  const int B = 4, H = 2, L = 300, D = H * 64;
-  auto hq = rand_bf16(size_t(B) * L * 3 * D, 1.0f, false);
-  DevBuf dq(hq.size() * 2), dout(size_t(B) * L * D * 2);
-  CK(cudaMemcpy(dq.p, hq.data(), hq.size() * 2, cudaMemcpyHostToDevice));
-  uint16_t* base = (uint16_t*)dq.p;
-  auto call = [&](int flags) {
-    return b200enc_attention(dq.p, (long long)L * 3 * D, 3 * D, base + D, base + 2 * D, (long long)L * 3 * D, 3 * D, dout.p,
-                             (long long)L * D, D, B, H, L, L, 64, 0.125f, flags, nullptr);
-  };
-  if (b200enc_async_status(0) != 0) {
-    printf("  [FAIL] status word already set\n");
-    return false;
-  }
-  cudaEvent_t e0, e1;
-  CK(cudaEventCreate(&e0));
-  CK(cudaEventCreate(&e1));
-  CK(cudaEventRecord(e0));
-  int rc = call(B200ENC_ATTN_DEBUG_FAULT);
-  CK(cudaEventRecord(e1));
-  cudaError_t e = cudaDeviceSynchronize();
-  float ms = 0;
-  cudaEventElapsedTime(&ms, e0, e1);
-  const unsigned st = b200enc_async_status(0);
-  printf("  faulty launch: rc=%d sync=%s %.0f ms, status word 0x%08x\n", rc, cudaGetErrorString(e), ms, st);
-  bool ok = rc == 0 && e == cudaSuccess && st != 0 && ms > 1000.f && ms < 20000.f;
-  rc = call(0);
-  printf("  next call while the word is set: rc=%d (%s)\n", rc, b200enc_last_error());
-  ok = ok && rc == -3;
-  b200enc_async_status(1);
-  rc = call(0);
-  e = cudaDeviceSynchronize();
-  printf("  after acknowledging: rc=%d sync=%s status 0x%08x\n", rc, cudaGetErrorString(e), b200enc_async_status(0));
-  ok = ok && rc == 0 && e == cudaSuccess && b200enc_async_status(0) == 0;
-  printf("  [%s] watchdog\n", ok ? "ok" : "FAIL");
-  return ok;
-}
 
 #ifdef ATT_TRACE
 extern "C" void b200enc_debug_attention_trace(long long* buf);
@@ -806,10 +755,6 @@ int main(int argc, char** argv) {
       found = true;
       ok = run_attn(c) && ok;
     }
-  }
-  if (which == "attn:fault") {
-    found = true;
-    ok = run_attn_fault() && ok;
   }
 #ifdef ATT_TRACE
   if (which == "attn:trace") {

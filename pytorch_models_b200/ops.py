@@ -96,7 +96,6 @@ def linear(
     rowstats: Tensor | None = None,
     residual: Tensor | None = None,
     gelu: bool | str = False,
-    direct_store: bool = False,
     ln_eps: float = 0.0,
     stats_out: Tensor | None = None,
     stats_rows: int = 0,
@@ -146,11 +145,10 @@ def linear(
         act = acts[gelu]
     else:
         raise ValueError(f"gelu must be False, True, 'tanh', 'relu' or 'silu', got {gelu!r}")
-    flags = act | (_lib.LINEAR_DIRECT_STORE if direct_store else 0)
     args = _lib.LinearArgs(
         x.data_ptr(), x.stride(0), x.stride(1), w.data_ptr(), w.stride(0), _ptr(bias), _ptr(colsum),
         _ptr(rowstats), parts, float(ln_eps), _ptr(residual), res_bs, ldr, out.data_ptr(), out.stride(0), out.stride(1),
-        _ptr(stats_out), batches, M, N, K, flags, int(stats_rows), int(stats_row_offset), None,
+        _ptr(stats_out), batches, M, N, K, act, int(stats_rows), int(stats_row_offset), None,
     )
     _call(
         "b200enc_linear", dict(batches=batches, M=M, N=N, K=K, fold=colsum is not None, gelu=gelu, res=residual is not None),
@@ -205,8 +203,8 @@ def attention(q: Tensor, k: Tensor, v: Tensor, out: Tensor, n_heads: int, scale:
     ``bias``: fp32 (B, H, Lq, Lkv) view added to the scaled scores (``attn_mask`` of SDPA); broadcast dimensions may
     have stride 0 (``Tensor.expand``), the last stride must be 1.
     head_dim 64: unmasked calls with Lkv <= 256 run the single-pass kernel (csrc/attention_short.cuh); ``streaming=True``
-    forces the online-softmax kernel there too (A/B measurements and tests). Wider heads run csrc/attention_wide.cuh
-    for every shape, mask and bias (``streaming`` has nothing to select there)."""
+    forces the online-softmax kernel there too (the reference the tests check the single-pass kernel against). Wider
+    heads run csrc/attention_wide.cuh for every shape, mask and bias (``streaming`` has nothing to select there)."""
     dev = _need_cuda(q, k, v, out, bias)
     for name, t in (("q", q), ("k", k), ("v", v), ("out", out)):
         _need(t, torch.bfloat16, name)
