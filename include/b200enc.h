@@ -204,6 +204,49 @@ int b200enc_whisper_logmel(const float* audio, long long audio_stride, int N, in
                            float* out, int* sample_max, void* stream);
 
 /*
+ * Incremental decoding: single-query attention over a KV cache (csrc/attention_decode.cuh).
+ *
+ *   out[b][hd*h + :] = softmax_j( q[b][hd*h + :] . k[b][j][hd*h + :] * scale ) v[b][j][hd*h + :]
+ *
+ * Replaces F.scaled_dot_product_attention at transformer.py:52 for ONE query row per sequence, where the keys and
+ * values of the earlier positions come from a cache instead of being recomputed: the causal self-attention of
+ * DecoderLayer (transformer.py:97) one token at a time, and its cross-attention (:98) against a memory whose k|v
+ * projection was computed once. head_dim is 64, 80, 96, 112 or 128. q, out: one row per sequence (batch strides in
+ * elements). k_cache / v_cache: [B][capacity] rows of row stride ld_cache and batch stride cache_batch_stride (the K
+ * and V halves of one k|v buffer are two pointers with the same strides).
+ *
+ *   append mode (len != NULL): the keys are cache rows [0, *len) plus the new row k_new / v_new (the step's output of
+ *     the fused q|k|v projection, batch stride new_batch_stride). The new row is also written to cache row *len. *len
+ *     is read on the device, so a step's arguments are the same at every position (CUDA-graph capture); the caller
+ *     advances it (b200enc_decode_advance). A *len outside [0, capacity) gives NaN outputs and writes no cache row.
+ *     Lkv is ignored.
+ *   cross mode (len == NULL, k_new = v_new = NULL): the keys are cache rows [0, Lkv), Lkv <= capacity; read-only.
+ *
+ * workspace: fp32 device scratch of at least b200enc_attention_decode_workspace_bytes(B, H, head_dim, keys) bytes with
+ * keys = capacity (append mode) or Lkv (cross mode): per (sequence, head, chunk of keys) the partial softmax state.
+ * Two launches: the chunk partials, then their combination in a fixed order (repeats are bit-identical).
+ */
+int b200enc_attention_decode(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
+                             long long new_batch_stride, void* k_cache, void* v_cache, long long cache_batch_stride,
+                             int ld_cache, int capacity, const int* len, int Lkv, void* out, long long out_batch_stride,
+                             int B, int H, int head_dim, float scale, float* workspace, long long workspace_bytes,
+                             void* stream);
+
+/* Workspace size in bytes of b200enc_attention_decode (0 for non-positive arguments). Host-only, no device needed. */
+long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys);
+
+/*
+ * b200enc_embed_rows at a position held on the device: out[r][:] = bf16(tok[ids[r]][:] + pos[*pos0 + r % L][:]) for
+ * r < rows. The embedding of a decode step (text/gpt2.py:22-23 at position L - 1 of the growing sequence), with *pos0
+ * the cache length. pos has n_pos rows; a position outside [0, n_pos) or an id outside [0, vocab) gives a NaN row.
+ */
+int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos, int n_pos,
+                          const int* pos0, int dtype, int vocab, int d, void* out, void* stream);
+
+/* *len += delta on the device: the last launch of a decode step, so that the captured step can be replayed. */
+int b200enc_decode_advance(int* len, int delta, void* stream);
+
+/*
  * Launch plan: a recorded sequence of the entry points above, enqueued by ONE call.
  *
  * The reference's forward is a Python loop over modules (nn.Sequential at transformer.py:133-149, the layer body at

@@ -5,7 +5,9 @@ from . import _lib, ops, plans
 from .audio2text import Whisper, WhisperDecoder, WhisperEncoder, WhisperPreprocessor
 from .image import ViT
 from .text import BERT, GPT, GPT2
-from .transformer import MHA, MLP, Decoder, DecoderLayer, Encoder, EncoderLayer, invalidate_packed
+from .graphs import GraphedStep
+from .transformer import MHA, MLP, Decoder, DecoderLayer, Encoder, EncoderLayer, KVCache, invalidate_packed
 
 __all__ = ["MHA", "MLP", "Encoder", "EncoderLayer", "Decoder", "DecoderLayer", "ViT", "WhisperEncoder", "WhisperDecoder",
-           "Whisper", "WhisperPreprocessor", "BERT", "GPT", "GPT2", "ops", "plans", "invalidate_packed", "_lib"]
+           "Whisper", "WhisperPreprocessor", "BERT", "GPT", "GPT2", "ops", "plans", "invalidate_packed", "_lib",
+           "KVCache", "GraphedStep"]

@@ -94,6 +94,15 @@ _SIGNATURES = {
         c_int, [c_void_p, c_longlong, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "b200enc_time_rows": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "b200enc_run_ops": (c_int, [ctypes.POINTER(Op), c_int, ctypes.POINTER(c_int), c_void_p]),
+    "b200enc_attention_decode": (
+        c_int,
+        [c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p,
+         c_int, c_void_p, c_longlong, c_int, c_int, c_int, c_float, c_void_p, c_longlong, c_void_p],
+    ),
+    "b200enc_attention_decode_workspace_bytes": (c_longlong, [c_int, c_int, c_int, c_int]),
+    "b200enc_embed_rows_at": (
+        c_int, [c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "b200enc_decode_advance": (c_int, [c_void_p, c_int, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -1,0 +1,260 @@
+// Single-query attention over a KV cache: one decode step of a causal decoder, or its cross-attention against a
+// cached encoder memory (reference: F.scaled_dot_product_attention at transformer.py:52 with Lq = 1).
+//
+//   out[b, h] = softmax_j(scale · q[b, h] · k[b, j, h]) · v[b, j, h]
+//
+// Per key the kernel does 4·head_dim FLOPs and reads 4·head_dim bytes, so it is bound by HBM: there is no tensor-core
+// work and the design is about keeping enough loads in flight.
+//
+//   decode_partial_kernel  persistent grid over work items (b·H + h, chunk of kc keys). A CTA of 4 warps walks its
+//                          chunk; a group of kLanes lanes owns one key at a time (lane c holds columns [8c, 8c+8) of
+//                          q, k and v), each lane has kUnroll keys' 16-byte K and V loads in flight before it reduces.
+//                          Scores, the online softmax and the P·V sum are fp32 on the CUDA cores. The CTA merges its
+//                          warps and writes (max, sum, o[head_dim]) of the chunk, unnormalised, to the workspace.
+//   decode_combine_kernel  one CTA per (b, h): merges the chunk partials in chunk order (fixed order: bit-identical
+//                          repeats) and writes bf16 out.
+//
+// Append mode (len != nullptr): the keys are cache rows [0, len) plus the new row, which is read from the QKV GEMM's
+// output (k_new / v_new) instead of the cache; the one CTA whose chunk holds key `len` also copies the new row into
+// cache row `len`. No CTA reads a row that another CTA of the launch writes. `len` is read on the device, and the grid
+// and the chunk size depend only on (B, H, head_dim, capacity), so a decode step's launch arguments do not change from
+// one step to the next (CUDA-graph replay). A length outside [0, capacity) writes NaN outputs and touches no cache row.
+// Cross mode (len == nullptr): keys [0, Lkv) of a read-only cache.
+#pragma once
+#include "ptx.cuh"
+
+namespace b200 {
+
+constexpr int DEC_WARPS = 4;
+constexpr int DEC_THREADS = DEC_WARPS * 32;
+constexpr int DEC_UNROLL = 4;          // keys per lane group whose K/V loads are issued before the first is used
+constexpr int DEC_MIN_CHUNK = 64;      // keys per work item: a multiple of 64 (one CTA iteration is 32 or 64 keys)
+constexpr int DEC_MAX_CHUNK = 4096;
+constexpr int DEC_CTAS_PER_SM = 6;
+
+struct DecodeParams {
+  const __nv_bfloat16* q;      // [B] rows, head h at columns [hd*h, hd*h + hd)
+  long long q_bs;
+  const __nv_bfloat16* k_new;  // append mode: the step's k / v rows (batch stride new_bs), else nullptr
+  const __nv_bfloat16* v_new;
+  long long new_bs;
+  __nv_bfloat16* k_cache;      // [B][capacity] rows of row stride ld_cache, batch stride cache_bs
+  __nv_bfloat16* v_cache;
+  long long cache_bs;
+  long long ld_cache;
+  int capacity;
+  const int* len;              // device length (append mode) or nullptr (cross mode: Lkv keys)
+  int Lkv;
+  __nv_bfloat16* out;          // [B] rows, batch stride out_bs
+  long long out_bs;
+  int B, H, head_dim;
+  float scale_log2e;
+  int kc;                      // keys per chunk
+  int max_chunks;              // ceil(capacity + 1, kc) in append mode, ceil(Lkv, kc) in cross mode
+  float* ws;                   // [B*H][max_chunks][head_dim + 2] fp32
+};
+
+// number of keys of this launch, or -1 if the device length is out of range
+__device__ __forceinline__ int decode_keys(const DecodeParams& p) {
+  if (p.len == nullptr) return p.Lkv;
+  const int n = *p.len;
+  return (n >= 0 && n < p.capacity) ? n + 1 : -1;
+}
+
+__device__ __forceinline__ float dec_scale(float m, float mx) { return m == -INFINITY ? 0.0f : exp2f(m - mx); }
+
+__device__ __forceinline__ void dec_unpack(uint4 w, float (&f)[8]) {
+  const uint32_t u[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    f[2 * i] = __uint_as_float(u[i] << 16);
+    f[2 * i + 1] = __uint_as_float(u[i] & 0xffff0000u);
+  }
+}
+
+// kLanes = lanes per key (8: head_dim 64, 16: head_dim 80-128); lanes c >= head_dim / 8 of a group idle.
+template <int kLanes>
+__global__ void __launch_bounds__(DEC_THREADS, DEC_CTAS_PER_SM) decode_partial_kernel(const DecodeParams p) {
+  constexpr int kGroups = 32 / kLanes;
+  __shared__ float sm_ml[DEC_WARPS][2];
+  __shared__ float sm_o[DEC_WARPS][128];
+  griddep_wait();  // the previous kernel (the QKV GEMM) wrote q and the new k / v row
+  const int n_keys = decode_keys(p);
+  if (n_keys < 0) return;  // the combine kernel writes NaN
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int grp = lane / kLanes, c = lane % kLanes;
+  const int hd = p.head_dim;
+  const bool col_ok = c < (hd >> 3);
+  const int nch = (n_keys + p.kc - 1) / p.kc;
+  const int n_items = p.B * p.H * nch;
+  const int new_row = p.len != nullptr ? n_keys - 1 : -1;
+  for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
+    const int bh = item / nch, chunk = item - bh * nch;
+    const int b = bh / p.H, h = bh - b * p.H;
+    const long long col = (long long)h * hd + 8 * c;
+    float qf[8];
+    {
+      uint4 qw = make_uint4(0, 0, 0, 0);
+      if (col_ok) qw = __ldg(reinterpret_cast<const uint4*>(p.q + b * p.q_bs + col));
+      dec_unpack(qw, qf);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) qf[i] *= p.scale_log2e;
+    }
+    const __nv_bfloat16* kc_base = p.k_cache + b * p.cache_bs + col;
+    const __nv_bfloat16* vc_base = p.v_cache + b * p.cache_bs + col;
+    const int j0 = chunk * p.kc, j1 = min(j0 + p.kc, n_keys);
+    float m = -INFINITY, l = 0.0f, o[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) o[i] = 0.0f;
+    constexpr int kStep = DEC_WARPS * kGroups * DEC_UNROLL;
+    for (int jb = j0 + warp * kGroups * DEC_UNROLL; jb < j1; jb += kStep) {
+      uint4 kw[DEC_UNROLL], vw[DEC_UNROLL];
+#pragma unroll
+      for (int u = 0; u < DEC_UNROLL; ++u) {
+        const int j = jb + u * kGroups + grp;
+        kw[u] = vw[u] = make_uint4(0, 0, 0, 0);
+        if (col_ok && j < j1) {
+          const __nv_bfloat16 *kr, *vr;
+          if (j == new_row) {
+            kr = p.k_new + b * p.new_bs + col;
+            vr = p.v_new + b * p.new_bs + col;
+          } else {
+            kr = kc_base + j * p.ld_cache;
+            vr = vc_base + j * p.ld_cache;
+          }
+          kw[u] = __ldg(reinterpret_cast<const uint4*>(kr));
+          vw[u] = __ldg(reinterpret_cast<const uint4*>(vr));
+        }
+      }
+      float s[DEC_UNROLL];
+      float mx = m;
+#pragma unroll
+      for (int u = 0; u < DEC_UNROLL; ++u) {
+        float kf[8];
+        dec_unpack(kw[u], kf);
+        float d = 0.0f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) d = fmaf(qf[i], kf[i], d);
+#pragma unroll
+        for (int off = kLanes / 2; off > 0; off >>= 1) d += __shfl_xor_sync(0xffffffffu, d, off);
+        s[u] = (jb + u * kGroups + grp < j1) ? d : -INFINITY;
+        mx = fmaxf(mx, s[u]);
+      }
+      if (mx == -INFINITY) continue;  // no key of this group in range (group-uniform)
+      const float alpha = dec_scale(m, mx);
+      l *= alpha;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) o[i] *= alpha;
+#pragma unroll
+      for (int u = 0; u < DEC_UNROLL; ++u) {
+        const float pu = exp2f(s[u] - mx);  // 0 for keys out of range
+        float vf[8];
+        dec_unpack(vw[u], vf);
+        l += pu;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) o[i] = fmaf(pu, vf[i], o[i]);
+      }
+      m = mx;
+    }
+    // merge the lane groups of the warp (lanes c, c + kLanes, ... hold the same columns)
+#pragma unroll
+    for (int off = kLanes; off < 32; off <<= 1) {
+      const float m2 = __shfl_xor_sync(0xffffffffu, m, off);
+      const float l2 = __shfl_xor_sync(0xffffffffu, l, off);
+      const float mx = fmaxf(m, m2);
+      const float a = dec_scale(m, mx), a2 = dec_scale(m2, mx);
+      l = l * a + l2 * a2;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) o[i] = o[i] * a + __shfl_xor_sync(0xffffffffu, o[i], off) * a2;
+      m = mx;
+    }
+    if (lane == 0) sm_ml[warp][0] = m, sm_ml[warp][1] = l;
+    if (lane < kLanes && col_ok) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i) sm_o[warp][8 * c + i] = o[i];
+    }
+    // the chunk that holds the new key copies it into the cache (nobody in this launch reads that cache row)
+    if (new_row >= j0 && new_row < j1 && warp == 0 && lane < kLanes && col_ok) {
+      const long long src = b * p.new_bs + col, dst = b * p.cache_bs + col + new_row * p.ld_cache;
+      *reinterpret_cast<uint4*>(p.k_cache + dst) = __ldg(reinterpret_cast<const uint4*>(p.k_new + src));
+      *reinterpret_cast<uint4*>(p.v_cache + dst) = __ldg(reinterpret_cast<const uint4*>(p.v_new + src));
+    }
+    __syncthreads();
+    float* rec = p.ws + ((long long)bh * p.max_chunks + chunk) * (hd + 2);
+    float mx = sm_ml[0][0];
+#pragma unroll
+    for (int w = 1; w < DEC_WARPS; ++w) mx = fmaxf(mx, sm_ml[w][0]);
+    for (int t = threadIdx.x; t < hd + 2; t += DEC_THREADS) {
+      float acc = 0.0f;
+#pragma unroll
+      for (int w = 0; w < DEC_WARPS; ++w) {
+        const float a = dec_scale(sm_ml[w][0], mx);
+        acc += a * (t == 0 ? 0.0f : (t == 1 ? sm_ml[w][1] : sm_o[w][t - 2]));
+      }
+      rec[t] = t == 0 ? mx : acc;
+    }
+    __syncthreads();
+  }
+  griddep_launch_dependents();
+}
+
+// One CTA per (b, h); thread t < head_dim owns output column t.
+__global__ void __launch_bounds__(128) decode_combine_kernel(const DecodeParams p) {
+  griddep_wait();
+  const int bh = blockIdx.x, t = threadIdx.x, hd = p.head_dim;
+  if (t >= hd) return;
+  const int b = bh / p.H, h = bh - b * p.H;
+  __nv_bfloat16* dst = p.out + b * p.out_bs + (long long)h * hd + t;
+  const int n_keys = decode_keys(p);
+  if (n_keys < 0) {
+    *dst = __float2bfloat16_rn(__int_as_float(0x7fc00000));
+    return;
+  }
+  const int nch = (n_keys + p.kc - 1) / p.kc;
+  const float* rec = p.ws + (long long)bh * p.max_chunks * (hd + 2);
+  float mx = -INFINITY;
+  for (int c = 0; c < nch; ++c) mx = fmaxf(mx, rec[c * (hd + 2)]);
+  float l = 0.0f, o = 0.0f;
+  for (int c = 0; c < nch; ++c) {
+    const float* r = rec + c * (hd + 2);
+    const float a = dec_scale(r[0], mx);
+    l += a * r[1];
+    o += a * r[2 + t];
+  }
+  *dst = __float2bfloat16_rn(o / l);
+}
+
+// out[r] = bf16(tok[ids[r]] + pos[*pos0 + r % L]): the embedding of a decode step, whose position is the cache length
+// on the device. An id outside [0, vocab) or a position outside [0, n_pos) gives a NaN row.
+template <typename TIn>
+__global__ void __launch_bounds__(256)
+embed_rows_at_kernel(const long long* __restrict__ ids, long long rows, int L, const TIn* __restrict__ tok,
+                     const TIn* __restrict__ pos, int n_pos, const int* __restrict__ pos0, int vocab, int d,
+                     __nv_bfloat16* __restrict__ out) {
+  const int vec_per_row = d >> 3;
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= rows * vec_per_row) return;
+  const long long r = t / vec_per_row;
+  const int c = int(t % vec_per_row) * 8;
+  const long long id = ids[r];
+  const long long pr = (long long)*pos0 + r % L;
+  const bool ok = id >= 0 && id < vocab && pr >= 0 && pr < n_pos;
+  const TIn* trow = tok + (ok ? id : 0) * (long long)d + c;
+  const TIn* prow = pos + (ok ? pr : 0) * (long long)d + c;
+  uint32_t packed[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float a = ok ? float(trow[2 * i]) + float(prow[2 * i]) : __int_as_float(0x7fc00000);
+    const float b = ok ? float(trow[2 * i + 1]) + float(prow[2 * i + 1]) : __int_as_float(0x7fc00000);
+    packed[i] = pack_bf16x2(a, b);
+  }
+  *reinterpret_cast<uint4*>(out + r * d + c) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
+}
+
+// *len += delta: the last launch of a decode step
+__global__ void decode_advance_kernel(int* len, int delta) {
+  griddep_wait();
+  *len += delta;
+}
+
+}  // namespace b200

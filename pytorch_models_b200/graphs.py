@@ -12,6 +12,7 @@ import torch
 from torch import Tensor, nn
 
 from . import ops, plans
+from .transformer import step_ids_batch
 
 
 class GraphedForward:
@@ -53,5 +54,51 @@ class GraphedForward:
                              f"got {tuple(x.shape)} {x.dtype}")
         self.static_in.copy_(x, non_blocking=True)
         self.graph.replay()
+        ops.LAUNCHES += self.launches
+        return self.static_out.clone()
+
+
+class GraphedStep:
+    """``g = GraphedStep(model, cache)``; ``logits = g(ids)`` replays one captured ``model.step(ids, cache)``: the
+    decode step's counterpart of `GraphedForward` for ``GPT2`` / ``GPT`` / ``WhisperDecoder``.
+
+    A step's launches read the position from the cache's device-side length and advance it on the device, so one
+    captured graph serves every position. Capture runs warm-up steps (which write the rows past the current length and
+    advance it) and then restores the cache's length, so the cache is left as it was found. ``ids``: (B,) or (B, 1).
+    """
+
+    def __init__(self, model: nn.Module, cache, warmup: int = 2) -> None:
+        self.model, self.cache = model, cache
+        self.static_ids = torch.zeros(cache.batch, 1, device=cache.length.device, dtype=torch.long)
+        self.capture(warmup)
+
+    @torch.no_grad()
+    def capture(self, warmup: int = 2) -> None:
+        cache = self.cache
+        cache.check_step(cache.batch)  # the warm-up needs at least one free row
+        saved_len, saved_n = cache.length.clone(), cache.n
+        side = torch.cuda.Stream(cache.length.device)
+        side.wait_stream(torch.cuda.current_stream())
+        try:
+            with torch.cuda.stream(side):
+                for _ in range(max(1, min(warmup, cache.capacity - cache.n))):
+                    self.model.step(self.static_ids, cache)
+            cache.n = saved_n  # the captured step's argument checks see the cache as it was found
+            self.graph = torch.cuda.CUDAGraph()
+            n0 = ops.LAUNCHES
+            with torch.cuda.graph(self.graph):
+                self.static_out = self.model.step(self.static_ids, cache)
+            self.launches = ops.LAUNCHES - n0
+        finally:
+            torch.cuda.current_stream().wait_stream(side)
+            cache.length.copy_(saved_len)
+            cache.n = saved_n
+
+    @torch.no_grad()
+    def __call__(self, ids: Tensor) -> Tensor:
+        self.cache.check_step(step_ids_batch(ids))
+        self.static_ids.copy_(ids.reshape(-1, 1), non_blocking=True)
+        self.graph.replay()
+        self.cache.n += 1
         ops.LAUNCHES += self.launches
         return self.static_out.clone()

@@ -426,3 +426,82 @@ def whisper_logmel(audio: Tensor, filters_t: Tensor, out: Tensor) -> Tensor:
         audio.data_ptr(), audio.stride(0), N, L, filters_t.data_ptr(), n_mels, out.data_ptr(), scratch.data_ptr(),
     )
     return out
+
+
+def decode_workspace_bytes(B: int, n_heads: int, head_dim: int, keys: int) -> int:
+    """Bytes of fp32 workspace `attention_decode` needs (keys = cache capacity, or Lkv in cross mode)."""
+    return int(_lib.load().b200enc_attention_decode_workspace_bytes(B, n_heads, head_dim, keys))
+
+
+def attention_decode(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n_heads: int, scale: float,
+                     workspace: Tensor, *, k_new: Tensor | None = None, v_new: Tensor | None = None,
+                     length: Tensor | None = None, Lkv: int = 0) -> Tensor:
+    """One query row per sequence against a KV cache (csrc/attention_decode.cuh).
+
+    q, out: (B, H*hd) views with unit inner stride; k_cache / v_cache: (B, capacity, H*hd) views sharing strides;
+    workspace: fp32, at least `decode_workspace_bytes` bytes.
+    Append mode (``length`` = int32 device tensor of one element): attends over cache rows [0, length) plus the new row
+    ``k_new`` / ``v_new`` ((B, H*hd) views) and writes the new row into cache row ``length``; ``length`` itself is not
+    changed (`decode_advance`). Cross mode (``length`` None): attends over cache rows [0, Lkv)."""
+    dev = _need_cuda(q, k_cache, v_cache, out, workspace, k_new, v_new, length)
+    for name, t in (("q", q), ("k_cache", k_cache), ("v_cache", v_cache), ("out", out), ("k_new", k_new),
+                    ("v_new", v_new)):
+        _need(t, torch.bfloat16, name)
+    _need(workspace, torch.float32, "workspace"), _need(length, torch.int32, "length")
+    B, D = q.shape
+    if D % n_heads != 0:
+        raise ValueError("width not divisible by n_heads")
+    if (k_cache.dim() != 3 or k_cache.shape != v_cache.shape or k_cache.stride() != v_cache.stride()
+            or k_cache.shape[0] != B or k_cache.shape[2] != D or k_cache.stride(2) != 1):
+        raise ValueError(f"k_cache / v_cache must be (B, capacity, {D}) views sharing strides, got "
+                         f"{tuple(k_cache.shape)} / {tuple(v_cache.shape)}")
+    if out.shape != q.shape or q.stride(1) != 1 or out.stride(1) != 1:
+        raise ValueError("q / out must be (B, H*head_dim) views with unit inner stride")
+    if (k_new is None) != (length is None) or (v_new is None) != (length is None):
+        raise ValueError("append mode takes k_new, v_new and length together; cross mode none of them")
+    new_bs = 0
+    if k_new is not None:
+        if k_new.shape != q.shape or v_new.shape != q.shape or k_new.stride() != v_new.stride() or k_new.stride(1) != 1:
+            raise ValueError("k_new / v_new must be (B, H*head_dim) views sharing strides")
+        new_bs = k_new.stride(0)
+    if not workspace.is_contiguous():
+        raise ValueError("workspace must be contiguous")
+    _call(
+        "b200enc_attention_decode", dict(B=B, H=n_heads, keys=k_cache.shape[1], append=length is not None), dev,
+        q.data_ptr(), q.stride(0), _ptr(k_new), _ptr(v_new), new_bs, k_cache.data_ptr(), v_cache.data_ptr(),
+        k_cache.stride(0), k_cache.stride(1), k_cache.shape[1], _ptr(length), int(Lkv), out.data_ptr(), out.stride(0),
+        B, n_heads, D // n_heads, float(scale), workspace.data_ptr(), workspace.numel() * 4,
+    )
+    return out
+
+
+def embed_rows_at(ids: Tensor, tok: Tensor, pos: Tensor, pos0: Tensor, out: Tensor) -> Tensor:
+    """`embed_rows` at a device-side position: out[b, l] = tok[ids[b, l]] + pos[pos0 + l] with ``pos0`` an int32 device
+    tensor of one element (a decode step's cache length). A position past the table gives a NaN row."""
+    dev = _need_cuda(ids, tok, pos, pos0, out)
+    _need(ids, torch.int64, "ids"), _need(out, torch.bfloat16, "out"), _need(pos0, torch.int32, "pos0")
+    if tok.dtype != pos.dtype:
+        raise TypeError(f"token and position tables must share a dtype, got {tok.dtype} and {pos.dtype}")
+    dt = {torch.bfloat16: _lib.DTYPE_BF16, torch.float32: _lib.DTYPE_F32}.get(tok.dtype)
+    if dt is None:
+        raise TypeError(f"embedding tables must be bfloat16 or float32, got {tok.dtype}")
+    if ids.dim() != 2 or not (ids.is_contiguous() and tok.is_contiguous() and pos.is_contiguous() and out.is_contiguous()):
+        raise ValueError("embed_rows_at expects contiguous (B, L) ids, (vocab, d) / (P, d) tables and (B, L, d) output")
+    B, L = ids.shape
+    vocab, d = tok.shape
+    if pos.shape[1] != d or out.shape != (B, L, d):
+        raise ValueError(f"shape mismatch: ids {tuple(ids.shape)}, tok {tuple(tok.shape)}, pos {tuple(pos.shape)}")
+    _call(
+        "b200enc_embed_rows_at", dict(rows=B * L, d=d), dev,
+        ids.data_ptr(), B * L, L, tok.data_ptr(), pos.data_ptr(), pos.shape[0], pos0.data_ptr(), dt, vocab, d,
+        out.data_ptr(),
+    )
+    return out
+
+
+def decode_advance(length: Tensor, delta: int = 1) -> Tensor:
+    """length += delta on the device (int32, one element): the last launch of a decode step."""
+    dev = _need_cuda(length)
+    _need(length, torch.int32, "length")
+    _call("b200enc_decode_advance", dict(delta=delta), dev, length.data_ptr(), int(delta))
+    return length

@@ -2,7 +2,7 @@
 (``pytorch_models/text/generator.py:11-39``): ``DecoderGenerator(model, tokenizer).generate(prompt, max_tokens, topk)``.
 
 Behaviour kept from the reference: the prompt is encoded with ``tokenizer.encode``, one token is appended per model
-call on the whole prefix (no KV cache), ``topk == 1`` is greedy, otherwise the next token is sampled from the softmax of
+call on the whole prefix (no KV cache; ``use_cache=True`` decodes incrementally instead), ``topk == 1`` is greedy, otherwise the next token is sampled from the softmax of
 the ``topk`` largest logits, and generation stops after ``max_tokens`` new tokens or at ``tokenizer.eos_token_id``.
 The model call is the sm_100a forward of ``GPT2`` / ``GPT`` (1-D token tensor in, ``(L, vocab)`` logits out).
 """
@@ -10,6 +10,8 @@ from __future__ import annotations
 
 import torch
 from torch import Tensor, nn
+
+from ..graphs import GraphedStep
 
 
 def _pick(last_logits: Tensor, topk: int) -> int:
@@ -28,13 +30,32 @@ class DecoderGenerator:
         self.tokenizer = tokenizer
 
     @torch.inference_mode()
-    def generate(self, prompt: str, max_tokens: int = 100, topk: int = 1) -> str:
+    def generate(self, prompt: str, max_tokens: int = 100, topk: int = 1, use_cache: bool = False) -> str:
+        """``use_cache=True``: one prefill of the prompt into a KV cache, then one CUDA-graph replay of
+        ``model.step`` per new token (`graphs.GraphedStep`) instead of a forward over the whole prefix. Same stopping
+        rules and sampling; the logits agree with the uncached ones within bf16 rounding, so greedy decoding can take
+        a different branch where the two best logits are closer than that."""
         device = next(self.model.parameters()).device
         eos = self.tokenizer.eos_token_id
         ids = list(self.tokenizer.encode(prompt))
+        if use_cache and max_tokens > 0:
+            return self.tokenizer.decode(self._generate_cached(ids, max_tokens, topk, eos, device))
         for _ in range(max_tokens):
             prefix = torch.tensor(ids, device=device, dtype=torch.long)
             ids.append(_pick(self.model(prefix)[-1], topk))
             if ids[-1] == eos:
                 break
         return self.tokenizer.decode(ids)
+
+    def _generate_cached(self, ids: list, max_tokens: int, topk: int, eos, device) -> list:
+        cache = self.model.new_kv_cache(1, min(self.model.max_seq_len, len(ids) + max_tokens))
+        logits = self.model.prefill(torch.tensor(ids, device=device, dtype=torch.long), cache)[-1]
+        step = None
+        for i in range(max_tokens):
+            ids.append(_pick(logits, topk))
+            if ids[-1] == eos or i + 1 == max_tokens:
+                break
+            if step is None:
+                step = GraphedStep(self.model, cache)
+            logits = step(torch.tensor([ids[-1]], device=device, dtype=torch.long))[0]
+        return ids

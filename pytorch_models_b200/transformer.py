@@ -475,6 +475,80 @@ class DecoderLayer(nn.Module):
             ops.layernorm(ws.tmp, g2, b2, self.mlp_norm.eps, out2)
         return None
 
+    def step(self, x2: Tensor, out2: Tensor, ws: SimpleNamespace, cache: "KVCache", i: int,
+             stats_in: Tensor | None = None, want_stats: bool = False) -> Tensor | None:
+        """`run` for one new token per sequence against layer ``i`` of a KV cache: x2 (B, d) -> out2 (B, d).
+
+        The same launches and LayerNorm statistics chain as `run` at L = 1, except that each attention is
+        `ops.attention_decode` over the cache (the self-attention appends this token's k|v row) and the memory's
+        [k; v] projection is not recomputed (it lives in the cache)."""
+        sa, ca, mlp = self.sa, self.ca, self.mlp
+        B, d = x2.shape
+        inner = sa.n_heads * sa.head_dim
+        pq = self._pack_qkv()
+        po = sa._pack("out", [sa.out_proj])
+        p1 = mlp.pack1(self.mlp_norm if self.pre_norm else None)
+        p2 = mlp.pack2()
+        qkv = ws.qkv.view(B, 3 * inner)
+        att = ws.att.view(B, inner)
+        kv = cache.kv[i]
+
+        def attend_self() -> None:
+            ops.attention_decode(qkv[:, :inner], kv[:, :, :inner], kv[:, :, inner:], att, sa.n_heads, sa.scale,
+                                 cache.work, k_new=qkv[:, inner:2 * inner], v_new=qkv[:, 2 * inner:],
+                                 length=cache.length)
+
+        if ca is not None:
+            ci = ca.n_heads * ca.head_dim
+            pco = ca._pack("out", [ca.out_proj])
+            pcq = self._pack_proj(self._pcq, [ca.q_proj], self.ca_norm)
+            cq, catt = ws.cqkv.view(B, 3 * ci)[:, :ci], ws.catt.view(B, ci)
+            mkv = cache.memory_kv[i]
+
+            def attend_cross() -> None:
+                ops.attention_decode(cq, mkv[:, :, :ci], mkv[:, :, ci:], catt, ca.n_heads, ca.scale, cache.work,
+                                     Lkv=mkv.shape[1])
+
+        if self.pre_norm:
+            if stats_in is None:
+                stats_in = ops.row_stats(x2, self.sa_norm.eps, ws.stats)
+            ops.linear(x2, pq.w, pq.bias, qkv, colsum=pq.colsum, rowstats=stats_in, ln_eps=self.sa_norm.eps)
+            attend_self()
+            ops.linear(att, po.w, po.bias, ws.mid, residual=x2, stats_out=ws.parts_mid)
+            mid, mid_stats = ws.mid, ws.parts_mid
+            if ca is not None:
+                if mid_stats is None:
+                    mid_stats = ops.row_stats(mid, self.ca_norm.eps, ws.stats)
+                ops.linear(mid, pcq.w, pcq.bias, cq, colsum=pcq.colsum, rowstats=mid_stats, ln_eps=self.ca_norm.eps)
+                attend_cross()
+                ops.linear(catt, pco.w, pco.bias, ws.mid2, residual=mid, stats_out=ws.parts_mid2)
+                mid, mid_stats = ws.mid2, ws.parts_mid2
+            if mid_stats is None:
+                mid_stats = ops.row_stats(mid, self.mlp_norm.eps, ws.stats)
+            ops.linear(mid, p1.w, p1.bias, ws.hidden, colsum=p1.colsum, rowstats=mid_stats,
+                       ln_eps=self.mlp_norm.eps, gelu=mlp.gelu_mode)
+            out_stats = ws.parts_out if want_stats else None
+            ops.linear(ws.hidden, p2.w, p2.bias, out2, residual=mid, stats_out=out_stats)
+            return out_stats
+        g1, b1 = norm_vectors(self.sa_norm)
+        g2, b2 = norm_vectors(self.mlp_norm)
+        ops.linear(x2, pq.w, pq.bias, qkv)
+        attend_self()
+        ops.linear(att, po.w, po.bias, ws.tmp, residual=x2)
+        ops.layernorm(ws.tmp, g1, b1, self.sa_norm.eps, ws.mid)
+        mid = ws.mid
+        if ca is not None:
+            gc, bc = norm_vectors(self.ca_norm)
+            ops.linear(mid, pcq.w, pcq.bias, cq)
+            attend_cross()
+            ops.linear(catt, pco.w, pco.bias, ws.tmp, residual=mid)
+            ops.layernorm(ws.tmp, gc, bc, self.ca_norm.eps, ws.mid2)
+            mid = ws.mid2
+        ops.linear(mid, p1.w, p1.bias, ws.hidden, gelu=mlp.gelu_mode)
+        ops.linear(ws.hidden, p2.w, p2.bias, ws.tmp, residual=mid)
+        ops.layernorm(ws.tmp, g2, b2, self.mlp_norm.eps, out2)
+        return None
+
     def forward(self, x: Tensor, memory: Tensor | None = None) -> Tensor:
         d = self.sa_norm.normalized_shape[0]
         x3, meta = _as_tokens(x, d)
@@ -638,6 +712,129 @@ class Decoder(nn.ModuleList):
             return _restore(self.run(x3, m3), meta)
         return _restore(plans.run(self, (x3,) if m3 is None else (x3, m3), self.run), meta)
 
+    # -- incremental decoding ------------------------------------------------------------------
+    def _check_decodable(self) -> None:
+        for layer in self:
+            layer.sa.check_supported()
+            layer.mlp.check_supported()
+            if layer.ca is not None:
+                layer.ca.check_supported()
+
+    def new_kv_cache(self, batch: int, capacity: int, memory: Tensor | None = None) -> "KVCache":
+        """An empty `KVCache` for ``batch`` sequences of up to ``capacity`` tokens. A decoder with cross-attention
+        needs its encoder ``memory`` (batch, Lm, d): the [k; v] projection of every layer runs on it here, once."""
+        if not len(self):
+            raise ValueError("a decoder without layers has nothing to cache")
+        self._check_decodable()
+        if batch < 1 or capacity < 1:
+            raise ValueError(f"batch={batch} and capacity={capacity} must be >= 1")
+        m3 = None
+        if self[0].ca is not None:
+            if memory is None:
+                # without memory the block attends k = v = q over the current tokens without a mask
+                # (transformer.py:44-45, 413-419 here): every token changes every earlier output
+                raise NotImplementedError("a cross-attention decoder without memory cannot be decoded incrementally")
+            if memory.dim() != 3 or memory.shape[0] != batch or memory.shape[2] != self.d_model or memory.shape[1] < 1:
+                raise ValueError(f"memory {tuple(memory.shape)} does not match (batch={batch}, Lm, d={self.d_model})")
+            m3, _ = _as_tokens(memory, self.d_model)
+        return KVCache(self, batch, capacity, m3)
+
+    def prefill(self, x3: Tensor, cache: "KVCache") -> tuple[Tensor, Tensor | None]:
+        """`run` (``final_stats=True``) on the first P tokens of an EMPTY cache, keeping every layer's k|v rows in it:
+        x3 bf16 contiguous (B, P, d) -> (tokens, partial statistics or None). Sets the cache length to P."""
+        self._check_decodable()
+        B, P, _ = x3.shape
+        cache.check_prefill(B, P)
+        layers = list(self)
+        ws = layers[0].workspace(B, P, x3.device, 0 if cache.memory3 is None else cache.memory3.shape[1])
+        bufs = [torch.empty_like(x3), torch.empty_like(x3) if len(layers) > 1 else None]
+        cur, stats = x3, None
+        for i, layer in enumerate(layers):
+            stats = layer.run(cur, bufs[i % 2], ws, stats_in=stats, want_stats=True, memory3=cache.memory3)
+            inner = layer.sa.n_heads * layer.sa.head_dim
+            cache.kv[i][:, :P].copy_(ws.qkv[:, :, inner:])
+            cur = bufs[i % 2]
+        cache.length.fill_(P)
+        cache.n = P
+        return cur, stats
+
+    def step(self, x3: Tensor, cache: "KVCache") -> tuple[Tensor, Tensor | None]:
+        """One token per sequence: x3 bf16 contiguous (B, 1, d) at position ``cache.n`` -> (tokens (B, 1, d), partial
+        statistics or None). Appends every layer's k|v row to the cache and advances its length by one, on the device
+        (the launches are the same at every position, so `graphs.GraphedStep` can capture them). The returned tokens
+        live in a buffer of the cache that the next step overwrites."""
+        self._check_decodable()
+        B = x3.shape[0]
+        cache.check_step(B)
+        ws = cache.ws
+        cur, stats = x3.view(B, self.d_model), None
+        for i, layer in enumerate(self):
+            out = cache.bufs[i % 2]
+            stats = layer.step(cur, out, ws, cache, i, stats_in=stats, want_stats=True)
+            cur = out
+        ops.decode_advance(cache.length)
+        cache.n += 1
+        return cur.view(B, 1, self.d_model), stats
+
+
+class KVCache:
+    """Keys and values of the tokens a `Decoder` has seen, for incremental decoding (`Decoder.new_kv_cache`).
+
+    Per layer: ``kv[i]`` (batch, capacity, 2·inner) bf16, the self-attention k|v rows of positions [0, n); with
+    cross-attention ``memory_kv[i]`` (batch, Lm, 2·inner), the projected memory. ``length`` is the device-side int32
+    length the decode kernels read and the step advances; ``n`` is its host mirror, used for the argument checks. Also
+    holds the step's scratch buffers and the fp32 workspace of the decode kernel.
+
+    All sequences of a batch have the same length. A cache is valid for the weights it was filled with: after changing
+    the model's parameters, start a new cache (this is not detected)."""
+
+    def __init__(self, decoder: Decoder, batch: int, capacity: int, memory3: Tensor | None) -> None:
+        layers = list(decoder)
+        p = next(decoder.parameters())
+        dev = p.device
+        self.batch, self.capacity = batch, capacity
+        self.n = 0
+        self.length = torch.zeros(1, device=dev, dtype=torch.int32)
+        self.memory3 = memory3
+        e = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)  # noqa: E731
+        self.kv = [e(batch, capacity, 2 * layer.sa.n_heads * layer.sa.head_dim) for layer in layers]
+        self.memory_kv = None
+        ws_bytes = max(ops.decode_workspace_bytes(batch, layer.sa.n_heads, layer.sa.head_dim, capacity)
+                       for layer in layers)
+        if memory3 is not None:
+            Lm, d = memory3.shape[1], memory3.shape[2]
+            self.memory_kv = []
+            for layer in layers:
+                ca = layer.ca
+                ci = ca.n_heads * ca.head_dim
+                pkv = ca._pack("kv", [ca.k_proj, ca.v_proj])
+                mkv = e(batch, Lm, 2 * ci)
+                ops.linear(memory3.view(batch * Lm, d), pkv.w, pkv.bias, mkv.view(batch * Lm, 2 * ci))
+                self.memory_kv.append(mkv)
+                ws_bytes = max(ws_bytes, ops.decode_workspace_bytes(batch, ca.n_heads, ca.head_dim, Lm))
+        self.work = torch.empty((ws_bytes + 3) // 4, device=dev, dtype=torch.float32)
+        self.ws = layers[0].workspace(batch, 1, dev, 0)
+        self.bufs = [e(batch, decoder.d_model), e(batch, decoder.d_model)]
+
+    def reset(self) -> None:
+        """Empty the cache (for a new prefill); the buffers are kept."""
+        self.length.zero_()
+        self.n = 0
+
+    def check_prefill(self, batch: int, P: int) -> None:
+        if batch != self.batch:
+            raise ValueError(f"batch {batch} does not match the cache's batch {self.batch}")
+        if self.n != 0:
+            raise ValueError(f"prefill needs an empty cache (it holds {self.n} tokens; call reset())")
+        if not 1 <= P <= self.capacity:
+            raise ValueError(f"prefill of {P} tokens into a cache of capacity {self.capacity}")
+
+    def check_step(self, batch: int) -> None:
+        if batch != self.batch:
+            raise ValueError(f"batch {batch} does not match the cache's batch {self.batch}")
+        if self.n >= self.capacity:
+            raise ValueError(f"the cache is full ({self.n} of {self.capacity} tokens)")
+
 
 # ----------------------------------------------------------------------------------------------- language-model ends
 def embed_tokens(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor) -> Tensor:
@@ -660,6 +857,32 @@ def embed_tokens(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor) -> Ten
     ids2 = ids.reshape(-1, L).to(torch.int64).contiguous()
     out = torch.empty(ids2.shape[0], L, tok.shape[1], device=ids.device, dtype=torch.bfloat16)
     return ops.embed_rows(ids2, tok.contiguous(), pos.contiguous(), out)
+
+
+def embed_tokens_at(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor, cache: KVCache) -> Tensor:
+    """`embed_tokens` of one new token per sequence at position ``cache.n``: (B,) or (B, 1) int64 -> contiguous bf16
+    (B, 1, d). The position is read on the device (the cache length), so the launch is the same at every step."""
+    if not ids.is_cuda:
+        raise RuntimeError(
+            "pytorch_models_b200 runs only on CUDA (sm_100a) tensors; there is no CPU fallback "
+            f"(got a {ids.device} tensor)"
+        )
+    tok = token_embs.weight.detach()
+    pos = pos_embs.detach()
+    if tok.dtype not in (torch.float32, torch.bfloat16):
+        tok = tok.float()
+    if pos.dtype != tok.dtype:
+        pos = pos.to(tok.dtype)
+    ids2 = ids.reshape(-1, 1).to(torch.int64).contiguous()
+    out = torch.empty(ids2.shape[0], 1, tok.shape[1], device=ids.device, dtype=torch.bfloat16)
+    return ops.embed_rows_at(ids2, tok.contiguous(), pos.contiguous(), cache.length, out)
+
+
+def step_ids_batch(ids: Tensor) -> int:
+    """Batch of a decode step's token ids: (B,) or (B, 1)."""
+    if ids.dim() > 2 or (ids.dim() == 2 and ids.shape[1] != 1):
+        raise ValueError(f"a decode step takes one token per sequence, (B,) or (B, 1) ids; got {tuple(ids.shape)}")
+    return ids.shape[0] if ids.dim() else 1
 
 
 class TiedLogits:
