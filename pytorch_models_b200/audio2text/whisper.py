@@ -20,8 +20,8 @@ from torch import Tensor, nn
 
 from .. import ops, plans
 from ..compile import compilable, compilable_module, float_like
-from ..transformer import (Decoder, Encoder, KVCache, TiedLogits, _as_tokens, _Packed, embed_tokens, embed_tokens_at,
-                           norm_vectors, step_ids_batch)
+from ..transformer import (Decoder, DecoderLM, Encoder, KVCache, TiedLogits, _as_tokens, _Packed, embed_tokens,
+                           norm_vectors)
 
 
 @compilable_module
@@ -156,7 +156,7 @@ def _load_openai(half: nn.Module, state_dict: dict, prefix: str) -> None:
 
 
 @compilable_module
-class WhisperDecoder(nn.Module):
+class WhisperDecoder(DecoderLM, nn.Module):
     """Reference ``WhisperDecoder`` (whisper.py:37-53)."""
 
     max_seq_len = 448
@@ -172,43 +172,17 @@ class WhisperDecoder(nn.Module):
     @compilable(lambda self, x, extra: ((*x.shape, self.token_embs.weight.shape[0]), self.token_embs.weight.dtype))
     def forward(self, x: Tensor, memory: Tensor) -> Tensor:
         """x: (N, L) int64 token ids, memory: (N, Lm, d) encoder output -> (N, L, vocab) logits (whisper.py:46-52)."""
-        out_dtype = self.token_embs.weight.dtype
-        d = self.token_embs.weight.shape[1]
-        m3, _ = _as_tokens(memory, d)
+        m3, _ = _as_tokens(memory, self.token_embs.weight.shape[1])
         h, stats = self.layers.run(embed_tokens(x, self.token_embs, self.pos_embs), m3, final_stats=True)
-        logits = self._logits(h, self.token_embs, self.norm, stats)
-        logits = logits.reshape(*x.shape, logits.shape[-1])
-        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
+        return self._logits_as(h, stats, x.shape)
 
-    # -- incremental decoding (no reference counterpart: the reference recomputes the whole prefix) ----------------
     def new_kv_cache(self, memory: Tensor, capacity: int) -> KVCache:
         """An empty KV cache for the (N, Lm, d) encoder output ``memory`` and up to ``capacity`` <= max_seq_len tokens.
         Every layer's cross-attention [k; v] projection of the memory runs here, once."""
-        if capacity > self.pos_embs.shape[0]:
-            raise ValueError(f"capacity {capacity} exceeds the {self.pos_embs.shape[0]} rows of the position table")
+        self._check_capacity(capacity)
         if memory.dim() != 3:
             raise ValueError(f"memory must be (N, Lm, d), got {tuple(memory.shape)}")
         return self.layers.new_kv_cache(memory.shape[0], capacity, memory)
-
-    def prefill(self, x: Tensor, cache: KVCache) -> Tensor:
-        """`forward` on the first (N, P) target ids against the cache's memory, filling the empty ``cache``:
-        (N, P, vocab) logits."""
-        cache.check_prefill(x.reshape(-1, x.shape[-1]).shape[0], x.shape[-1])
-        out_dtype = self.token_embs.weight.dtype
-        h, stats = self.layers.prefill(embed_tokens(x, self.token_embs, self.pos_embs), cache)
-        logits = self._logits(h, self.token_embs, self.norm, stats)
-        logits = logits.reshape(*x.shape, logits.shape[-1])
-        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
-
-    def step(self, x: Tensor, cache: KVCache) -> Tensor:
-        """The next token of every sequence, (N,) or (N, 1) ids at position ``cache.n`` -> (N, vocab) logits.
-        Appends to the cache."""
-        cache.check_step(step_ids_batch(x))
-        self.layers._check_decodable()
-        out_dtype = self.token_embs.weight.dtype
-        h, stats = self.layers.step(embed_tokens_at(x, self.token_embs, self.pos_embs, cache), cache)
-        logits = self._logits(h, self.token_embs, self.norm, stats)[:, 0]
-        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
 
 
 _OPENAI_SIZES = {

@@ -379,25 +379,30 @@ def time_rows(x: Tensor, rows: Tensor) -> Tensor:
     return rows
 
 
+def _embed_args(name: str, ids: Tensor, tok: Tensor, pos: Tensor, out: Tensor) -> int:
+    """Argument checks shared by `embed_rows` and `embed_rows_at`; returns the library's dtype code of the tables."""
+    _need(ids, torch.int64, "ids"), _need(out, torch.bfloat16, "out")
+    if tok.dtype != pos.dtype:
+        raise TypeError(f"token and position tables must share a dtype, got {tok.dtype} and {pos.dtype}")
+    dt = {torch.bfloat16: _lib.DTYPE_BF16, torch.float32: _lib.DTYPE_F32}.get(tok.dtype)
+    if dt is None:
+        raise TypeError(f"embedding tables must be bfloat16 or float32, got {tok.dtype}")
+    if ids.dim() != 2 or not (ids.is_contiguous() and tok.is_contiguous() and pos.is_contiguous() and out.is_contiguous()):
+        raise ValueError(f"{name} expects contiguous (B, L) ids, (vocab, d) / (P, d) tables and (B, L, d) output")
+    if pos.shape[1] != tok.shape[1] or out.shape != (*ids.shape, tok.shape[1]):
+        raise ValueError(f"shape mismatch: ids {tuple(ids.shape)}, tok {tuple(tok.shape)}, pos {tuple(pos.shape)}")
+    return dt
+
+
 def embed_rows(ids: Tensor, tok: Tensor, pos: Tensor, out: Tensor) -> Tensor:
     """ids: (B, L) int64, tok: (vocab, d), pos: (>= L, d) [both fp32 or both bf16] -> out (B, L, d) bf16 =
     tok[ids] + pos[:L]. Rows whose id is out of range come back as NaN (device code cannot raise)."""
     dev = _need_cuda(ids, tok, pos, out)
-    _need(ids, torch.int64, "ids"), _need(out, torch.bfloat16, "out")
-    if tok.dtype != pos.dtype:
-        raise TypeError(f"token and position tables must share a dtype, got {tok.dtype} and {pos.dtype}")
-    if tok.dtype == torch.bfloat16:
-        dt = _lib.DTYPE_BF16
-    elif tok.dtype == torch.float32:
-        dt = _lib.DTYPE_F32
-    else:
-        raise TypeError(f"embedding tables must be bfloat16 or float32, got {tok.dtype}")
-    if ids.dim() != 2 or not (ids.is_contiguous() and tok.is_contiguous() and pos.is_contiguous() and out.is_contiguous()):
-        raise ValueError("embed_rows expects contiguous (B, L) ids, (vocab, d) / (P, d) tables and (B, L, d) output")
+    dt = _embed_args("embed_rows", ids, tok, pos, out)
     B, L = ids.shape
     vocab, d = tok.shape
-    if pos.shape[1] != d or pos.shape[0] < L or out.shape != (B, L, d):
-        raise ValueError(f"shape mismatch: ids {tuple(ids.shape)}, tok {tuple(tok.shape)}, pos {tuple(pos.shape)}")
+    if pos.shape[0] < L:
+        raise ValueError(f"the position table has {pos.shape[0]} rows, fewer than the {L} ids of a row")
     if B * L == 0:
         return out
     _call(
@@ -479,18 +484,10 @@ def embed_rows_at(ids: Tensor, tok: Tensor, pos: Tensor, pos0: Tensor, out: Tens
     """`embed_rows` at a device-side position: out[b, l] = tok[ids[b, l]] + pos[pos0 + l] with ``pos0`` an int32 device
     tensor of one element (a decode step's cache length). A position past the table gives a NaN row."""
     dev = _need_cuda(ids, tok, pos, pos0, out)
-    _need(ids, torch.int64, "ids"), _need(out, torch.bfloat16, "out"), _need(pos0, torch.int32, "pos0")
-    if tok.dtype != pos.dtype:
-        raise TypeError(f"token and position tables must share a dtype, got {tok.dtype} and {pos.dtype}")
-    dt = {torch.bfloat16: _lib.DTYPE_BF16, torch.float32: _lib.DTYPE_F32}.get(tok.dtype)
-    if dt is None:
-        raise TypeError(f"embedding tables must be bfloat16 or float32, got {tok.dtype}")
-    if ids.dim() != 2 or not (ids.is_contiguous() and tok.is_contiguous() and pos.is_contiguous() and out.is_contiguous()):
-        raise ValueError("embed_rows_at expects contiguous (B, L) ids, (vocab, d) / (P, d) tables and (B, L, d) output")
+    _need(pos0, torch.int32, "pos0")
+    dt = _embed_args("embed_rows_at", ids, tok, pos, out)
     B, L = ids.shape
     vocab, d = tok.shape
-    if pos.shape[1] != d or out.shape != (B, L, d):
-        raise ValueError(f"shape mismatch: ids {tuple(ids.shape)}, tok {tuple(tok.shape)}, pos {tuple(pos.shape)}")
     _call(
         "b200enc_embed_rows_at", dict(rows=B * L, d=d), dev,
         ids.data_ptr(), B * L, L, tok.data_ptr(), pos.data_ptr(), pos.shape[0], pos0.data_ptr(), dt, vocab, d,
@@ -500,7 +497,7 @@ def embed_rows_at(ids: Tensor, tok: Tensor, pos: Tensor, pos0: Tensor, out: Tens
 
 
 def decode_advance(length: Tensor, delta: int = 1) -> Tensor:
-    """length += delta on the device (int32, one element): the last launch of a decode step."""
+    """length += delta on the device (int32, one element): issued at the end of a decode step's decoder stack."""
     dev = _need_cuda(length)
     _need(length, torch.int32, "length")
     _call("b200enc_decode_advance", dict(delta=delta), dev, length.data_ptr(), int(delta))

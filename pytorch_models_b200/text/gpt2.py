@@ -11,11 +11,11 @@ import torch
 from torch import Tensor, nn
 
 from ..compile import compilable, compilable_module
-from ..transformer import Decoder, KVCache, TiedLogits, embed_tokens, embed_tokens_at, step_ids_batch
+from ..transformer import Decoder, DecoderLM, TiedLogits, embed_tokens
 
 
 @compilable_module
-class GPT2(nn.Module):
+class GPT2(DecoderLM, nn.Module):
     vocab_size = 50257
     max_seq_len: int = 1024
 
@@ -30,37 +30,8 @@ class GPT2(nn.Module):
     @compilable(lambda self, x, extra: ((*x.shape, self.token_embs.weight.shape[0]), self.token_embs.weight.dtype))
     def forward(self, x: Tensor) -> Tensor:
         """(*, L) int64 token ids -> (*, L, vocab) logits in the parameters' dtype (gpt2.py:21-27)."""
-        out_dtype = self.token_embs.weight.dtype
         h, stats = self.layers.run(embed_tokens(x, self.token_embs, self.pos_embs), final_stats=True)
-        logits = self._logits(h, self.token_embs, self.norm, stats)
-        logits = logits.reshape(*x.shape, logits.shape[-1])
-        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
-
-    # -- incremental decoding (no reference counterpart: the reference recomputes the whole prefix) ----------------
-    def new_kv_cache(self, batch: int, capacity: int) -> KVCache:
-        """An empty KV cache for ``batch`` sequences of up to ``capacity`` <= max_seq_len tokens (see `prefill`)."""
-        if capacity > self.pos_embs.shape[0]:
-            raise ValueError(f"capacity {capacity} exceeds the {self.pos_embs.shape[0]} rows of the position table")
-        return self.layers.new_kv_cache(batch, capacity)
-
-    def prefill(self, x: Tensor, cache: KVCache) -> Tensor:
-        """`forward` on the prompt, (B, P) or (P,) ids, that also fills an empty ``cache``: (*, P, vocab) logits."""
-        cache.check_prefill(x.reshape(-1, x.shape[-1]).shape[0], x.shape[-1])
-        out_dtype = self.token_embs.weight.dtype
-        h, stats = self.layers.prefill(embed_tokens(x, self.token_embs, self.pos_embs), cache)
-        logits = self._logits(h, self.token_embs, self.norm, stats)
-        logits = logits.reshape(*x.shape, logits.shape[-1])
-        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
-
-    def step(self, x: Tensor, cache: KVCache) -> Tensor:
-        """The next token of every sequence, (B,) or (B, 1) ids at position ``cache.n`` -> (B, vocab) logits, equal
-        to ``forward(prefix)[:, -1]`` within bf16 rounding. Appends to the cache."""
-        cache.check_step(step_ids_batch(x))
-        self.layers._check_decodable()
-        out_dtype = self.token_embs.weight.dtype
-        h, stats = self.layers.step(embed_tokens_at(x, self.token_embs, self.pos_embs, cache), cache)
-        logits = self._logits(h, self.token_embs, self.norm, stats)[:, 0]
-        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
+        return self._logits_as(h, stats, x.shape)
 
     @staticmethod
     def from_hf(model_tag: str, *, pretrained: bool = False, **kwargs) -> "GPT2":

@@ -393,29 +393,28 @@ class DecoderLayer(nn.Module):
 
         ``stats_in``: partial LayerNorm statistics of x3 written by the producing GEMM (else a row_stats pass runs).
         Returns the partial statistics of out3 when ``want_stats`` (for the next layer's sa_norm), else None."""
-        sa, ca, mlp = self.sa, self.ca, self.mlp
+        sa, ca = self.sa, self.ca
         sa.check_supported()
-        mlp.check_supported()
+        self.mlp.check_supported()
         B, L, d = x3.shape
-        M = B * L
         inner = sa.n_heads * sa.head_dim
-        x2, out2 = x3.view(M, d), out3.view(M, d)
-        pq = self._pack_qkv()
-        po = sa._pack("out", [sa.out_proj])
-        p1 = mlp.pack1(self.mlp_norm if self.pre_norm else None)
-        p2 = mlp.pack2()
-        qkv2 = ws.qkv.view(M, 3 * inner)
-        q, k, v = ws.qkv[:, :, :inner], ws.qkv[:, :, inner:2 * inner], ws.qkv[:, :, 2 * inner:]
+        qkv = ws.qkv
+
+        def attend_self(_qkv2: Tensor, _att2: Tensor) -> None:  # takes the (B, L, ·) views of the same buffers
+            ops.attention(qkv[:, :, :inner], qkv[:, :, inner:2 * inner], qkv[:, :, 2 * inner:], ws.att, sa.n_heads,
+                          sa.scale, self._causal)
+
+        cross = None
         if ca is not None:
             ca.check_supported()
             ci = ca.n_heads * ca.head_dim
-            pco = ca._pack("out", [ca.out_proj])
             if memory3 is None:
                 # memory=None: MHA.forward(q, None) takes k = v = q (transformer.py:44-45), i.e. the cross-attention
                 # block degenerates to un-masked self-attention with the ca weights on ca_norm(x) (pre-norm) / x
                 if ws.Lm != 0:
                     raise ValueError("workspace was sized for a memory but none was given")
-                pcqkv = self._pack_proj(self._pcqkv, [ca.q_proj, ca.k_proj, ca.v_proj], self.ca_norm)
+                pcq = self._pack_proj(self._pcqkv, [ca.q_proj, ca.k_proj, ca.v_proj], self.ca_norm)
+                cq_out = ws.cqkv.view(B * L, 3 * ci)
                 cq, ck, cv = ws.cqkv[:, :, :ci], ws.cqkv[:, :, ci:2 * ci], ws.cqkv[:, :, 2 * ci:]
             else:
                 if memory3.shape[0] != B or memory3.shape[2] != d or memory3.shape[1] != ws.Lm:
@@ -423,104 +422,76 @@ class DecoderLayer(nn.Module):
                 Mm = B * ws.Lm
                 pcq = self._pack_proj(self._pcq, [ca.q_proj], self.ca_norm)
                 pckv = ca._pack("kv", [ca.k_proj, ca.v_proj])
+                cq_out = ws.cq.view(B * L, ci)
                 cq, ck, cv = ws.cq, ws.ckv[:, :, :ci], ws.ckv[:, :, ci:]
-        if self.pre_norm:
-            if stats_in is None:
-                stats_in = ops.row_stats(x2, self.sa_norm.eps, ws.stats)
-            ops.linear(x2, pq.w, pq.bias, qkv2, colsum=pq.colsum, rowstats=stats_in, ln_eps=self.sa_norm.eps)
-            ops.attention(q, k, v, ws.att, sa.n_heads, sa.scale, self._causal)
-            ops.linear(ws.att.view(M, inner), po.w, po.bias, ws.mid, residual=x2, stats_out=ws.parts_mid)
-            mid, mid_stats = ws.mid, ws.parts_mid
-            if ca is not None:
-                if mid_stats is None:
-                    mid_stats = ops.row_stats(mid, self.ca_norm.eps, ws.stats)
-                if memory3 is None:
-                    ops.linear(mid, pcqkv.w, pcqkv.bias, ws.cqkv.view(M, 3 * ci), colsum=pcqkv.colsum,
-                               rowstats=mid_stats, ln_eps=self.ca_norm.eps)
-                else:
-                    ops.linear(mid, pcq.w, pcq.bias, ws.cq.view(M, ci), colsum=pcq.colsum, rowstats=mid_stats,
-                               ln_eps=self.ca_norm.eps)
+
+            def attend_cross(_catt2: Tensor) -> None:
+                if memory3 is not None:  # the memory is not normalised (transformer.py:98)
                     ops.linear(memory3.view(Mm, d), pckv.w, pckv.bias, ws.ckv.view(Mm, 2 * ci))
                 ops.attention(cq, ck, cv, ws.catt, ca.n_heads, ca.scale)
-                ops.linear(ws.catt.view(M, ci), pco.w, pco.bias, ws.mid2, residual=mid, stats_out=ws.parts_mid2)
-                mid, mid_stats = ws.mid2, ws.parts_mid2
-            if mid_stats is None:
-                mid_stats = ops.row_stats(mid, self.mlp_norm.eps, ws.stats)
-            ops.linear(mid, p1.w, p1.bias, ws.hidden, colsum=p1.colsum, rowstats=mid_stats,
-                       ln_eps=self.mlp_norm.eps, gelu=mlp.gelu_mode)
-            out_stats = ws.parts_out if want_stats else None
-            ops.linear(ws.hidden, p2.w, p2.bias, out2, residual=mid, stats_out=out_stats)
-            return out_stats
-        else:  # post-norm (BERT, GPT): transformer.py:101-103,128-129
-            g1, b1 = norm_vectors(self.sa_norm)
-            g2, b2 = norm_vectors(self.mlp_norm)
-            ops.linear(x2, pq.w, pq.bias, qkv2)
-            ops.attention(q, k, v, ws.att, sa.n_heads, sa.scale, self._causal)
-            ops.linear(ws.att.view(M, inner), po.w, po.bias, ws.tmp, residual=x2)
-            ops.layernorm(ws.tmp, g1, b1, self.sa_norm.eps, ws.mid)
-            mid = ws.mid
-            if ca is not None:
-                gc, bc = norm_vectors(self.ca_norm)
-                if memory3 is None:
-                    ops.linear(mid, pcqkv.w, pcqkv.bias, ws.cqkv.view(M, 3 * ci))
-                else:
-                    ops.linear(mid, pcq.w, pcq.bias, ws.cq.view(M, ci))
-                    ops.linear(memory3.view(Mm, d), pckv.w, pckv.bias, ws.ckv.view(Mm, 2 * ci))
-                ops.attention(cq, ck, cv, ws.catt, ca.n_heads, ca.scale)
-                ops.linear(ws.catt.view(M, ci), pco.w, pco.bias, ws.tmp, residual=mid)
-                ops.layernorm(ws.tmp, gc, bc, self.ca_norm.eps, ws.mid2)
-                mid = ws.mid2
-            ops.linear(mid, p1.w, p1.bias, ws.hidden, gelu=mlp.gelu_mode)
-            ops.linear(ws.hidden, p2.w, p2.bias, ws.tmp, residual=mid)
-            ops.layernorm(ws.tmp, g2, b2, self.mlp_norm.eps, out2)
-        return None
+
+            cross = (pcq, cq_out, attend_cross)
+        return self._launch(x3.view(B * L, d), out3.view(B * L, d), ws, stats_in, want_stats, attend_self, cross)
 
     def step(self, x2: Tensor, out2: Tensor, ws: SimpleNamespace, cache: "KVCache", i: int,
              stats_in: Tensor | None = None, want_stats: bool = False) -> Tensor | None:
         """`run` for one new token per sequence against layer ``i`` of a KV cache: x2 (B, d) -> out2 (B, d).
 
-        The same launches and LayerNorm statistics chain as `run` at L = 1, except that each attention is
-        `ops.attention_decode` over the cache (the self-attention appends this token's k|v row) and the memory's
-        [k; v] projection is not recomputed (it lives in the cache)."""
-        sa, ca, mlp = self.sa, self.ca, self.mlp
-        B, d = x2.shape
+        Each attention is `ops.attention_decode` over the cache (the self-attention appends this token's k|v row); the
+        memory's [k; v] projection is not recomputed (it lives in the cache)."""
+        sa, ca = self.sa, self.ca
+        B = x2.shape[0]
         inner = sa.n_heads * sa.head_dim
-        pq = self._pack_qkv()
-        po = sa._pack("out", [sa.out_proj])
-        p1 = mlp.pack1(self.mlp_norm if self.pre_norm else None)
-        p2 = mlp.pack2()
-        qkv = ws.qkv.view(B, 3 * inner)
-        att = ws.att.view(B, inner)
         kv = cache.kv[i]
 
-        def attend_self() -> None:
+        def attend_self(qkv: Tensor, att: Tensor) -> None:
             ops.attention_decode(qkv[:, :inner], kv[:, :, :inner], kv[:, :, inner:], att, sa.n_heads, sa.scale,
                                  cache.work, k_new=qkv[:, inner:2 * inner], v_new=qkv[:, 2 * inner:],
                                  length=cache.length)
 
+        cross = None
         if ca is not None:
             ci = ca.n_heads * ca.head_dim
-            pco = ca._pack("out", [ca.out_proj])
-            pcq = self._pack_proj(self._pcq, [ca.q_proj], self.ca_norm)
-            cq, catt = ws.cqkv.view(B, 3 * ci)[:, :ci], ws.catt.view(B, ci)
-            mkv = cache.memory_kv[i]
+            cq, mkv = ws.cqkv.view(B, 3 * ci)[:, :ci], cache.memory_kv[i]
 
-            def attend_cross() -> None:
+            def attend_cross(catt: Tensor) -> None:
                 ops.attention_decode(cq, mkv[:, :, :ci], mkv[:, :, ci:], catt, ca.n_heads, ca.scale, cache.work,
                                      Lkv=mkv.shape[1])
 
+            cross = (self._pack_proj(self._pcq, [ca.q_proj], self.ca_norm), cq, attend_cross)
+        return self._launch(x2, out2, ws, stats_in, want_stats, attend_self, cross)
+
+    def _launch(self, x2: Tensor, out2: Tensor, ws: SimpleNamespace, stats_in: Tensor | None, want_stats: bool,
+                attend_self, cross: tuple | None) -> Tensor | None:
+        """The layer's launches on M token rows, x2 (M, d) -> out2 (M, d), for `run` and `step`.
+
+        ``attend_self(qkv, att)`` fills ``ws.att`` from the q|k|v rows in ``ws.qkv``; it is given their (M, ·) views.
+        With cross-attention, ``cross`` is ``(pack, q_out, attend_cross)``: the cross-attention query projection (with
+        ca_norm folded in pre-norm) writes ``q_out``, then ``attend_cross(catt)`` fills ``ws.catt``, given its (M, ·)
+        view."""
+        sa, mlp = self.sa, self.mlp
+        M = x2.shape[0]
+        pq = self._pack_qkv()
+        po = sa._pack("out", [sa.out_proj])
+        p1 = mlp.pack1(self.mlp_norm if self.pre_norm else None)
+        p2 = mlp.pack2()
+        qkv, att = ws.qkv.view(M, -1), ws.att.view(M, -1)
+        if cross is not None:
+            pc, cq, attend_cross = cross
+            pco = self.ca._pack("out", [self.ca.out_proj])
+            catt = ws.catt.view(M, -1)
         if self.pre_norm:
             if stats_in is None:
                 stats_in = ops.row_stats(x2, self.sa_norm.eps, ws.stats)
             ops.linear(x2, pq.w, pq.bias, qkv, colsum=pq.colsum, rowstats=stats_in, ln_eps=self.sa_norm.eps)
-            attend_self()
+            attend_self(qkv, att)
             ops.linear(att, po.w, po.bias, ws.mid, residual=x2, stats_out=ws.parts_mid)
             mid, mid_stats = ws.mid, ws.parts_mid
-            if ca is not None:
+            if cross is not None:
                 if mid_stats is None:
                     mid_stats = ops.row_stats(mid, self.ca_norm.eps, ws.stats)
-                ops.linear(mid, pcq.w, pcq.bias, cq, colsum=pcq.colsum, rowstats=mid_stats, ln_eps=self.ca_norm.eps)
-                attend_cross()
+                ops.linear(mid, pc.w, pc.bias, cq, colsum=pc.colsum, rowstats=mid_stats, ln_eps=self.ca_norm.eps)
+                attend_cross(catt)
                 ops.linear(catt, pco.w, pco.bias, ws.mid2, residual=mid, stats_out=ws.parts_mid2)
                 mid, mid_stats = ws.mid2, ws.parts_mid2
             if mid_stats is None:
@@ -530,17 +501,18 @@ class DecoderLayer(nn.Module):
             out_stats = ws.parts_out if want_stats else None
             ops.linear(ws.hidden, p2.w, p2.bias, out2, residual=mid, stats_out=out_stats)
             return out_stats
+        # post-norm (BERT, GPT): transformer.py:101-103,128-129
         g1, b1 = norm_vectors(self.sa_norm)
         g2, b2 = norm_vectors(self.mlp_norm)
         ops.linear(x2, pq.w, pq.bias, qkv)
-        attend_self()
+        attend_self(qkv, att)
         ops.linear(att, po.w, po.bias, ws.tmp, residual=x2)
         ops.layernorm(ws.tmp, g1, b1, self.sa_norm.eps, ws.mid)
         mid = ws.mid
-        if ca is not None:
+        if cross is not None:
             gc, bc = norm_vectors(self.ca_norm)
-            ops.linear(mid, pcq.w, pcq.bias, cq)
-            attend_cross()
+            ops.linear(mid, pc.w, pc.bias, cq)
+            attend_cross(catt)
             ops.linear(catt, pco.w, pco.bias, ws.tmp, residual=mid)
             ops.layernorm(ws.tmp, gc, bc, self.ca_norm.eps, ws.mid2)
             mid = ws.mid2
@@ -651,13 +623,14 @@ def partial_stats_of(row: Tensor) -> Tensor:
 
 
 def _run_stack(layers: list, x3: Tensor, memory3: Tensor | None, final_stats: bool = False,
-               stats0: Tensor | None = None):
+               stats0: Tensor | None = None, after_layer=None):
     """Run a list of layers over bf16 contiguous (B, L, d) tokens with one shared workspace and two ping-pong output
     buffers; the LayerNorm statistics travel from each layer's last GEMM to the next layer's first.
 
     With ``final_stats`` returns ``(tokens, stats)`` where stats are the partial LayerNorm statistics of the output
     rows (None when the stack cannot produce them) for a LayerNorm folded into whatever consumes the tokens.
-    ``stats0``: partial statistics of x3's rows if its producer wrote them (saves the first layer's row_stats pass)."""
+    ``stats0``: partial statistics of x3's rows if its producer wrote them (saves the first layer's row_stats pass).
+    ``after_layer(i, ws)`` runs after layer ``i``, before the next layer overwrites the workspace."""
     if not layers or x3.numel() == 0:
         return (x3.clone(), None) if final_stats else x3.clone()
     B, L, _ = x3.shape
@@ -667,6 +640,8 @@ def _run_stack(layers: list, x3: Tensor, memory3: Tensor | None, final_stats: bo
     for i, layer in enumerate(layers):
         want = final_stats or i + 1 < len(layers)
         stats = layer.run(cur, bufs[i % 2], ws, stats_in=stats, want_stats=want, memory3=memory3)
+        if after_layer is not None:
+            after_layer(i, ws)
         cur = bufs[i % 2]
     return (cur, stats) if final_stats else cur
 
@@ -732,7 +707,7 @@ class Decoder(nn.ModuleList):
         if self[0].ca is not None:
             if memory is None:
                 # without memory the block attends k = v = q over the current tokens without a mask
-                # (transformer.py:44-45, 413-419 here): every token changes every earlier output
+                # (transformer.py:44-45, `DecoderLayer.run` here): every token changes every earlier output
                 raise NotImplementedError("a cross-attention decoder without memory cannot be decoded incrementally")
             if memory.dim() != 3 or memory.shape[0] != batch or memory.shape[2] != self.d_model or memory.shape[1] < 1:
                 raise ValueError(f"memory {tuple(memory.shape)} does not match (batch={batch}, Lm, d={self.d_model})")
@@ -745,18 +720,14 @@ class Decoder(nn.ModuleList):
         self._check_decodable()
         B, P, _ = x3.shape
         cache.check_prefill(B, P)
-        layers = list(self)
-        ws = layers[0].workspace(B, P, x3.device, 0 if cache.memory3 is None else cache.memory3.shape[1])
-        bufs = [torch.empty_like(x3), torch.empty_like(x3) if len(layers) > 1 else None]
-        cur, stats = x3, None
-        for i, layer in enumerate(layers):
-            stats = layer.run(cur, bufs[i % 2], ws, stats_in=stats, want_stats=True, memory3=cache.memory3)
-            inner = layer.sa.n_heads * layer.sa.head_dim
-            cache.kv[i][:, :P].copy_(ws.qkv[:, :, inner:])
-            cur = bufs[i % 2]
+
+        def keep_kv(i: int, ws: SimpleNamespace) -> None:
+            cache.kv[i][:, :P].copy_(ws.qkv[:, :, ws.qkv.shape[2] // 3:])  # the k|v of the layer's q|k|v rows
+
+        out = _run_stack(list(self), x3, cache.memory3, final_stats=True, after_layer=keep_kv)
         cache.length.fill_(P)
         cache.n = P
-        return cur, stats
+        return out
 
     def step(self, x3: Tensor, cache: "KVCache") -> tuple[Tensor, Tensor | None]:
         """One token per sequence: x3 bf16 contiguous (B, 1, d) at position ``cache.n`` -> (tokens (B, 1, d), partial
@@ -837,45 +808,42 @@ class KVCache:
 
 
 # ----------------------------------------------------------------------------------------------- language-model ends
-def embed_tokens(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor) -> Tensor:
-    """``token_embs(ids) + pos_embs[:L]`` (bert.py:35-36, gpt2.py:22-23, gpt.py:25-26, whisper.py:47-48):
-    (*, L) int64 -> contiguous bf16 (B, L, d) in one gather kernel."""
+def _embedding_tables(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor) -> tuple[Tensor, Tensor]:
+    """Refuse ids that are not on a CUDA device; the token and position tables as contiguous tensors of the one dtype
+    (fp32 or bf16) the gather kernels take."""
     if not ids.is_cuda:
         raise RuntimeError(
             "pytorch_models_b200 runs only on CUDA (sm_100a) tensors; there is no CPU fallback "
             f"(got a {ids.device} tensor)"
         )
-    L = ids.shape[-1]
-    if L > pos_embs.shape[0]:
-        raise ValueError(f"sequence length {L} exceeds the {pos_embs.shape[0]} rows of the position table")
     tok = token_embs.weight.detach()
     pos = pos_embs.detach()
     if tok.dtype not in (torch.float32, torch.bfloat16):
         tok = tok.float()
     if pos.dtype != tok.dtype:
         pos = pos.to(tok.dtype)
+    return tok.contiguous(), pos.contiguous()
+
+
+def embed_tokens(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor) -> Tensor:
+    """``token_embs(ids) + pos_embs[:L]`` (bert.py:35-36, gpt2.py:22-23, gpt.py:25-26, whisper.py:47-48):
+    (*, L) int64 -> contiguous bf16 (B, L, d) in one gather kernel."""
+    tok, pos = _embedding_tables(ids, token_embs, pos_embs)
+    L = ids.shape[-1]
+    if L > pos.shape[0]:
+        raise ValueError(f"sequence length {L} exceeds the {pos.shape[0]} rows of the position table")
     ids2 = ids.reshape(-1, L).to(torch.int64).contiguous()
     out = torch.empty(ids2.shape[0], L, tok.shape[1], device=ids.device, dtype=torch.bfloat16)
-    return ops.embed_rows(ids2, tok.contiguous(), pos.contiguous(), out)
+    return ops.embed_rows(ids2, tok, pos, out)
 
 
 def embed_tokens_at(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor, cache: KVCache) -> Tensor:
     """`embed_tokens` of one new token per sequence at position ``cache.n``: (B,) or (B, 1) int64 -> contiguous bf16
     (B, 1, d). The position is read on the device (the cache length), so the launch is the same at every step."""
-    if not ids.is_cuda:
-        raise RuntimeError(
-            "pytorch_models_b200 runs only on CUDA (sm_100a) tensors; there is no CPU fallback "
-            f"(got a {ids.device} tensor)"
-        )
-    tok = token_embs.weight.detach()
-    pos = pos_embs.detach()
-    if tok.dtype not in (torch.float32, torch.bfloat16):
-        tok = tok.float()
-    if pos.dtype != tok.dtype:
-        pos = pos.to(tok.dtype)
+    tok, pos = _embedding_tables(ids, token_embs, pos_embs)
     ids2 = ids.reshape(-1, 1).to(torch.int64).contiguous()
     out = torch.empty(ids2.shape[0], 1, tok.shape[1], device=ids.device, dtype=torch.bfloat16)
-    return ops.embed_rows_at(ids2, tok.contiguous(), pos.contiguous(), cache.length, out)
+    return ops.embed_rows_at(ids2, tok, pos, cache.length, out)
 
 
 def step_ids_batch(ids: Tensor) -> int:
@@ -929,3 +897,42 @@ class TiedLogits:
                     stats = ops.row_stats(x2, norm.eps, torch.empty(B * L, 2, device=x3.device, dtype=torch.float32))
                 ops.linear(x2, pk.w, pk.bias, out.view(B * L, V8), colsum=pk.colsum, rowstats=stats, ln_eps=norm.eps)
         return out[:, :, :pk.V]
+
+
+class DecoderLM:
+    """What ``GPT2``, ``GPT`` and ``WhisperDecoder`` share: token + position embedding, a `Decoder`, logits against the
+    tied token table, and cached decoding on top of it. Holds no parameters; the model defines ``token_embs``,
+    ``pos_embs``, ``layers`` (the `Decoder`), ``_logits`` (a `TiedLogits`) and, except for GPT, the final ``norm``."""
+
+    def _logits_as(self, h: Tensor, stats: Tensor | None, lead: tuple) -> Tensor:
+        """bf16 tokens (B, L, d) -> logits (*lead, vocab) in the parameters' dtype; ``stats``: partial LayerNorm
+        statistics of h's rows, if its producer wrote them."""
+        logits = self._logits(h, self.token_embs, getattr(self, "norm", None), stats)
+        logits = logits.reshape(*lead, logits.shape[-1])
+        out_dtype = self.token_embs.weight.dtype
+        return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
+
+    # -- incremental decoding (no reference counterpart: the reference recomputes the whole prefix) ----------------
+    def _check_capacity(self, capacity: int) -> None:
+        if capacity > self.pos_embs.shape[0]:
+            raise ValueError(f"capacity {capacity} exceeds the {self.pos_embs.shape[0]} rows of the position table")
+
+    def new_kv_cache(self, batch: int, capacity: int) -> KVCache:
+        """An empty KV cache for ``batch`` sequences of up to ``capacity`` <= max_seq_len tokens (see `prefill`)."""
+        self._check_capacity(capacity)
+        return self.layers.new_kv_cache(batch, capacity)
+
+    def prefill(self, x: Tensor, cache: KVCache) -> Tensor:
+        """`forward` on the prompt, (B, P) or (P,) ids (against the cache's memory for ``WhisperDecoder``), that also
+        fills an empty ``cache``: (*, P, vocab) logits."""
+        cache.check_prefill(x.reshape(-1, x.shape[-1]).shape[0], x.shape[-1])
+        h, stats = self.layers.prefill(embed_tokens(x, self.token_embs, self.pos_embs), cache)
+        return self._logits_as(h, stats, x.shape)
+
+    def step(self, x: Tensor, cache: KVCache) -> Tensor:
+        """The next token of every sequence, (B,) or (B, 1) ids at position ``cache.n`` -> (B, vocab) logits, equal
+        to ``forward(prefix)[:, -1]`` within bf16 rounding. Appends to the cache."""
+        cache.check_step(step_ids_batch(x))
+        self.layers._check_decodable()
+        h, stats = self.layers.step(embed_tokens_at(x, self.token_embs, self.pos_embs, cache), cache)
+        return self._logits_as(h, stats, h.shape[:1])
