@@ -232,6 +232,21 @@ int b200enc_attention_decode(const void* q, long long q_batch_stride, const void
                              int B, int H, int head_dim, float scale, float* workspace, long long workspace_bytes,
                              void* stream);
 
+/*
+ * b200enc_attention_decode in append mode for a ragged batch: sequence b has its own device length lens[b] (B ints),
+ * so the prompts of one batch can hold different numbers of tokens (text/generator.py:11-39 run on several prompts
+ * at once). The keys of sequence b are cache rows [0, lens[b]) plus its new row, which is written to cache row
+ * lens[b]. A lens[b] outside [0, capacity) gives NaN outputs for sequence b only and writes none of its rows. The
+ * chunking, the grid and the workspace are those of b200enc_attention_decode with keys = capacity; work items past a
+ * sequence's own length are skipped, so the K/V bytes read follow the sum of the lengths. With equal lengths the
+ * outputs are bit-identical to b200enc_attention_decode. There is no cross mode: lens must not be NULL.
+ */
+int b200enc_attention_decode_ragged(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
+                                    long long new_batch_stride, void* k_cache, void* v_cache,
+                                    long long cache_batch_stride, int ld_cache, int capacity, const int* lens,
+                                    void* out, long long out_batch_stride, int B, int H, int head_dim, float scale,
+                                    float* workspace, long long workspace_bytes, void* stream);
+
 /* Workspace size in bytes of b200enc_attention_decode (0 for non-positive arguments). Host-only, no device needed. */
 long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys);
 
@@ -243,8 +258,19 @@ long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, i
 int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos, int n_pos,
                           const int* pos0, int dtype, int vocab, int d, void* out, void* stream);
 
+/*
+ * b200enc_embed_rows_at with one device position per sequence of L rows: out[r][:] = bf16(tok[ids[r]][:] +
+ * pos[pos0[r / L] + r % L][:]), pos0 holding rows / L ints. The embedding of a decode step of a ragged batch
+ * (text/gpt2.py:22-23 at each sequence's own position), with pos0 the per-sequence cache lengths.
+ */
+int b200enc_embed_rows_at_ragged(const long long* ids, long long rows, int L, const void* tok, const void* pos,
+                                 int n_pos, const int* pos0, int dtype, int vocab, int d, void* out, void* stream);
+
 /* *len += delta on the device: the last launch of a decode step, so that the captured step can be replayed. */
 int b200enc_decode_advance(int* len, int delta, void* stream);
+
+/* lens[i] += delta for i < n on the device: b200enc_decode_advance for the per-sequence lengths of a ragged batch. */
+int b200enc_decode_advance_ragged(int* lens, int n, int delta, void* stream);
 
 /*
  * Launch plan: a recorded sequence of the entry points above, enqueued by ONE call.

@@ -40,19 +40,13 @@ int launch_pdl(Kern kern, int grid, int threads, cudaStream_t s, Args... args) {
 }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-}  // namespace
 
-extern "C" long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys) {
-  if (B < 1 || H < 1 || head_dim < 1 || keys < 1) return 0;
-  return decode_ws_bytes(B, H, head_dim, keys);
-}
-
-extern "C" int b200enc_attention_decode(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
-                                        long long new_batch_stride, void* k_cache, void* v_cache,
-                                        long long cache_batch_stride, int ld_cache, int capacity, const int* len,
-                                        int Lkv, void* out, long long out_batch_stride, int B, int H, int head_dim,
-                                        float scale, float* workspace, long long workspace_bytes, void* stream) {
-  const char* who = "b200enc_attention_decode";
+// b200enc_attention_decode (len_stride 0) and b200enc_attention_decode_ragged (len_stride 1, append mode only)
+int attention_decode(const char* who, const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
+                     long long new_batch_stride, void* k_cache, void* v_cache, long long cache_batch_stride,
+                     int ld_cache, int capacity, const int* len, int len_stride, int Lkv, void* out,
+                     long long out_batch_stride, int B, int H, int head_dim, float scale, float* workspace,
+                     long long workspace_bytes, void* stream) {
   if (int rc0 = check_abort(who)) return rc0;
   B200_CHECK_ARG(q && k_cache && v_cache && out && workspace, "%s: null pointer (q=%p k_cache=%p v_cache=%p out=%p "
                  "workspace=%p)", who, q, k_cache, v_cache, out, static_cast<void*>(workspace));
@@ -102,6 +96,7 @@ extern "C" int b200enc_attention_decode(const void* q, long long q_batch_stride,
   p.ld_cache = ld_cache;
   p.capacity = capacity;
   p.len = len;
+  p.len_stride = len_stride;
   p.Lkv = append ? 0 : Lkv;
   p.out = static_cast<__nv_bfloat16*>(out);
   p.out_bs = out_batch_stride;
@@ -116,14 +111,15 @@ extern "C" int b200enc_attention_decode(const void* q, long long q_batch_stride,
   const long long slots = (long long)sm_count() * DEC_CTAS_PER_SM;
   const int grid = int(items < slots ? items : slots);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const auto partial = head_dim == 64 ? decode_partial_kernel<8> : decode_partial_kernel<16>;
+  const auto partial = len_stride != 0
+                           ? (head_dim == 64 ? decode_partial_kernel<8, true> : decode_partial_kernel<16, true>)
+                           : (head_dim == 64 ? decode_partial_kernel<8, false> : decode_partial_kernel<16, false>);
   if (int rc = launch_pdl(partial, grid, DEC_THREADS, s, p)) return rc;
   return launch_pdl(decode_combine_kernel, B * H, 128, s, p);
 }
 
-extern "C" int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos,
-                                     int n_pos, const int* pos0, int dtype, int vocab, int d, void* out, void* stream) {
-  const char* who = "b200enc_embed_rows_at";
+int embed_rows_at(const char* who, const long long* ids, long long rows, int L, const void* tok, const void* pos,
+                  int n_pos, const int* pos0, int pos0_stride, int dtype, int vocab, int d, void* out, void* stream) {
   B200_CHECK_ARG(ids && tok && pos && pos0 && out, "%s: null pointer", who);
   B200_CHECK_ARG(rows >= 1 && L >= 1 && rows % L == 0, "%s: rows=%lld must be a positive multiple of L=%d", who, rows,
                  L);
@@ -136,18 +132,70 @@ extern "C" int b200enc_embed_rows_at(const long long* ids, long long rows, int L
   __nv_bfloat16* dst = static_cast<__nv_bfloat16*>(out);
   if (dtype == B200ENC_DTYPE_BF16)
     embed_rows_at_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(ids, rows, L, static_cast<const __nv_bfloat16*>(tok),
-                                                             static_cast<const __nv_bfloat16*>(pos), n_pos, pos0, vocab,
-                                                             d, dst);
+                                                             static_cast<const __nv_bfloat16*>(pos), n_pos, pos0,
+                                                             pos0_stride, vocab, d, dst);
   else if (dtype == B200ENC_DTYPE_F32)
     embed_rows_at_kernel<float><<<grid, 256, 0, s>>>(ids, rows, L, static_cast<const float*>(tok),
-                                                     static_cast<const float*>(pos), n_pos, pos0, vocab, d, dst);
+                                                     static_cast<const float*>(pos), n_pos, pos0, pos0_stride, vocab,
+                                                     d, dst);
   else
     return set_error(-1, "%s: unsupported dtype %d", who, dtype);
   B200_CUDA(cudaGetLastError());
   return 0;
 }
 
+int decode_advance(const char* who, int* len, int n, int delta, void* stream) {
+  B200_CHECK_ARG(len != nullptr, "%s: null len", who);
+  B200_CHECK_ARG(n >= 1, "%s: n=%d must be >= 1", who, n);
+  const int threads = n < 256 ? n : 256;
+  return launch_pdl(decode_advance_kernel, 1, threads, static_cast<cudaStream_t>(stream), len, n, delta);
+}
+}  // namespace
+
+extern "C" long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys) {
+  if (B < 1 || H < 1 || head_dim < 1 || keys < 1) return 0;
+  return decode_ws_bytes(B, H, head_dim, keys);
+}
+
+extern "C" int b200enc_attention_decode(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
+                                        long long new_batch_stride, void* k_cache, void* v_cache,
+                                        long long cache_batch_stride, int ld_cache, int capacity, const int* len,
+                                        int Lkv, void* out, long long out_batch_stride, int B, int H, int head_dim,
+                                        float scale, float* workspace, long long workspace_bytes, void* stream) {
+  return attention_decode("b200enc_attention_decode", q, q_batch_stride, k_new, v_new, new_batch_stride, k_cache,
+                          v_cache, cache_batch_stride, ld_cache, capacity, len, 0, Lkv, out, out_batch_stride, B, H,
+                          head_dim, scale, workspace, workspace_bytes, stream);
+}
+
+extern "C" int b200enc_attention_decode_ragged(const void* q, long long q_batch_stride, const void* k_new,
+                                               const void* v_new, long long new_batch_stride, void* k_cache,
+                                               void* v_cache, long long cache_batch_stride, int ld_cache, int capacity,
+                                               const int* lens, void* out, long long out_batch_stride, int B, int H,
+                                               int head_dim, float scale, float* workspace, long long workspace_bytes,
+                                               void* stream) {
+  const char* who = "b200enc_attention_decode_ragged";
+  B200_CHECK_ARG(lens != nullptr, "%s: lens=(nil): per-sequence lengths are append mode only", who);
+  return attention_decode(who, q, q_batch_stride, k_new, v_new, new_batch_stride, k_cache, v_cache,
+                          cache_batch_stride, ld_cache, capacity, lens, 1, 0, out, out_batch_stride, B, H, head_dim,
+                          scale, workspace, workspace_bytes, stream);
+}
+
+extern "C" int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos,
+                                     int n_pos, const int* pos0, int dtype, int vocab, int d, void* out, void* stream) {
+  return embed_rows_at("b200enc_embed_rows_at", ids, rows, L, tok, pos, n_pos, pos0, 0, dtype, vocab, d, out, stream);
+}
+
+extern "C" int b200enc_embed_rows_at_ragged(const long long* ids, long long rows, int L, const void* tok,
+                                            const void* pos, int n_pos, const int* pos0, int dtype, int vocab, int d,
+                                            void* out, void* stream) {
+  return embed_rows_at("b200enc_embed_rows_at_ragged", ids, rows, L, tok, pos, n_pos, pos0, 1, dtype, vocab, d, out,
+                       stream);
+}
+
 extern "C" int b200enc_decode_advance(int* len, int delta, void* stream) {
-  B200_CHECK_ARG(len != nullptr, "b200enc_decode_advance: null len");
-  return launch_pdl(decode_advance_kernel, 1, 1, static_cast<cudaStream_t>(stream), len, delta);
+  return decode_advance("b200enc_decode_advance", len, 1, delta, stream);
+}
+
+extern "C" int b200enc_decode_advance_ragged(int* lens, int n, int delta, void* stream) {
+  return decode_advance("b200enc_decode_advance_ragged", lens, n, delta, stream);
 }

@@ -14,11 +14,21 @@
 //   decode_combine_kernel  one CTA per (b, h): merges the chunk partials in chunk order (fixed order: bit-identical
 //                          repeats) and writes bf16 out.
 //
-// Append mode (len != nullptr): the keys are cache rows [0, len) plus the new row, which is read from the QKV GEMM's
-// output (k_new / v_new) instead of the cache; the one CTA whose chunk holds key `len` also copies the new row into
-// cache row `len`. No CTA reads a row that another CTA of the launch writes. `len` is read on the device, and the grid
-// and the chunk size depend only on (B, H, head_dim, capacity), so a decode step's launch arguments do not change from
-// one step to the next (CUDA-graph replay). A length outside [0, capacity) writes NaN outputs and touches no cache row.
+// Append mode (len != nullptr): the keys of sequence b are cache rows [0, len_b) plus the new row, which is read from
+// the QKV GEMM's output (k_new / v_new) instead of the cache; the one CTA whose chunk holds key `len_b` also copies the
+// new row into cache row `len_b`. No CTA reads a row that another CTA of the launch writes. The lengths are read on the
+// device, and the grid and the chunk size depend only on (B, H, head_dim, capacity), so a decode step's launch
+// arguments do not change from one step to the next (CUDA-graph replay). A sequence whose length is outside
+// [0, capacity) gets NaN outputs and touches no cache row; the other sequences of the launch are unaffected.
+//   len_stride 0: one length `len[0]` shared by the batch.
+//   len_stride 1: per-sequence lengths `len[b]` (a ragged batch). Sequence b has nch_b = ceil(keys_b / kc) chunks;
+//     the items are numbered densely in (b, h, chunk) order, H·nch_b per sequence, and every CTA reduces the lengths
+//     to the item count H·Σ nch_b. A CTA's items increase, so it finds each item's sequence by advancing a cursor over
+//     the sequences (B length reads per CTA in all). Only real items are enumerated, so the grid stride spreads them as
+//     evenly over the CTAs as the shared-length launch does, and the K/V bytes read follow the sum of the lengths, not
+//     B times the longest. With equal lengths the numbering is the shared-length one: every item does the same
+//     arithmetic (bit-identical outputs). The ragged enumeration is its own instantiation (kRagged), so the
+//     shared-length one keeps its direct item -> (b, h, chunk) division.
 // Cross mode (len == nullptr): keys [0, Lkv) of a read-only cache.
 #pragma once
 #include "ptx.cuh"
@@ -43,7 +53,8 @@ struct DecodeParams {
   long long cache_bs;
   long long ld_cache;
   int capacity;
-  const int* len;              // device length (append mode) or nullptr (cross mode: Lkv keys)
+  const int* len;              // device length(s) (append mode) or nullptr (cross mode: Lkv keys)
+  int len_stride;              // 0: len[0] for every sequence, 1: len[b] for sequence b
   int Lkv;
   __nv_bfloat16* out;          // [B] rows, batch stride out_bs
   long long out_bs;
@@ -54,10 +65,10 @@ struct DecodeParams {
   float* ws;                   // [B*H][max_chunks][head_dim + 2] fp32
 };
 
-// number of keys of this launch, or -1 if the device length is out of range
-__device__ __forceinline__ int decode_keys(const DecodeParams& p) {
+// number of keys of sequence b, or -1 if its device length is out of range
+__device__ __forceinline__ int decode_keys(const DecodeParams& p, int b) {
   if (p.len == nullptr) return p.Lkv;
-  const int n = *p.len;
+  const int n = p.len[b * p.len_stride];
   return (n >= 0 && n < p.capacity) ? n + 1 : -1;
 }
 
@@ -73,24 +84,54 @@ __device__ __forceinline__ void dec_unpack(uint4 w, float (&f)[8]) {
 }
 
 // kLanes = lanes per key (8: head_dim 64, 16: head_dim 80-128); lanes c >= head_dim / 8 of a group idle.
-template <int kLanes>
+// kRagged: per-sequence lengths (len_stride 1), else one length or Lkv for the whole batch.
+template <int kLanes, bool kRagged>
 __global__ void __launch_bounds__(DEC_THREADS, DEC_CTAS_PER_SM) decode_partial_kernel(const DecodeParams p) {
   constexpr int kGroups = 32 / kLanes;
   __shared__ float sm_ml[DEC_WARPS][2];
   __shared__ float sm_o[DEC_WARPS][128];
+  __shared__ int sm_chunks[DEC_WARPS];
   griddep_wait();  // the previous kernel (the QKV GEMM) wrote q and the new k / v row
-  const int n_keys = decode_keys(p);
-  if (n_keys < 0) return;  // the combine kernel writes NaN
+  int n_keys = decode_keys(p, 0);
+  if (!kRagged && n_keys < 0) return;  // the combine kernel writes NaN
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  // chunks of a sequence: 0 when its length is out of range (the combine kernel writes its NaN)
+  auto chunks = [&](int keys) { return keys < 0 ? 0 : (keys + p.kc - 1) / p.kc; };
+  int nch = chunks(n_keys), total = p.B * nch;
+  if constexpr (kRagged) {
+    total = 0;
+    for (int b = threadIdx.x; b < p.B; b += DEC_THREADS) total += chunks(decode_keys(p, b));
+    total = __reduce_add_sync(0xffffffffu, total);
+    if (lane == 0) sm_chunks[warp] = total;
+    __syncthreads();
+    total = 0;
+#pragma unroll
+    for (int w = 0; w < DEC_WARPS; ++w) total += sm_chunks[w];
+  }
   const int grp = lane / kLanes, c = lane % kLanes;
   const int hd = p.head_dim;
   const bool col_ok = c < (hd >> 3);
-  const int nch = (n_keys + p.kc - 1) / p.kc;
-  const int n_items = p.B * p.H * nch;
-  const int new_row = p.len != nullptr ? n_keys - 1 : -1;
+  const int n_items = p.H * total;
+  int b = 0, first = 0;                 // ragged: the items of sequence b start at `first`
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-    const int bh = item / nch, chunk = item - bh * nch;
-    const int b = bh / p.H, h = bh - b * p.H;
+    int bh, h, chunk;
+    if constexpr (kRagged) {
+      while (item >= first + p.H * nch) {  // a later sequence (CTA-uniform; skips sequences without items)
+        first += p.H * nch;
+        n_keys = decode_keys(p, ++b);
+        nch = chunks(n_keys);
+      }
+      const int local = item - first;
+      h = local / nch;
+      chunk = local - h * nch;
+      bh = b * p.H + h;
+    } else {
+      bh = item / nch;
+      chunk = item - bh * nch;
+      b = bh / p.H;
+      h = bh - b * p.H;
+    }
+    const int new_row = p.len != nullptr ? n_keys - 1 : -1;
     const long long col = (long long)h * hd + 8 * c;
     float qf[8];
     {
@@ -205,7 +246,7 @@ __global__ void __launch_bounds__(128) decode_combine_kernel(const DecodeParams 
   if (t >= hd) return;
   const int b = bh / p.H, h = bh - b * p.H;
   __nv_bfloat16* dst = p.out + b * p.out_bs + (long long)h * hd + t;
-  const int n_keys = decode_keys(p);
+  const int n_keys = decode_keys(p, b);
   if (n_keys < 0) {
     *dst = __float2bfloat16_rn(__int_as_float(0x7fc00000));
     return;
@@ -224,20 +265,21 @@ __global__ void __launch_bounds__(128) decode_combine_kernel(const DecodeParams 
   *dst = __float2bfloat16_rn(o / l);
 }
 
-// out[r] = bf16(tok[ids[r]] + pos[*pos0 + r % L]): the embedding of a decode step, whose position is the cache length
-// on the device. An id outside [0, vocab) or a position outside [0, n_pos) gives a NaN row.
+// out[r] = bf16(tok[ids[r]] + pos[pos0[(r / L) * pos0_stride] + r % L]): the embedding of a decode step, whose
+// position is the cache length on the device (pos0_stride 0: one length for all rows, 1: one per sequence of L rows).
+// An id outside [0, vocab) or a position outside [0, n_pos) gives a NaN row.
 template <typename TIn>
 __global__ void __launch_bounds__(256)
 embed_rows_at_kernel(const long long* __restrict__ ids, long long rows, int L, const TIn* __restrict__ tok,
-                     const TIn* __restrict__ pos, int n_pos, const int* __restrict__ pos0, int vocab, int d,
-                     __nv_bfloat16* __restrict__ out) {
+                     const TIn* __restrict__ pos, int n_pos, const int* __restrict__ pos0, int pos0_stride, int vocab,
+                     int d, __nv_bfloat16* __restrict__ out) {
   const int vec_per_row = d >> 3;
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= rows * vec_per_row) return;
   const long long r = t / vec_per_row;
   const int c = int(t % vec_per_row) * 8;
   const long long id = ids[r];
-  const long long pr = (long long)*pos0 + r % L;
+  const long long pr = (long long)pos0[(r / L) * pos0_stride] + r % L;
   const bool ok = id >= 0 && id < vocab && pr >= 0 && pr < n_pos;
   const TIn* trow = tok + (ok ? id : 0) * (long long)d + c;
   const TIn* prow = pos + (ok ? pr : 0) * (long long)d + c;
@@ -251,10 +293,10 @@ embed_rows_at_kernel(const long long* __restrict__ ids, long long rows, int L, c
   *reinterpret_cast<uint4*>(out + r * d + c) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
 }
 
-// *len += delta: the last launch of a decode step
-__global__ void decode_advance_kernel(int* len, int delta) {
+// len[i] += delta for i < n: the last launch of a decode step (n = 1 shared length, or one per sequence)
+__global__ void decode_advance_kernel(int* len, int n, int delta) {
   griddep_wait();
-  *len += delta;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) len[i] += delta;
 }
 
 }  // namespace b200

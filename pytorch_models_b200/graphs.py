@@ -65,6 +65,10 @@ class GraphedStep:
     A step's launches read the position from the cache's device-side length and advance it on the device, so one
     captured graph serves every position. Capture runs warm-up steps (which write the rows past the current length and
     advance it) and then restores the cache's length, so the cache is left as it was found. ``ids``: (B,) or (B, 1).
+
+    The graph reads the length tensor the cache used at capture: the shared length, or the per-sequence lengths of a
+    ragged fill (`KVCache.seq_lengths`). Replay is refused once the cache has switched to the other kind (``reset()``
+    and a prefill with or without ``lengths``); capture again then.
     """
 
     def __init__(self, model: nn.Module, cache, warmup: int = 2) -> None:
@@ -76,6 +80,7 @@ class GraphedStep:
     def capture(self, warmup: int = 2) -> None:
         cache = self.cache
         cache.check_step(cache.batch)  # the warm-up needs at least one free row
+        self.length = cache.length  # the tensor the captured launches read and advance
         saved_len, saved_n = cache.length.clone(), cache.n
         side = torch.cuda.Stream(cache.length.device)
         side.wait_stream(torch.cuda.current_stream())
@@ -97,6 +102,10 @@ class GraphedStep:
     @torch.no_grad()
     def __call__(self, ids: Tensor) -> Tensor:
         self.cache.check_step(step_ids_batch(ids))
+        if self.cache.length is not self.length:
+            kind = "per-sequence" if self.cache.ragged else "shared"
+            raise ValueError(f"the cache now holds {kind} lengths, not the kind it held when this step was captured; "
+                             "capture a new GraphedStep")
         self.static_ids.copy_(ids.reshape(-1, 1), non_blocking=True)
         self.graph.replay()
         self.cache.n += 1

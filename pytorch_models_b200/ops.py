@@ -433,6 +433,16 @@ def whisper_logmel(audio: Tensor, filters_t: Tensor, out: Tensor) -> Tensor:
     return out
 
 
+def _per_sequence(length: Tensor | None, B: int, name: str) -> bool:
+    """True if a device length tensor holds one length per sequence (B > 1 elements), False if it holds one shared
+    length; anything else is refused."""
+    if length is None or length.numel() == 1:
+        return False
+    if length.dim() != 1 or length.numel() != B or not length.is_contiguous():
+        raise ValueError(f"{name} must be a contiguous int32 tensor of 1 or {B} elements, got {tuple(length.shape)}")
+    return True
+
+
 def decode_workspace_bytes(B: int, n_heads: int, head_dim: int, keys: int) -> int:
     """Bytes of fp32 workspace `attention_decode` needs (keys = cache capacity, or Lkv in cross mode)."""
     return int(_lib.load().b200enc_attention_decode_workspace_bytes(B, n_heads, head_dim, keys))
@@ -447,7 +457,8 @@ def attention_decode(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n
     workspace: fp32, at least `decode_workspace_bytes` bytes.
     Append mode (``length`` = int32 device tensor of one element): attends over cache rows [0, length) plus the new row
     ``k_new`` / ``v_new`` ((B, H*hd) views) and writes the new row into cache row ``length``; ``length`` itself is not
-    changed (`decode_advance`). Cross mode (``length`` None): attends over cache rows [0, Lkv)."""
+    changed (`decode_advance`). A ``length`` of B elements gives each sequence its own length (a ragged batch,
+    ``b200enc_attention_decode_ragged``). Cross mode (``length`` None): attends over cache rows [0, Lkv)."""
     dev = _need_cuda(q, k_cache, v_cache, out, workspace, k_new, v_new, length)
     for name, t in (("q", q), ("k_cache", k_cache), ("v_cache", v_cache), ("out", out), ("k_new", k_new),
                     ("v_new", v_new)):
@@ -471,6 +482,15 @@ def attention_decode(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n
         new_bs = k_new.stride(0)
     if not workspace.is_contiguous():
         raise ValueError("workspace must be contiguous")
+    if _per_sequence(length, B, "length"):
+        _call(
+            "b200enc_attention_decode_ragged", dict(B=B, H=n_heads, keys=k_cache.shape[1], append=True), dev,
+            q.data_ptr(), q.stride(0), k_new.data_ptr(), v_new.data_ptr(), new_bs, k_cache.data_ptr(),
+            v_cache.data_ptr(), k_cache.stride(0), k_cache.stride(1), k_cache.shape[1], length.data_ptr(),
+            out.data_ptr(), out.stride(0), B, n_heads, D // n_heads, float(scale), workspace.data_ptr(),
+            workspace.numel() * 4,
+        )
+        return out
     _call(
         "b200enc_attention_decode", dict(B=B, H=n_heads, keys=k_cache.shape[1], append=length is not None), dev,
         q.data_ptr(), q.stride(0), _ptr(k_new), _ptr(v_new), new_bs, k_cache.data_ptr(), v_cache.data_ptr(),
@@ -482,14 +502,16 @@ def attention_decode(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n
 
 def embed_rows_at(ids: Tensor, tok: Tensor, pos: Tensor, pos0: Tensor, out: Tensor) -> Tensor:
     """`embed_rows` at a device-side position: out[b, l] = tok[ids[b, l]] + pos[pos0 + l] with ``pos0`` an int32 device
-    tensor of one element (a decode step's cache length). A position past the table gives a NaN row."""
+    tensor of one element (a decode step's cache length), or of B elements, pos0[b] for sequence b (a ragged batch).
+    A position past the table gives a NaN row."""
     dev = _need_cuda(ids, tok, pos, pos0, out)
     _need(pos0, torch.int32, "pos0")
     dt = _embed_args("embed_rows_at", ids, tok, pos, out)
     B, L = ids.shape
     vocab, d = tok.shape
+    name = "b200enc_embed_rows_at_ragged" if _per_sequence(pos0, B, "pos0") else "b200enc_embed_rows_at"
     _call(
-        "b200enc_embed_rows_at", dict(rows=B * L, d=d), dev,
+        name, dict(rows=B * L, d=d), dev,
         ids.data_ptr(), B * L, L, tok.data_ptr(), pos.data_ptr(), pos.shape[0], pos0.data_ptr(), dt, vocab, d,
         out.data_ptr(),
     )
@@ -497,8 +519,13 @@ def embed_rows_at(ids: Tensor, tok: Tensor, pos: Tensor, pos0: Tensor, out: Tens
 
 
 def decode_advance(length: Tensor, delta: int = 1) -> Tensor:
-    """length += delta on the device (int32, one element): issued at the end of a decode step's decoder stack."""
+    """length += delta on the device (int32, one element, or one per sequence of a ragged batch): issued at the end of
+    a decode step's decoder stack."""
     dev = _need_cuda(length)
     _need(length, torch.int32, "length")
-    _call("b200enc_decode_advance", dict(delta=delta), dev, length.data_ptr(), int(delta))
+    n = length.numel()
+    if _per_sequence(length, n, "length"):
+        _call("b200enc_decode_advance_ragged", dict(n=n, delta=delta), dev, length.data_ptr(), n, int(delta))
+    else:
+        _call("b200enc_decode_advance", dict(delta=delta), dev, length.data_ptr(), int(delta))
     return length

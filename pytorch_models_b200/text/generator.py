@@ -24,6 +24,16 @@ def _pick(last_logits: Tensor, topk: int) -> int:
     return int(ids[choice])
 
 
+def _pick_rows(logits: Tensor, topk: int) -> Tensor:
+    """`_pick` for every row of (B, vocab) logits at once -> (B,) int64 device tensor, without a host synchronisation."""
+    scores = logits.float()
+    if topk <= 1:
+        return scores.argmax(dim=-1)
+    best, ids = scores.topk(topk, dim=-1)
+    choice = torch.multinomial(torch.softmax(best, dim=-1), num_samples=1)
+    return ids.gather(1, choice)[:, 0]
+
+
 class DecoderGenerator:
     def __init__(self, model: nn.Module, tokenizer) -> None:
         self.model = model
@@ -46,6 +56,42 @@ class DecoderGenerator:
             if ids[-1] == eos:
                 break
         return self.tokenizer.decode(ids)
+
+    @torch.inference_mode()
+    def generate_batch(self, prompts: list[str], max_tokens: int = 100, topk: int = 1) -> list[str]:
+        """`generate` (``use_cache=True``) for several prompts of any lengths at once: one ragged prefill of the
+        right-padded prompts (``model.prefill(..., lengths=...)``), then one CUDA-graph replay of ``model.step`` per
+        token for the whole batch, with one host synchronisation per step to read the picked tokens. Each sequence
+        stops at its own EOS (the batch keeps stepping; its later tokens are dropped) or after ``max_tokens`` new
+        tokens. Returns one string per prompt, what ``generate(prompt, max_tokens, topk, use_cache=True)`` returns up
+        to bf16 rounding (see `generate`)."""
+        device = next(self.model.parameters()).device
+        eos = self.tokenizer.eos_token_id
+        seqs = [list(self.tokenizer.encode(p)) for p in prompts]
+        if not seqs or max_tokens <= 0:
+            return [self.tokenizer.decode(s) for s in seqs]
+        lengths = [len(s) for s in seqs]
+        P = max(lengths)
+        ids = torch.zeros(len(seqs), P, dtype=torch.long)
+        for b, s in enumerate(seqs):
+            ids[b, :len(s)] = torch.tensor(s, dtype=torch.long)
+        cache = self.model.new_kv_cache(len(seqs), min(self.model.max_seq_len, P + max_tokens))
+        logits = self.model.prefill(ids.to(device), cache, lengths=lengths)
+        last = logits[torch.arange(len(seqs), device=device), torch.tensor(lengths, device=device) - 1]
+        done = [False] * len(seqs)
+        step = None
+        for i in range(max_tokens):
+            picked = _pick_rows(last, topk)
+            for b, t in enumerate(picked.tolist()):
+                if not done[b]:
+                    seqs[b].append(t)
+                    done[b] = t == eos
+            if all(done) or i + 1 == max_tokens:
+                break
+            if step is None:
+                step = GraphedStep(self.model, cache)
+            last = step(picked)
+        return [self.tokenizer.decode(s) for s in seqs]
 
     def _generate_cached(self, ids: list, max_tokens: int, topk: int, eos, device) -> list:
         cache = self.model.new_kv_cache(1, min(self.model.max_seq_len, len(ids) + max_tokens))

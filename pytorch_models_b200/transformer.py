@@ -714,19 +714,24 @@ class Decoder(nn.ModuleList):
             m3, _ = _as_tokens(memory, self.d_model)
         return KVCache(self, batch, capacity, m3)
 
-    def prefill(self, x3: Tensor, cache: "KVCache") -> tuple[Tensor, Tensor | None]:
+    def prefill(self, x3: Tensor, cache: "KVCache", lengths=None) -> tuple[Tensor, Tensor | None]:
         """`run` (``final_stats=True``) on the first P tokens of an EMPTY cache, keeping every layer's k|v rows in it:
-        x3 bf16 contiguous (B, P, d) -> (tokens, partial statistics or None). Sets the cache length to P."""
+        x3 bf16 contiguous (B, P, d) -> (tokens, partial statistics or None). Sets the cache length to P.
+
+        ``lengths``: B host ints in [1, P] for a ragged batch of right-padded sequences; sequence b then holds
+        ``lengths[b]`` tokens. Causal attention keeps every real token away from the padding rows after it, so the
+        stack runs unchanged; the padding rows' k|v land in cache rows at or past each sequence's length, which no step
+        reads and the steps overwrite. The output rows of padding positions are not meaningful."""
         self._check_decodable()
         B, P, _ = x3.shape
         cache.check_prefill(B, P)
+        lengths = cache.check_lengths(lengths, P)
 
         def keep_kv(i: int, ws: SimpleNamespace) -> None:
             cache.kv[i][:, :P].copy_(ws.qkv[:, :, ws.qkv.shape[2] // 3:])  # the k|v of the layer's q|k|v rows
 
         out = _run_stack(list(self), x3, cache.memory3, final_stats=True, after_layer=keep_kv)
-        cache.length.fill_(P)
-        cache.n = P
+        cache.set_lengths(P, lengths)
         return out
 
     def step(self, x3: Tensor, cache: "KVCache") -> tuple[Tensor, Tensor | None]:
@@ -756,8 +761,11 @@ class KVCache:
     length the decode kernels read and the step advances; ``n`` is its host mirror, used for the argument checks. Also
     holds the step's scratch buffers and the fp32 workspace of the decode kernel.
 
-    All sequences of a batch have the same length. A cache is valid for the weights it was filled with: after changing
-    the model's parameters, start a new cache (this is not detected)."""
+    All sequences of a batch have the same length, unless the cache was filled by a ragged prefill (``lengths``): then
+    ``length`` is the cache's (batch,) int32 tensor of per-sequence lengths, which the step's launches read and advance
+    instead; ``n`` is the longest sequence's length and ``pad[b]`` how many tokens sequence b is shorter, fixed for the
+    whole fill. `seq_lengths` reads the per-sequence lengths on the host. A cache is valid for the weights it was
+    filled with: after changing the model's parameters, start a new cache (this is not detected)."""
 
     def __init__(self, decoder: Decoder, batch: int, capacity: int, memory3: Tensor | None) -> None:
         layers = list(decoder)
@@ -765,7 +773,11 @@ class KVCache:
         dev = p.device
         self.batch, self.capacity = batch, capacity
         self.n = 0
-        self.length = torch.zeros(1, device=dev, dtype=torch.int32)
+        self.pad = None
+        self.shared_length = torch.zeros(1, device=dev, dtype=torch.int32)
+        # allocated once, so that a step captured on a ragged fill keeps reading the same tensor after later fills
+        self.seq_length = torch.zeros(batch, device=dev, dtype=torch.int32)
+        self.length = self.shared_length
         self.memory3 = memory3
         e = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)  # noqa: E731
         self.kv = [e(batch, capacity, 2 * layer.sa.n_heads * layer.sa.head_dim) for layer in layers]
@@ -789,8 +801,49 @@ class KVCache:
 
     def reset(self) -> None:
         """Empty the cache (for a new prefill); the buffers are kept."""
+        self.length = self.shared_length
         self.length.zero_()
         self.n = 0
+        self.pad = None
+
+    @property
+    def ragged(self) -> bool:
+        """True when the sequences have their own lengths (the cache was filled by a prefill with ``lengths``)."""
+        return self.pad is not None
+
+    @property
+    def seq_lengths(self) -> list[int]:
+        """The number of tokens each sequence holds, from the host mirror (no device synchronisation)."""
+        return [self.n] * self.batch if self.pad is None else [self.n - p for p in self.pad]
+
+    def check_lengths(self, lengths, P: int) -> list[int] | None:
+        """Validate the ``lengths`` of a ragged prefill of P tokens per row: None, or B host ints in [1, P]."""
+        if lengths is None:
+            return None
+        if isinstance(lengths, Tensor):
+            if lengths.is_cuda:
+                raise ValueError("lengths must be host ints (a list or a CPU tensor), not a CUDA tensor: the checks "
+                                 "and the host mirror of the cache need them without a device synchronisation")
+            lengths = lengths.reshape(-1).tolist()
+        lengths = [int(n) for n in lengths]
+        if len(lengths) != self.batch:
+            raise ValueError(f"lengths has {len(lengths)} entries for a batch of {self.batch}")
+        bad = [n for n in lengths if not 1 <= n <= P]
+        if bad:
+            raise ValueError(f"length {bad[0]} is outside [1, {P}] (the prompts are right-padded to {P} tokens)")
+        return lengths
+
+    def set_lengths(self, P: int, lengths: list[int] | None) -> None:
+        """After a prefill of P tokens per row: every sequence holds P tokens, or ``lengths[b]`` (ragged)."""
+        if lengths is None:
+            self.length = self.shared_length
+            self.length.fill_(P)
+            self.pad = None
+        else:
+            self.length = self.seq_length
+            self.length.copy_(torch.tensor(lengths, dtype=torch.int32))
+            self.pad = [P - n for n in lengths]
+        self.n = P
 
     def check_prefill(self, batch: int, P: int) -> None:
         if batch != self.batch:
@@ -922,11 +975,21 @@ class DecoderLM:
         self._check_capacity(capacity)
         return self.layers.new_kv_cache(batch, capacity)
 
-    def prefill(self, x: Tensor, cache: KVCache) -> Tensor:
+    def prefill(self, x: Tensor, cache: KVCache, lengths=None) -> Tensor:
         """`forward` on the prompt, (B, P) or (P,) ids (against the cache's memory for ``WhisperDecoder``), that also
-        fills an empty ``cache``: (*, P, vocab) logits."""
-        cache.check_prefill(x.reshape(-1, x.shape[-1]).shape[0], x.shape[-1])
-        h, stats = self.layers.prefill(embed_tokens(x, self.token_embs, self.pos_embs), cache)
+        fills an empty ``cache``: (*, P, vocab) logits.
+
+        ``lengths``: B host ints in [1, P] (a list or a CPU tensor) for prompts of different lengths, right-padded to P
+        tokens; prompt b is ``x[b, :lengths[b]]``, and the steps then continue each sequence at its own position. The
+        padding ids are replaced by a valid id before the embedding; the logits of padding positions are not
+        meaningful (those of prompt b's last token are at ``lengths[b] - 1``)."""
+        P = x.shape[-1]
+        cache.check_prefill(x.reshape(-1, P).shape[0], P)
+        lengths = cache.check_lengths(lengths, P)
+        if lengths is not None:
+            pad = torch.arange(P)[None, :] >= torch.tensor(lengths)[:, None]
+            x = x.masked_fill(pad.reshape(x.shape).to(x.device), 0)
+        h, stats = self.layers.prefill(embed_tokens(x, self.token_embs, self.pos_embs), cache, lengths)
         return self._logits_as(h, stats, x.shape)
 
     def step(self, x: Tensor, cache: KVCache) -> Tensor:
