@@ -266,6 +266,39 @@ int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const voi
 int b200enc_embed_rows_at_ragged(const long long* ids, long long rows, int L, const void* tok, const void* pos,
                                  int n_pos, const int* pos0, int dtype, int vocab, int d, void* out, void* stream);
 
+/*
+ * Extending a filled KV cache by P rows per sequence (multi-turn continuation, chunked prefill): causal attention whose
+ * queries start at each sequence's cache length ("bottom-right aligned").
+ *
+ *   out[b][i][hd*h + :] = softmax_{j <= n_b + i}( q[b][i][hd*h + :] . k[b][j][hd*h + :] * scale ) v[b][j][hd*h + :]
+ *
+ * with n_b = lens[b * len_stride] the device cache length of sequence b (len_stride 0: one length for the batch,
+ * 1: one per sequence) and i < P. Replaces F.scaled_dot_product_attention at transformer.py:52 for the causal
+ * self-attention of DecoderLayer (transformer.py:97) when the keys and values of the first n_b positions come from a
+ * cache: the P query rows see the cached keys and the new ones up to their own position. The new rows' k|v must
+ * already be in cache rows [n_b, n_b + P) (b200enc_kv_append), so every key is read from the cache. q, out: P rows
+ * per sequence as in b200enc_attention; k_cache / v_cache: [B][capacity] rows of row stride ld_cache and batch stride
+ * cache_batch_stride (the K and V halves of one k|v buffer). head_dim 64 or 80-128 (the streaming kernels of
+ * b200enc_attention with the causal diagonal shifted by n_b). Only the K/V blocks below row n_b + P are read, so a
+ * ragged batch costs what its own lengths cost. The lengths are read on the device; P <= capacity is checked here and
+ * n_b + P <= capacity is the caller's (a sequence whose n_b is outside [0, capacity - P] gets NaN outputs).
+ * With n_b = 0 the result is bit-identical to b200enc_attention with B200ENC_ATTN_CAUSAL on the same rows.
+ */
+int b200enc_attention_extend(const void* q, long long q_batch_stride, int ldq, const void* k_cache, const void* v_cache,
+                             long long cache_batch_stride, int ld_cache, int capacity, const int* lens, int len_stride,
+                             void* out, long long out_batch_stride, int ldo, int B, int H, int P, int head_dim,
+                             float scale, void* stream);
+
+/*
+ * cache[b][n_b + r][:width] = src[b][r][:width] for r < P, n_b = lens[b * len_stride] on the device: writes the k|v
+ * rows of the fused q|k|v projection (transformer.py:47-49) into a KV cache at each sequence's length, ahead of
+ * b200enc_attention_extend. bf16, strides in elements, rows 16-byte aligned, width % 8 == 0. A row that would land
+ * outside [0, capacity) is not written; the lengths are not changed.
+ */
+int b200enc_kv_append(const void* src, long long src_batch_stride, int ld_src, void* cache, long long cache_batch_stride,
+                      int ld_cache, int capacity, const int* lens, int len_stride, int B, int P, int width,
+                      void* stream);
+
 /* *len += delta on the device: the last launch of a decode step, so that the captured step can be replayed. */
 int b200enc_decode_advance(int* len, int delta, void* stream);
 

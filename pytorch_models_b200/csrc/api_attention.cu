@@ -40,7 +40,8 @@ int launch_pdl(Kern kern, int grid, int threads, int smem, cudaStream_t s, const
 static int attention_wide(const void* q, long long qbs, int ldq, const void* k, const void* v, long long kbs, int ldkv,
                           void* out, long long obs, int ldo, int B, int H, int Lq, int Lkv, int head_dim,
                           float scale_log2e, int flags, const float* bias, long long bias_b_stride,
-                          long long bias_h_stride, long long bias_row_stride, cudaStream_t s) {
+                          long long bias_h_stride, long long bias_row_stride, const int* off, int off_stride,
+                          cudaStream_t s) {
   // 4-D maps (head_dim columns, H heads, L rows, B): a tile is two 64-column boxes; the columns >= head_dim of the
   // second box are zero-filled on load and clipped on store. Output: 32 rows x 64 columns per softmax warp and store.
   auto map = [&](CUtensorMap* m, const void* base, int L, int ld, long long bs, uint32_t box_rows) {
@@ -70,28 +71,34 @@ static int attention_wide(const void* q, long long qbs, int ldq, const void* k, 
   p.bias_h_stride = bias_h_stride;
   p.bias_row_stride = bias_row_stride;
   p.abort_word = abort_word();
+  p.off = off;
+  p.off_stride = off_stride;
   const int grid = p.n_items < sm_count() ? p.n_items : sm_count();
-  const auto kern = bias != nullptr ? attention_wide_kernel<true> : attention_wide_kernel<false>;
+  const auto kern = off != nullptr    ? attention_wide_kernel<false, true>
+                    : bias != nullptr ? attention_wide_kernel<true>
+                                      : attention_wide_kernel<false>;
   return launch_pdl(kern, grid, ATT_THREADS, ATW_SMEM_BYTES, s, tq, tk, tv, to, p);
 }
 
-static int attention_impl(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
-                          long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride, int ldo, int B,
-                          int H, int Lq, int Lkv, int head_dim, float scale, int flags, const float* bias,
-                          long long bias_b_stride, long long bias_h_stride, long long bias_row_stride, void* stream) {
-  if (int rc0 = check_abort("b200enc_attention")) return rc0;
-  B200_CHECK_ARG(q && k && v && out, "b200enc_attention: null tensor pointer");
+// off != nullptr: offset-causal mode (b200enc_attention_extend): Lkv is the cache capacity, the query rows of sequence b
+// start at position off[b * off_stride]; always the streaming kernels, flags = B200ENC_ATTN_CAUSAL, no bias.
+static int attention_impl(const char* who, const void* q, long long q_batch_stride, int ldq, const void* k,
+                          const void* v, long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride,
+                          int ldo, int B, int H, int Lq, int Lkv, int head_dim, float scale, int flags,
+                          const float* bias, long long bias_b_stride, long long bias_h_stride,
+                          long long bias_row_stride, const int* off, int off_stride, void* stream) {
+  if (int rc0 = check_abort(who)) return rc0;
+  B200_CHECK_ARG(q && k && v && out, "%s: null tensor pointer", who);
   B200_CHECK_ARG(head_dim == ATT_HD || (head_dim > ATT_HD && head_dim <= ATW_MAX_HD && head_dim % 16 == 0),
-                 "b200enc_attention: head_dim=%d is not supported (64, 80, 96, 112 or 128)", head_dim);
-  B200_CHECK_ARG(B >= 1 && H >= 1 && Lq >= 1 && Lkv >= 1, "b200enc_attention: bad shape B=%d H=%d Lq=%d Lkv=%d", B, H,
-                 Lq, Lkv);
+                 "%s: head_dim=%d is not supported (64, 80, 96, 112 or 128)", who, head_dim);
+  B200_CHECK_ARG(B >= 1 && H >= 1 && Lq >= 1 && Lkv >= 1, "%s: bad shape B=%d H=%d Lq=%d Lkv=%d", who, B, H, Lq, Lkv);
   B200_CHECK_ARG(ldq >= H * head_dim && ldkv >= H * head_dim && ldo >= H * head_dim,
-                 "b200enc_attention: leading dimension smaller than H*head_dim");
+                 "%s: leading dimension smaller than H*head_dim", who);
   B200_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 15u) == 0 && ldo % 8 == 0 && out_batch_stride % 8 == 0,
-                 "b200enc_attention: output rows must be 16-byte aligned");
+                 "%s: output rows must be 16-byte aligned", who);
   constexpr int kAttnFlags = B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL;
-  B200_CHECK_ARG((flags & ~kAttnFlags) == 0, "b200enc_attention: flags=%d has bits outside the documented set (0x%x)",
-                 flags, kAttnFlags);
+  B200_CHECK_ARG((flags & ~kAttnFlags) == 0, "%s: flags=%d has bits outside the documented set (0x%x)", who, flags,
+                 kAttnFlags);
   const long long qbs = B > 1 ? q_batch_stride : (long long)Lq * ldq;
   const long long kbs = B > 1 ? kv_batch_stride : (long long)Lkv * ldkv;
   const long long obs = B > 1 ? out_batch_stride : (long long)Lq * ldo;
@@ -99,8 +106,9 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   if (head_dim != ATT_HD)
     return attention_wide(q, qbs, ldq, k, v, kbs, ldkv, out, obs, ldo, B, H, Lq, Lkv, head_dim, scale_log2e, flags,
-                          bias, bias_b_stride, bias_h_stride, bias_row_stride, s);
-  const bool short_kv = Lkv <= ATS_MAX_KV && bias == nullptr && !(flags & (B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL));
+                          bias, bias_b_stride, bias_h_stride, bias_row_stride, off, off_stride, s);
+  const bool short_kv = Lkv <= ATS_MAX_KV && bias == nullptr && off == nullptr &&
+                        !(flags & (B200ENC_ATTN_CAUSAL | B200ENC_ATTN_GENERAL));
   // K/V boxes: the whole row rounded up to 16 for the short kernel (N of its score MMA), 128-row blocks otherwise
   const int nk16 = (Lkv + 15) & ~15;
   const int kv_box = short_kv ? nk16 : ATT_BKV;
@@ -166,15 +174,20 @@ static int attention_impl(const void* q, long long q_batch_stride, int ldq, cons
   p.bias_row_stride = bias_row_stride;
   p.abort_word = abort_word();
   p.trace = trace;
-  const auto kern = bias != nullptr ? attention_kernel<true> : attention_kernel<false>;
+  p.off = off;
+  p.off_stride = off_stride;
+  const auto kern = off != nullptr    ? attention_kernel<false, true>
+                    : bias != nullptr ? attention_kernel<true>
+                                      : attention_kernel<false>;
   return launch_pdl(kern, grid, ATT_THREADS, ATT_SMEM_BYTES, s, tq, tk, tv, to, p);
 }
 
 extern "C" int b200enc_attention(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
                                  long long kv_batch_stride, int ldkv, void* out, long long out_batch_stride, int ldo,
                                  int B, int H, int Lq, int Lkv, int head_dim, float scale, int flags, void* stream) {
-  return attention_impl(q, q_batch_stride, ldq, k, v, kv_batch_stride, ldkv, out, out_batch_stride, ldo, B, H, Lq, Lkv,
-                        head_dim, scale, flags, nullptr, 0, 0, 0, stream);
+  return attention_impl("b200enc_attention", q, q_batch_stride, ldq, k, v, kv_batch_stride, ldkv, out,
+                        out_batch_stride, ldo, B, H, Lq, Lkv, head_dim, scale, flags, nullptr, 0, 0, 0, nullptr, 0,
+                        stream);
 }
 
 extern "C" int b200enc_attention_bias(const void* q, long long q_batch_stride, int ldq, const void* k, const void* v,
@@ -185,6 +198,31 @@ extern "C" int b200enc_attention_bias(const void* q, long long q_batch_stride, i
   B200_CHECK_ARG(bias != nullptr, "b200enc_attention_bias: null bias");
   B200_CHECK_ARG(bias_b_stride >= 0 && bias_h_stride >= 0 && bias_row_stride >= 0,
                  "b200enc_attention_bias: negative bias stride");
-  return attention_impl(q, q_batch_stride, ldq, k, v, kv_batch_stride, ldkv, out, out_batch_stride, ldo, B, H, Lq, Lkv,
-                        head_dim, scale, flags, bias, bias_b_stride, bias_h_stride, bias_row_stride, stream);
+  return attention_impl("b200enc_attention", q, q_batch_stride, ldq, k, v, kv_batch_stride, ldkv, out,
+                        out_batch_stride, ldo, B, H, Lq, Lkv, head_dim, scale, flags, bias, bias_b_stride,
+                        bias_h_stride, bias_row_stride, nullptr, 0, stream);
+}
+
+extern "C" int b200enc_attention_extend(const void* q, long long q_batch_stride, int ldq, const void* k_cache,
+                                        const void* v_cache, long long cache_batch_stride, int ld_cache, int capacity,
+                                        const int* lens, int len_stride, void* out, long long out_batch_stride,
+                                        int ldo, int B, int H, int P, int head_dim, float scale, void* stream) {
+  const char* who = "b200enc_attention_extend";
+  B200_CHECK_ARG(lens != nullptr, "%s: lens=(nil): the query offsets are the device cache lengths", who);
+  B200_CHECK_ARG(len_stride == 0 || len_stride == 1, "%s: len_stride=%d must be 0 (one length) or 1 (one per sequence)",
+                 who, len_stride);
+  B200_CHECK_ARG(capacity >= 1 && P >= 1 && P <= capacity, "%s: P=%d new rows do not fit a cache of capacity=%d", who,
+                 P, capacity);
+  B200_CHECK_ARG(cache_batch_stride >= (long long)capacity * ld_cache || B == 1,
+                 "%s: cache_batch_stride=%lld is smaller than capacity*ld_cache=%lld", who, cache_batch_stride,
+                 (long long)capacity * ld_cache);
+  const bool aligned = ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k_cache) |
+                         reinterpret_cast<uintptr_t>(v_cache)) & 15u) == 0;
+  B200_CHECK_ARG(aligned && ldq % 8 == 0 && ld_cache % 8 == 0 && (B == 1 || (q_batch_stride % 8 == 0 &&
+                                                                            cache_batch_stride % 8 == 0)),
+                 "%s: q and cache rows must be 16-byte aligned (q=%p k_cache=%p v_cache=%p ldq=%d ld_cache=%d)", who, q,
+                 k_cache, v_cache, ldq, ld_cache);
+  return attention_impl(who, q, q_batch_stride, ldq, k_cache, v_cache, cache_batch_stride, ld_cache, out,
+                        out_batch_stride, ldo, B, H, P, capacity, head_dim, scale, B200ENC_ATTN_CAUSAL, nullptr, 0, 0,
+                        0, lens, len_stride, stream);
 }

@@ -1,5 +1,6 @@
 // C-ABI entry points of incremental decoding (see include/b200enc.h): single-query attention over a KV cache, the
-// token + position embedding at the device-side cache length, and the length update that ends a decode step.
+// token + position embedding at the device-side cache length, the length update that ends a decode step, and the row
+// writer of an extend (its attention is b200enc_attention_extend in api_attention.cu).
 #include "../../include/b200enc.h"
 #include "attention_decode.cuh"
 #include "host_util.h"
@@ -190,6 +191,35 @@ extern "C" int b200enc_embed_rows_at_ragged(const long long* ids, long long rows
                                             void* out, void* stream) {
   return embed_rows_at("b200enc_embed_rows_at_ragged", ids, rows, L, tok, pos, n_pos, pos0, 1, dtype, vocab, d, out,
                        stream);
+}
+
+extern "C" int b200enc_kv_append(const void* src, long long src_batch_stride, int ld_src, void* cache,
+                                 long long cache_batch_stride, int ld_cache, int capacity, const int* lens,
+                                 int len_stride, int B, int P, int width, void* stream) {
+  const char* who = "b200enc_kv_append";
+  if (int rc0 = check_abort(who)) return rc0;
+  B200_CHECK_ARG(src && cache && lens, "%s: null pointer (src=%p cache=%p lens=%p)", who, src, cache,
+                 static_cast<const void*>(lens));
+  B200_CHECK_ARG(len_stride == 0 || len_stride == 1, "%s: len_stride=%d must be 0 (one length) or 1 (one per sequence)",
+                 who, len_stride);
+  B200_CHECK_ARG(B >= 1 && P >= 1 && width >= 8 && width % 8 == 0, "%s: bad shape B=%d P=%d width=%d (a multiple of 8)",
+                 who, B, P, width);
+  B200_CHECK_ARG(capacity >= 1 && P <= capacity, "%s: P=%d new rows do not fit a cache of capacity=%d", who, P,
+                 capacity);
+  B200_CHECK_ARG(ld_src >= width && ld_cache >= width, "%s: ld_src=%d / ld_cache=%d smaller than width=%d", who, ld_src,
+                 ld_cache, width);
+  B200_CHECK_ARG(cache_batch_stride >= (long long)capacity * ld_cache || B == 1,
+                 "%s: cache_batch_stride=%lld is smaller than capacity*ld_cache=%lld", who, cache_batch_stride,
+                 (long long)capacity * ld_cache);
+  B200_CHECK_ARG(aligned16(src) && aligned16(cache) && ld_src % 8 == 0 && ld_cache % 8 == 0 &&
+                     (B == 1 || (src_batch_stride % 8 == 0 && cache_batch_stride % 8 == 0)),
+                 "%s: rows must be 16-byte aligned (src=%p cache=%p ld_src=%d ld_cache=%d)", who, src, cache, ld_src,
+                 ld_cache);
+  const long long total = (long long)B * P * (width / 8);
+  return launch_pdl(kv_append_kernel, int((total + 255) / 256), 256, static_cast<cudaStream_t>(stream),
+                    static_cast<const __nv_bfloat16*>(src), src_batch_stride, ld_src,
+                    static_cast<__nv_bfloat16*>(cache), cache_batch_stride, ld_cache, capacity, lens, len_stride, B, P,
+                    width);
 }
 
 extern "C" int b200enc_decode_advance(int* len, int delta, void* stream) {

@@ -57,6 +57,34 @@ __device__ __forceinline__ float fmax3(float a, float b, float c) {
   return d;
 }
 
+// Offset-causal mode (the kOffset instantiation of the streaming kernels; b200enc_attention_extend): K/V are the rows
+// [0, capacity) of a KV cache, the Lq query rows of sequence b sit at absolute positions off_b + i, and query i sees
+// key j iff j <= off_b + i (bottom-right aligned causal). Sequence b has kv_len = off_b + Lq keys; blocks past it are
+// never visited. The rows [kv_len, capacity) of the cache are not ours: they may hold anything, NaN included, and
+// 0 * NaN = NaN in the P.V product. K there only feeds masked scores, but V rows [kv_len, ceil16(kv_len)) are inside
+// the last P.V K-step, so the MMA issuer zeroes them in shared memory (att_zero_rows) before it issues that P.V.
+// An offset outside [0, capacity - Lq] is computed as offset 0 and the sequence's outputs are set to NaN.
+struct AttOffset {
+  int off;   // query offset of the sequence (0 if out of range)
+  bool bad;  // the device offset was out of range
+};
+__device__ __forceinline__ AttOffset att_seq_offset(const int* off, int stride, int b, int Lq, int capacity) {
+  const int o = off[b * stride];
+  const bool bad = o < 0 || o > capacity - Lq;
+  return AttOffset{bad ? 0 : o, bad};
+}
+
+// Zero rows [r0, r1) of a 128-row x 128-byte shared-memory box (whole rows: the 128B swizzle only permutes the 16-byte
+// chunks inside a row), then make the generic-proxy stores visible to the tensor core. Called by one full warp.
+__device__ __forceinline__ void att_zero_rows(uint32_t box, int r0, int r1) {
+  const int lane = threadIdx.x & 31;
+  for (int i = r0 * 8 + lane; i < r1 * 8; i += 32) {
+    asm volatile("st.shared.v4.u32 [%0], {%1, %1, %1, %1};" ::"r"(box + 16u * i), "r"(0u) : "memory");
+  }
+  fence_proxy_async_smem();
+  __syncwarp();
+}
+
 // Event trace of the -DATT_TRACE build (make ../b200enc_trace): (event, clock) records of CTA 0 in per-role private
 // slots (no atomics: a store and a clock read per event). ATT_EV expects `p.trace`, `tr_n` and `tr_role` in scope;
 // AttTrace carries the same handle into a helper function (one designated lane per softmax warpgroup).

@@ -293,6 +293,25 @@ embed_rows_at_kernel(const long long* __restrict__ ids, long long rows, int L, c
   *reinterpret_cast<uint4*>(out + r * d + c) = make_uint4(packed[0], packed[1], packed[2], packed[3]);
 }
 
+// cache[b][len_b + r][:width] = src[b][r][:width] for r < P (len_b = len[b * len_stride]): the k|v rows of an extend,
+// written before its attention reads every key from the cache. One thread per 16-byte vector. A row that would land
+// outside [0, capacity) is not written.
+__global__ void kv_append_kernel(const __nv_bfloat16* __restrict__ src, long long src_bs, int ld_src,
+                                 __nv_bfloat16* __restrict__ cache, long long cache_bs, int ld_cache, int capacity,
+                                 const int* __restrict__ len, int len_stride, int B, int P, int width) {
+  griddep_wait();  // the previous kernel (the QKV GEMM) wrote the rows
+  const int vec_per_row = width >> 3;
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (long long)B * P * vec_per_row) return;
+  const long long row = t / vec_per_row;
+  const int c = int(t % vec_per_row) * 8;
+  const int b = int(row / P), r = int(row % P);
+  const int n = len[b * len_stride];
+  if (n < 0 || n >= capacity - r) return;
+  const uint4 v = *reinterpret_cast<const uint4*>(src + b * src_bs + (long long)r * ld_src + c);
+  *reinterpret_cast<uint4*>(cache + b * cache_bs + (long long)(n + r) * ld_cache + c) = v;
+}
+
 // len[i] += delta for i < n: the last launch of a decode step (n = 1 shared length, or one per sequence)
 __global__ void decode_advance_kernel(int* len, int n, int delta) {
   griddep_wait();

@@ -55,6 +55,9 @@ struct AttnParams {
   long long bias_b_stride, bias_h_stride, bias_row_stride;
   long long* trace;   // debug only: (event, clock) records of CTA 0 (nullptr in production)
   unsigned int* abort_word;  // raised by the watchdog warp when the CTA stops making progress; may be nullptr
+  // kOffset instantiation only (offset-causal mode, attention_common.cuh): query offsets off[b * off_stride]
+  const int* off;
+  int off_stride;
 };
 
 // One 128-column block of the online softmax for one query row (= one thread = one TMEM lane).
@@ -181,7 +184,8 @@ __device__ __forceinline__ void softmax_block(uint32_t tS, uint32_t tP, const So
   ATT_TR(sy.tr, 203);
 }
 
-template <bool kBias>
+// kOffset: offset-causal mode (attention_common.cuh); p.Lkv is then the cache capacity and p.causal is 1.
+template <bool kBias, bool kOffset = false>
 __global__ void __launch_bounds__(ATT_THREADS, 1)
 attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                  const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmO,
@@ -252,6 +256,10 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
   auto tile_blocks = [&](int item, int t) {
     const int row0 = (item % p.n_qp) * 256 + t * ATT_BQ;
     if (row0 >= p.Lq) return 0;
+    if (kOffset) {
+      const int o = att_seq_offset(p.off, p.off_stride, item / p.n_qp / p.H, p.Lq, p.Lkv).off;
+      return min(o + p.Lq - 1, o + row0 + ATT_BQ - 1) / ATT_BKV + 1;
+    }
     if (!p.causal) return n_kvb;
     return min(p.Lkv - 1, row0 + ATT_BQ - 1) / ATT_BKV + 1;
   };
@@ -308,13 +316,16 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         int item, j;
         uint32_t it, stage, phase;
         int nb0, nb1;  // blocks visited by query tile 0 / 1 of this item (0 = tile absent)
+        int kv;        // kOffset: keys of the item's sequence (offset + Lq)
       };
       auto active = [&](const Blk& bl, int t) { return bl.j < (t == 0 ? bl.nb0 : bl.nb1); };
       auto set_item = [&](Blk& bl) {
         bl.nb0 = bl.item < p.n_items ? tile_blocks(bl.item, 0) : 0;
         bl.nb1 = bl.item < p.n_items ? tile_blocks(bl.item, 1) : 0;
+        if (kOffset && bl.item < p.n_items)
+          bl.kv = att_seq_offset(p.off, p.off_stride, bl.item / p.n_qp / p.H, p.Lq, p.Lkv).off + p.Lq;
       };
-      auto n_mma_of = [&](int j) { return (min(ATT_BKV, p.Lkv - j * ATT_BKV) + 15) & ~15; };
+      auto n_mma_of = [&](const Blk& bl) { return (min(ATT_BKV, (kOffset ? bl.kv : p.Lkv) - bl.j * ATT_BKV) + 15) & ~15; };
       auto issue_qk = [&](const Blk& bl, int t) {
         if (nqk[t] > 0) {  // the softmax warps of this tile hold the previous scores in registers
           mbar_wait_plain(bar(S_EMPTY + t), (nqk[t] - 1) & 1u);
@@ -323,7 +334,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         const uint32_t sq = sbase + ATT_SMEM_Q + (bl.it & 1u) * 2 * ATT_TILE_BYTES + t * ATT_TILE_BYTES;
         const uint64_t dq = make_smem_desc_sw128(sq, 16, 1024);
         const uint64_t dk = make_smem_desc_sw128(sbase + ATT_SMEM_K + bl.stage * ATT_TILE_BYTES, 16, 1024);
-        const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, n_mma_of(bl.j), 0, 0);
+        const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, n_mma_of(bl), 0, 0);
         if (elect_one()) {
 #pragma unroll
           for (int k = 0; k < ATT_HD / 16; ++k)
@@ -362,7 +373,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         return bl;
       };
 
-      Blk cur{int(blockIdx.x), 0, 0u, 0u, 0u, 0, 0};
+      Blk cur{int(blockIdx.x), 0, 0u, 0u, 0u, 0, 0, p.Lkv};
       // Lean issue loop (round 2, second session). The event trace showed that this warp, not the softmax warps, set
       // the period: ~1000 clocks of its own serial work per (tile, block) around ~600 clocks of tcgen05.mma issue.
       // Here everything that does not depend on the softmax warps (operand barriers of block n+2, descriptors) happens
@@ -396,9 +407,14 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
           const uint32_t sq_n = sbase + ATT_SMEM_Q + (nx2.it & 1u) * 2 * ATT_TILE_BYTES;
           const uint64_t dq0 = make_smem_desc_sw128(sq_n, 16, 1024);
           const uint64_t dq1 = make_smem_desc_sw128(sq_n + ATT_TILE_BYTES, 16, 1024);
-          const int ksteps = n_mma_of(cur.j) / 16;
+          const int ksteps = n_mma_of(cur) / 16;
           const uint32_t acc0 = cur.j > 0 ? 1u : 0u;
-          const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, have2 ? n_mma_of(nx2.j) : ATT_BKV, 0, 0);
+          const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, have2 ? n_mma_of(nx2) : ATT_BKV, 0, 0);
+          if (kOffset) {  // V rows past the sequence's keys inside the last P.V K-step (see att_zero_rows)
+            const int keys = cur.kv - cur.j * ATT_BKV;
+            if (keys < ATT_BKV && (keys & 15) != 0)
+              att_zero_rows(sbase + ATT_SMEM_V + cur.stage * ATT_TILE_BYTES, keys, (keys + 15) & ~15);
+          }
           const bool q_done = have2 && nx2.j == max(nx2.nb0, nx2.nb1) - 1;
 #pragma unroll
           for (int t = 0; t < 2; ++t) {
@@ -508,16 +524,20 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       if (nb == 0) continue;                              // tile not scheduled at all (same rule as the MMA warp)
       const bool warp_live = row0 + qd * 32 < p.Lq;       // any valid row in this warp?
       const int qrow = row0 + r;
+      // kOffset: query row i is at position q_off + i, the sequence has kv_len keys
+      const AttOffset so = kOffset ? att_seq_offset(p.off, p.off_stride, b, p.Lq, p.Lkv) : AttOffset{0, false};
+      const int q_off = so.off;
+      const int kv_len = kOffset ? q_off + p.Lq : p.Lkv;
       // m: the maximum the exponentials are taken against. It trails the true running maximum by at most
       // ATT_RESCALE_LOG2 (in the log2 domain), so P <= 2^ATT_RESCALE_LOG2 and the accumulator in TMEM is rescaled
       // only when some row of the warp outgrows that head-room (rare after the first block).
       float m = -INFINITY, l = 0.0f;
 
       for (int j = 0; j < nb; ++j, ++g) {
-        const int nvalid = min(ATT_BKV, p.Lkv - j * ATT_BKV);
+        const int nvalid = min(ATT_BKV, kv_len - j * ATT_BKV);
         // columns of this block this row may attend to: all valid ones, or up to the diagonal with a causal mask
-        const bool diag = p.causal && j * ATT_BKV + ATT_BKV - 1 > row0;  // warp-uniform
-        const int lim = diag ? min(nvalid, qrow - j * ATT_BKV + 1) : nvalid;
+        const bool diag = p.causal && j * ATT_BKV + ATT_BKV - 1 > row0 + q_off;  // warp-uniform
+        const int lim = diag ? min(nvalid, qrow + q_off - j * ATT_BKV + 1) : nvalid;
         mbar_wait_plain(bar(S_FULL + t), g & 1u);
         if (lane == 0 && qd == 2) ATT_EV(200 + t);
         tc_fence_after();
@@ -578,7 +598,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         if (elect_one()) tma_store_wait_read<0>();  // the previous item's store has finished reading the staging
         __syncwarp();
         tmem_wait_ld();
-        const float inv = 1.0f / l;
+        const float inv = kOffset && so.bad ? __int_as_float(0x7fc00000) : 1.0f / l;
         uint8_t* dst = smem + ATT_SMEM_STG + (warp - 4) * ATT_STG_BYTES + lane * 128;
 #pragma unroll
         for (int i = 0; i < 8; ++i) {

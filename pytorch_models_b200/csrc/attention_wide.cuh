@@ -54,6 +54,9 @@ struct AttnWideParams {
   const float* bias;
   long long bias_b_stride, bias_h_stride, bias_row_stride;
   unsigned int* abort_word;  // raised by the watchdog warp when the CTA stops making progress; may be nullptr
+  // kOffset instantiation only (offset-causal mode, attention_common.cuh): query offsets off[b * off_stride]
+  const int* off;
+  int off_stride;
 };
 
 // One 128-column block of the online softmax for one query row (= one thread = one TMEM lane). The whole S row is
@@ -148,7 +151,8 @@ __device__ __forceinline__ void softmax_block_wide(uint32_t tS, int n_chunks, bo
   l += sum.x + sum.y;
 }
 
-template <bool kBias>
+// kOffset: offset-causal mode (attention_common.cuh); p.Lkv is then the cache capacity and p.causal is 1.
+template <bool kBias, bool kOffset = false>
 __global__ void __launch_bounds__(ATT_THREADS, 1)
 attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
                       const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmO,
@@ -211,6 +215,10 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
   auto tile_blocks = [&](int item, int t) {
     const int row0 = (item % p.n_qp) * 256 + t * ATT_BQ;
     if (row0 >= p.Lq) return 0;
+    if (kOffset) {
+      const int o = att_seq_offset(p.off, p.off_stride, item / p.n_qp / p.H, p.Lq, p.Lkv).off;
+      return min(o + p.Lq - 1, o + row0 + ATT_BQ - 1) / ATT_BKV + 1;
+    }
     if (!p.causal) return n_kvb;
     return min(p.Lkv - 1, row0 + ATT_BQ - 1) / ATT_BKV + 1;
   };
@@ -271,13 +279,16 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       int item, j;
       uint32_t it, stage, phase;
       int nb0, nb1;  // blocks visited by query tile 0 / 1 of this item (0 = tile absent)
+      int kv;        // kOffset: keys of the item's sequence (offset + Lq)
     };
     auto active = [&](const Blk& bl, int t) { return bl.j < (t == 0 ? bl.nb0 : bl.nb1); };
     auto set_item = [&](Blk& bl) {
       bl.nb0 = bl.item < p.n_items ? tile_blocks(bl.item, 0) : 0;
       bl.nb1 = bl.item < p.n_items ? tile_blocks(bl.item, 1) : 0;
+      if (kOffset && bl.item < p.n_items)
+        bl.kv = att_seq_offset(p.off, p.off_stride, bl.item / p.n_qp / p.H, p.Lq, p.Lkv).off + p.Lq;
     };
-    auto n_mma_of = [&](int j) { return (min(ATT_BKV, p.Lkv - j * ATT_BKV) + 15) & ~15; };
+    auto n_mma_of = [&](const Blk& bl) { return (min(ATT_BKV, (kOffset ? bl.kv : p.Lkv) - bl.j * ATT_BKV) + 15) & ~15; };
     auto advance = [&](Blk bl) {
       if (++bl.stage == ATW_KV_STAGES) {
         bl.stage = 0;
@@ -301,7 +312,7 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       }
     };
 
-    Blk cur{int(blockIdx.x), 0, 0u, 0u, 0u, 0, 0};
+    Blk cur{int(blockIdx.x), 0, 0u, 0u, 0u, 0, 0, p.Lkv};
     if (cur.item < p.n_items) {
       set_item(cur);
       // scores of the first block
@@ -310,7 +321,7 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       tc_fence_after();
       {
         const uint64_t dk0 = make_smem_desc_sw128(sbase + ATW_SMEM_K, 16, 1024);
-        const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, n_mma_of(0), 0, 0);
+        const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, n_mma_of(cur), 0, 0);
         if (elect_one()) {
           for (int t = 0; t < 2; ++t) {
             if (!active(cur, t)) continue;
@@ -331,9 +342,15 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
         }
         const uint64_t dv0 = make_smem_desc_sw128(sbase + ATW_SMEM_V + cur.stage * ATW_TILE_BYTES, ATW_BOX_BYTES, 1024);
         const uint64_t dk0 = make_smem_desc_sw128(sbase + ATW_SMEM_K + nxt.stage * ATW_TILE_BYTES, 16, 1024);
-        const int ksteps = n_mma_of(cur.j) / 16;
+        const int ksteps = n_mma_of(cur) / 16;
         const uint32_t acc0 = cur.j > 0 ? 1u : 0u;
-        const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, more ? n_mma_of(nxt.j) : ATT_BKV, 0, 0);
+        const uint32_t idesc_s = make_idesc_bf16(ATT_BQ, more ? n_mma_of(nxt) : ATT_BKV, 0, 0);
+        if (kOffset) {  // V rows past the sequence's keys inside the last P.V K-step (see att_zero_rows), both boxes
+          const int keys = cur.kv - cur.j * ATT_BKV;
+          if (keys < ATT_BKV && (keys & 15) != 0)
+            for (int x = 0; x < 2; ++x)
+              att_zero_rows(sbase + ATW_SMEM_V + cur.stage * ATW_TILE_BYTES + x * ATW_BOX_BYTES, keys, (keys + 15) & ~15);
+        }
         const bool q_done = more && nxt.j == max(nxt.nb0, nxt.nb1) - 1;  // last block that reads nxt's Q tiles
 #pragma unroll
         for (int t = 0; t < 2; ++t) {
@@ -417,16 +434,20 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       if (nb == 0) continue;                              // tile not scheduled at all (same rule as the MMA warp)
       const bool warp_live = row0 + qd * 32 < p.Lq;       // any valid row in this warp?
       const int qrow = row0 + r;
+      // kOffset: query row i is at position q_off + i, the sequence has kv_len keys
+      const AttOffset so = kOffset ? att_seq_offset(p.off, p.off_stride, b, p.Lq, p.Lkv) : AttOffset{0, false};
+      const int q_off = so.off;
+      const int kv_len = kOffset ? q_off + p.Lq : p.Lkv;
       // m: the maximum the exponentials are taken against. It trails the true running maximum by at most
       // ATW_RESCALE_LOG2 (in the log2 domain), so P <= 2^ATW_RESCALE_LOG2 and O is rescaled only when some row of
       // the warp outgrows that head-room (rare after the first block).
       float m = -INFINITY, l = 0.0f;
 
       for (int j = 0; j < nb; ++j, ++g) {
-        const int nvalid = min(ATT_BKV, p.Lkv - j * ATT_BKV);
+        const int nvalid = min(ATT_BKV, kv_len - j * ATT_BKV);
         // columns of this block this row may attend to: all valid ones, or up to the diagonal with a causal mask
-        const bool diag = p.causal && j * ATT_BKV + ATT_BKV - 1 > row0;  // warp-uniform
-        const int lim = diag ? min(nvalid, qrow - j * ATT_BKV + 1) : nvalid;
+        const bool diag = p.causal && j * ATT_BKV + ATT_BKV - 1 > row0 + q_off;  // warp-uniform
+        const int lim = diag ? min(nvalid, qrow + q_off - j * ATT_BKV + 1) : nvalid;
         mbar_wait_plain(bar(S_FULL + t), g & 1u);
         tc_fence_after();
         float alpha = 1.0f;
@@ -468,7 +489,7 @@ attention_wide_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       // normalise the head_dim output columns and hand the warp's 32 rows to two TMA stores of 64 columns (columns
       // >= head_dim and rows >= Lq are clipped by the tensor map); the halves share one staging buffer
       if (warp_live) {
-        const float inv = 1.0f / l;
+        const float inv = kOffset && so.bad ? __int_as_float(0x7fc00000) : 1.0f / l;
 #pragma unroll 1
         for (int half = 0; half < 2; ++half) {
           const int col0 = half * 64;

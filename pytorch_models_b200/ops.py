@@ -529,3 +529,53 @@ def decode_advance(length: Tensor, delta: int = 1) -> Tensor:
     else:
         _call("b200enc_decode_advance", dict(delta=delta), dev, length.data_ptr(), int(delta))
     return length
+
+
+def _cache_view(name: str, t: Tensor, B: int, W: int) -> None:
+    if t.dim() != 3 or t.shape[0] != B or t.shape[2] != W or t.stride(2) != 1:
+        raise ValueError(f"{name} must be a (B={B}, capacity, {W}) view with unit inner stride, got {tuple(t.shape)}")
+
+
+def kv_append(src: Tensor, cache: Tensor, length: Tensor) -> Tensor:
+    """cache[b, length_b + r] = src[b, r] for r < P on the device: src (B, P, W) view (the k|v columns of the q|k|v
+    rows), cache (B, capacity, W) view, ``length`` an int32 device tensor of 1 element (one length for the batch) or B
+    (one per sequence). A row that would land at or past the capacity is not written; ``length`` is not changed."""
+    dev = _need_cuda(src, cache, length)
+    _need(src, torch.bfloat16, "src"), _need(cache, torch.bfloat16, "cache"), _need(length, torch.int32, "length")
+    if src.dim() != 3 or src.stride(2) != 1:
+        raise ValueError(f"src must be a (B, P, W) view with unit inner stride, got {tuple(src.shape)}")
+    B, P, W = src.shape
+    _cache_view("cache", cache, B, W)
+    _call(
+        "b200enc_kv_append", dict(B=B, P=P, W=W), dev,
+        src.data_ptr(), src.stride(0), src.stride(1), cache.data_ptr(), cache.stride(0), cache.stride(1),
+        cache.shape[1], length.data_ptr(), int(_per_sequence(length, B, "length")), B, P, W,
+    )
+    return cache
+
+
+def attention_extend(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n_heads: int, scale: float,
+                     length: Tensor) -> Tensor:
+    """Causal attention of P new query rows per sequence against a KV cache, the rows of sequence b at positions
+    length_b + i (query i sees cache rows [0, length_b + i]): q, out (B, P, H*hd) views, k_cache / v_cache
+    (B, capacity, H*hd) views sharing strides that already hold the new rows (`kv_append`), ``length`` as in
+    `kv_append`. With every length 0 this is `attention(q, k, v, out, n_heads, scale, causal=True)` bit for bit."""
+    dev = _need_cuda(q, k_cache, v_cache, out, length)
+    for name, t in (("q", q), ("k_cache", k_cache), ("v_cache", v_cache), ("out", out)):
+        _need(t, torch.bfloat16, name)
+    _need(length, torch.int32, "length")
+    if q.dim() != 3 or q.stride(2) != 1 or out.shape != q.shape or out.stride(2) != 1:
+        raise ValueError("q / out must be (B, P, H*head_dim) views with unit inner stride")
+    B, P, D = q.shape
+    if D % n_heads != 0:
+        raise ValueError("width not divisible by n_heads")
+    _cache_view("k_cache", k_cache, B, D)
+    if k_cache.shape != v_cache.shape or k_cache.stride() != v_cache.stride():
+        raise ValueError("k_cache / v_cache must share shape and strides")
+    _call(
+        "b200enc_attention_extend", dict(B=B, H=n_heads, P=P, keys=k_cache.shape[1]), dev,
+        q.data_ptr(), q.stride(0), q.stride(1), k_cache.data_ptr(), v_cache.data_ptr(), k_cache.stride(0),
+        k_cache.stride(1), k_cache.shape[1], length.data_ptr(), int(_per_sequence(length, B, "length")),
+        out.data_ptr(), out.stride(0), out.stride(1), B, n_heads, P, D // n_heads, float(scale),
+    )
+    return out

@@ -461,9 +461,37 @@ class DecoderLayer(nn.Module):
             cross = (self._pack_proj(self._pcq, [ca.q_proj], self.ca_norm), cq, attend_cross)
         return self._launch(x2, out2, ws, stats_in, want_stats, attend_self, cross)
 
+    def extend(self, x2: Tensor, out2: Tensor, ws: SimpleNamespace, cache: "KVCache", i: int,
+               stats_in: Tensor | None = None, want_stats: bool = False) -> Tensor | None:
+        """`run` for P new tokens per sequence against layer ``i`` of a KV cache: x2 (B*P, d) -> out2 (B*P, d), with
+        ``ws`` the workspace of (B, P) rows (and the memory's length, for its cross-attention buffers).
+
+        The self-attention writes the new k|v rows into the cache at each sequence's length (`ops.kv_append`), then
+        attends causally from there over the cache (`ops.attention_extend`); the cross-attention reads the memory's
+        [k; v] from the cache."""
+        sa, ca = self.sa, self.ca
+        inner = sa.n_heads * sa.head_dim
+        kv = cache.kv[i]
+
+        def attend_self(_qkv2: Tensor, _att2: Tensor) -> None:  # takes the (B, P, ·) views of the same buffers
+            ops.kv_append(ws.qkv[:, :, inner:], kv, cache.length)
+            ops.attention_extend(ws.qkv[:, :, :inner], kv[:, :, :inner], kv[:, :, inner:], ws.att, sa.n_heads,
+                                 sa.scale, cache.length)
+
+        cross = None
+        if ca is not None:
+            ci = ca.n_heads * ca.head_dim
+            mkv = cache.memory_kv[i]
+
+            def attend_cross(_catt2: Tensor) -> None:
+                ops.attention(ws.cq, mkv[:, :, :ci], mkv[:, :, ci:], ws.catt, ca.n_heads, ca.scale)
+
+            cross = (self._pack_proj(self._pcq, [ca.q_proj], self.ca_norm), ws.cq.view(-1, ci), attend_cross)
+        return self._launch(x2, out2, ws, stats_in, want_stats, attend_self, cross)
+
     def _launch(self, x2: Tensor, out2: Tensor, ws: SimpleNamespace, stats_in: Tensor | None, want_stats: bool,
                 attend_self, cross: tuple | None) -> Tensor | None:
-        """The layer's launches on M token rows, x2 (M, d) -> out2 (M, d), for `run` and `step`.
+        """The layer's launches on M token rows, x2 (M, d) -> out2 (M, d), for `run`, `step` and `extend`.
 
         ``attend_self(qkv, att)`` fills ``ws.att`` from the q|k|v rows in ``ws.qkv``; it is given their (M, ·) views.
         With cross-attention, ``cross`` is ``(pack, q_out, attend_cross)``: the cross-attention query projection (with
@@ -752,6 +780,28 @@ class Decoder(nn.ModuleList):
         cache.n += 1
         return cur.view(B, 1, self.d_model), stats
 
+    def extend(self, x3: Tensor, cache: "KVCache", lengths=None) -> tuple[Tensor, Tensor | None]:
+        """P more tokens per sequence on a cache that may already hold some: x3 bf16 contiguous (B, P, d), the tokens
+        at positions ``seq_lengths[b] + i`` -> (tokens (B, P, d), partial statistics or None). The launches of
+        `prefill`, except that each layer writes its k|v rows into the cache at each sequence's length and attends
+        causally from there over the cache (and reads the memory's [k; v] from it); on an empty cache the result equals
+        `prefill`'s bit for bit. Each sequence grows by P tokens, or by ``lengths[b]`` (B host ints in [1, P], rows
+        right-padded as in a ragged `prefill`); a shared-length cache extended by unequal ``lengths`` becomes ragged."""
+        self._check_decodable()
+        B, P, d = x3.shape
+        cache.check_extend(B, P)
+        lengths = cache.check_lengths(lengths, P)
+        Lm = 0 if cache.memory3 is None else cache.memory3.shape[1]
+        ws = self[0].workspace(B, P, x3.device, Lm)
+        bufs = [torch.empty_like(x3), torch.empty_like(x3) if len(self) > 1 else None]
+        cur, stats = x3.view(B * P, d), None
+        for i, layer in enumerate(self):
+            out = bufs[i % 2].view(B * P, d)
+            stats = layer.extend(cur, out, ws, cache, i, stats_in=stats, want_stats=True)
+            cur = out
+        cache.extend_lengths(P, lengths)
+        return cur.view(B, P, d), stats
+
 
 class KVCache:
     """Keys and values of the tokens a `Decoder` has seen, for incremental decoding (`Decoder.new_kv_cache`).
@@ -853,6 +903,25 @@ class KVCache:
         if not 1 <= P <= self.capacity:
             raise ValueError(f"prefill of {P} tokens into a cache of capacity {self.capacity}")
 
+    def extend_lengths(self, P: int, lengths: list[int] | None) -> None:
+        """After an extend of P tokens per row: sequence b grows by ``lengths[b]`` (or P), on the host mirror and on
+        the device. The cache stays shared-length while every sequence has the same length, else it becomes ragged."""
+        new = [n + k for n, k in zip(self.seq_lengths, lengths or [P] * self.batch)]
+        if not self.ragged and len(set(new)) == 1:
+            self.length.fill_(new[0])
+        else:
+            self.length = self.seq_length
+            self.length.copy_(torch.tensor(new, dtype=torch.int32))
+            self.pad = [max(new) - n for n in new]
+        self.n = max(new)
+
+    def check_extend(self, batch: int, P: int) -> None:
+        if batch != self.batch:
+            raise ValueError(f"batch {batch} does not match the cache's batch {self.batch}")
+        if P < 1 or self.n + P > self.capacity:
+            raise ValueError(f"extend of {P} tokens onto {self.n} held tokens overflows a cache of capacity "
+                             f"{self.capacity}")
+
     def check_step(self, batch: int) -> None:
         if batch != self.batch:
             raise ValueError(f"batch {batch} does not match the cache's batch {self.batch}")
@@ -891,11 +960,12 @@ def embed_tokens(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor) -> Ten
 
 
 def embed_tokens_at(ids: Tensor, token_embs: nn.Embedding, pos_embs: Tensor, cache: KVCache) -> Tensor:
-    """`embed_tokens` of one new token per sequence at position ``cache.n``: (B,) or (B, 1) int64 -> contiguous bf16
-    (B, 1, d). The position is read on the device (the cache length), so the launch is the same at every step."""
+    """`embed_tokens` of new tokens at each sequence's cache length: (B,) or (B, 1) int64 (a step) or (B, P) (an
+    extend) -> contiguous bf16 (B, L, d), row l of sequence b at position ``length_b + l``. The position is read on
+    the device (the cache length), so a step's launch is the same at every position."""
     tok, pos = _embedding_tables(ids, token_embs, pos_embs)
-    ids2 = ids.reshape(-1, 1).to(torch.int64).contiguous()
-    out = torch.empty(ids2.shape[0], 1, tok.shape[1], device=ids.device, dtype=torch.bfloat16)
+    ids2 = ids.reshape(ids.shape[0] if ids.dim() else 1, -1).to(torch.int64).contiguous()
+    out = torch.empty(*ids2.shape, tok.shape[1], device=ids.device, dtype=torch.bfloat16)
     return ops.embed_rows_at(ids2, tok, pos, cache.length, out)
 
 
@@ -999,3 +1069,21 @@ class DecoderLM:
         self.layers._check_decodable()
         h, stats = self.layers.step(embed_tokens_at(x, self.token_embs, self.pos_embs, cache), cache)
         return self._logits_as(h, stats, h.shape[:1])
+
+    def extend(self, x: Tensor, cache: KVCache, lengths=None) -> Tensor:
+        """P more tokens of every sequence, (B, P) or (P,) ids continuing a cache that may already hold some (the next
+        turn of a conversation, the next chunk of a long prompt) -> (*, P, vocab) logits, equal within bf16 rounding
+        to ``forward`` of the whole sequence at those positions. On an empty cache it is `prefill`.
+
+        ``lengths``: B host ints in [1, P] when sequence b appends only ``x[b, :lengths[b]]`` (right-padded to P as in
+        `prefill`); the logits of padding positions are not meaningful."""
+        P = x.shape[-1]
+        ids = x.reshape(-1, P)
+        cache.check_extend(ids.shape[0], P)
+        lengths = cache.check_lengths(lengths, P)
+        self.layers._check_decodable()
+        if lengths is not None:
+            pad = torch.arange(P)[None, :] >= torch.tensor(lengths)[:, None]
+            ids = ids.masked_fill(pad.to(ids.device), 0)
+        h, stats = self.layers.extend(embed_tokens_at(ids, self.token_embs, self.pos_embs, cache), cache, lengths)
+        return self._logits_as(h, stats, x.shape)
