@@ -306,6 +306,32 @@ int b200enc_decode_advance(int* len, int delta, void* stream);
 int b200enc_decode_advance_ragged(int* lens, int n, int delta, void* stream);
 
 /*
+ * Greedy speculative decoding: the picks and the acceptance of one round (draft steps, one verify extend of the last
+ * token and k draft tokens, the argmax of its k + 1 logits rows per sequence, then the acceptance below), all on the
+ * device, so that a round can be captured as one CUDA graph.
+ *
+ * out[r * out_stride] = argmax_j logits[r * ld + j] over j < V for r < rows: bf16 logits rows of row stride ld (the
+ * tied-logits GEMM writes rows of ceil8(V) columns; the columns past V are never picked), int64 indices. The order is
+ * torch.argmax's: NaN is greater than any number and of equal values the lowest index wins. One kernel.
+ */
+int b200enc_argmax_rows(const void* logits, long long ld, int rows, int V, long long* out, long long out_stride,
+                        void* stream);
+
+/*
+ * The acceptance of a round with k in [1, 15] draft tokens, one thread per sequence b. ids (B, k+1) int64 holds the
+ * verify extend's input [last, d_1 .. d_k] per sequence, picks (B, k+1) int64 the target's argmax of each verify row
+ * [t_0 .. t_k]. With a the number of leading i < k where t_i == d_{i+1}, the candidates are d_1 .. d_a, t_a; they are
+ * cut after the first token equal to eos (-1: none) and at budget[b] tokens (a budget <= 0 keeps none), leaving m.
+ * Writes emitted[b * out_stride + i] = the kept tokens for i < m and -1 up to i = k, n_emitted[b * out_stride] = m,
+ * budget[b] -= m (0 after an EOS), len[b * len_stride] -= k + 1 - m in both caches (the target's extend and the
+ * draft's k + 1 steps each added k + 1 rows; the kept ones are last and the accepted drafts), and ids[b][0] = the last
+ * kept token when m > 0, the next round's input. len_stride 1: one length per sequence; 0: one length, with B = 1.
+ */
+int b200enc_speculative_accept(const long long* picks, long long* ids, int* budget, long long eos, int* len_target,
+                               int target_len_stride, int* len_draft, int draft_len_stride, long long* emitted,
+                               long long* n_emitted, long long out_stride, int B, int k, void* stream);
+
+/*
  * Launch plan: a recorded sequence of the entry points above, enqueued by ONE call.
  *
  * The reference's forward is a Python loop over modules (nn.Sequential at transformer.py:133-149, the layer body at

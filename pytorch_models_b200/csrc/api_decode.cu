@@ -1,9 +1,11 @@
 // C-ABI entry points of incremental decoding (see include/b200enc.h): single-query attention over a KV cache, the
 // token + position embedding at the device-side cache length, the length update that ends a decode step, and the row
-// writer of an extend (its attention is b200enc_attention_extend in api_attention.cu).
+// writer of an extend (its attention is b200enc_attention_extend in api_attention.cu), and the argmax and acceptance
+// kernels of a speculative-decoding round.
 #include "../../include/b200enc.h"
 #include "attention_decode.cuh"
 #include "host_util.h"
+#include "speculative.cuh"
 
 using namespace b200;
 
@@ -228,4 +230,46 @@ extern "C" int b200enc_decode_advance(int* len, int delta, void* stream) {
 
 extern "C" int b200enc_decode_advance_ragged(int* lens, int n, int delta, void* stream) {
   return decode_advance("b200enc_decode_advance_ragged", lens, n, delta, stream);
+}
+
+extern "C" int b200enc_argmax_rows(const void* logits, long long ld, int rows, int V, long long* out,
+                                   long long out_stride, void* stream) {
+  const char* who = "b200enc_argmax_rows";
+  if (int rc0 = check_abort(who)) return rc0;
+  B200_CHECK_ARG(logits && out, "%s: null pointer (logits=%p out=%p)", who, logits, static_cast<void*>(out));
+  B200_CHECK_ARG(rows >= 1 && V >= 1, "%s: bad shape rows=%d V=%d", who, rows, V);
+  B200_CHECK_ARG(ld >= V, "%s: ld=%lld is smaller than V=%d", who, ld, V);
+  B200_CHECK_ARG(aligned16(logits) && ld % 8 == 0, "%s: logits rows must be 16-byte aligned (logits=%p ld=%lld)", who,
+                 logits, ld);
+  B200_CHECK_ARG(out_stride >= 1 || rows == 1, "%s: out_stride=%lld must be >= 1", who, out_stride);
+  B200_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 7u) == 0, "%s: out=%p must be 8-byte aligned", who,
+                 static_cast<void*>(out));
+  return launch_pdl(argmax_rows_kernel, rows, ARGMAX_THREADS, static_cast<cudaStream_t>(stream),
+                    static_cast<const __nv_bfloat16*>(logits), ld, V, out, out_stride);
+}
+
+extern "C" int b200enc_speculative_accept(const long long* picks, long long* ids, int* budget, long long eos,
+                                          int* len_target, int target_len_stride, int* len_draft,
+                                          int draft_len_stride, long long* emitted, long long* n_emitted,
+                                          long long out_stride, int B, int k, void* stream) {
+  const char* who = "b200enc_speculative_accept";
+  if (int rc0 = check_abort(who)) return rc0;
+  B200_CHECK_ARG(picks && ids && budget && len_target && len_draft && emitted && n_emitted,
+                 "%s: null pointer (picks=%p ids=%p budget=%p len_target=%p len_draft=%p emitted=%p n_emitted=%p)",
+                 who, static_cast<const void*>(picks), static_cast<void*>(ids), static_cast<void*>(budget),
+                 static_cast<void*>(len_target), static_cast<void*>(len_draft), static_cast<void*>(emitted),
+                 static_cast<void*>(n_emitted));
+  B200_CHECK_ARG(B >= 1, "%s: B=%d must be >= 1", who, B);
+  B200_CHECK_ARG(k >= 1 && k <= 15, "%s: k=%d draft tokens, must be in [1, 15]", who, k);
+  B200_CHECK_ARG(target_len_stride == 1 || (target_len_stride == 0 && B == 1),
+                 "%s: target_len_stride=%d must be 1 (one length per sequence), or 0 (one length) with B=1 (B=%d)",
+                 who, target_len_stride, B);
+  B200_CHECK_ARG(draft_len_stride == 1 || (draft_len_stride == 0 && B == 1),
+                 "%s: draft_len_stride=%d must be 1 (one length per sequence), or 0 (one length) with B=1 (B=%d)", who,
+                 draft_len_stride, B);
+  B200_CHECK_ARG(out_stride >= k + 1 || B == 1, "%s: out_stride=%lld is smaller than k+1=%d", who, out_stride, k + 1);
+  B200_CHECK_ARG(eos >= -1, "%s: eos=%lld must be a token id or -1 (none)", who, eos);
+  return launch_pdl(speculative_accept_kernel, (B + 127) / 128, 128, static_cast<cudaStream_t>(stream), picks, ids,
+                    budget, eos, len_target, target_len_stride, len_draft, draft_len_stride, emitted, n_emitted,
+                    out_stride, B, k);
 }

@@ -11,7 +11,7 @@ from __future__ import annotations
 import torch
 from torch import Tensor, nn
 
-from . import ops, plans
+from . import ops, plans, speculative
 from .transformer import step_ids_batch
 
 
@@ -111,3 +111,76 @@ class GraphedStep:
         self.cache.n += 1
         ops.LAUNCHES += self.launches
         return self.static_out.clone()
+
+
+class SpeculativeRound:
+    """``r = SpeculativeRound(target, target_cache, draft, draft_cache, k)``; ``r.start(last, budget)``; then each
+    ``tokens = r()`` replays one captured greedy speculative round (`speculative.speculative_round`) with k draft
+    tokens and returns the tokens each sequence emitted, as host lists.
+
+    Both caches hold the same tokens of every sequence and ``last`` (the newest token, in neither cache) lives on the
+    device between rounds, so a replay needs no input from the host; `__call__` reads the result back with one small
+    device-to-host copy and updates both caches' host mirrors. Capture runs a warm-up round on a side stream and then
+    restores both caches' lengths, the ids and the budget. As for `GraphedStep`, the graph reads the length tensors
+    the caches used at capture; replay is refused once either cache has switched to the other kind."""
+
+    def __init__(self, target: nn.Module, target_cache, draft: nn.Module, draft_cache, k: int = 4, eos: int = -1,
+                 warmup: int = 1) -> None:
+        speculative.check_round(target, target_cache, draft, draft_cache, k)
+        self.target, self.target_cache, self.draft, self.draft_cache = target, target_cache, draft, draft_cache
+        self.k, self.eos = k, -1 if eos is None else int(eos)
+        dev = target_cache.length.device
+        self.ids = torch.zeros(target_cache.batch, k + 1, device=dev, dtype=torch.long)
+        self.budget = torch.zeros(target_cache.batch, device=dev, dtype=torch.int32)
+        self.capture(warmup)
+
+    def start(self, last: Tensor, budget: list[int]) -> None:
+        """Each sequence's newest token ((B,) ids on the device, not yet in either cache) and how many more tokens it
+        may emit (B host ints)."""
+        self.ids[:, 0].copy_(last.reshape(-1))
+        self.budget.copy_(torch.tensor(budget, dtype=torch.int32))
+
+    def _round(self) -> Tensor:
+        return speculative.speculative_round(self.target, self.target_cache, self.draft, self.draft_cache, self.ids,
+                                             self.budget, self.eos)
+
+    @torch.no_grad()
+    def capture(self, warmup: int = 1) -> None:
+        caches = (self.target_cache, self.draft_cache)
+        speculative.check_room(*caches, self.k)
+        self.lengths = tuple(c.length for c in caches)  # the tensors the captured launches read and update
+        saved = [(c.length.clone(), c.n) for c in caches]
+        saved_ids, saved_budget = self.ids.clone(), self.budget.clone()
+        side = torch.cuda.Stream(self.ids.device)
+        side.wait_stream(torch.cuda.current_stream())
+        try:
+            with torch.cuda.stream(side):
+                for _ in range(max(1, warmup)):
+                    self._round()
+                    for c, (length, _) in zip(caches, saved):
+                        c.length.copy_(length)
+            self.graph = torch.cuda.CUDAGraph()
+            n0 = ops.LAUNCHES
+            with torch.cuda.graph(self.graph):
+                self.result = self._round()
+            self.launches = ops.LAUNCHES - n0
+        finally:
+            torch.cuda.current_stream().wait_stream(side)
+            for c, (length, n) in zip(caches, saved):
+                c.length.copy_(length)
+                c.n = n
+            self.ids.copy_(saved_ids)
+            self.budget.copy_(saved_budget)
+
+    @torch.no_grad()
+    def __call__(self) -> list[list[int]]:
+        for name, cache, length in (("target", self.target_cache, self.lengths[0]),
+                                    ("draft", self.draft_cache, self.lengths[1])):
+            if cache.length is not length:
+                kind = "per-sequence" if cache.ragged else "shared"
+                raise ValueError(f"the {name} cache now holds {kind} lengths, not the kind it held when this round was "
+                                 "captured; capture a new SpeculativeRound")
+        speculative.check_room(self.target_cache, self.draft_cache, self.k)
+        self.graph.replay()
+        ops.LAUNCHES += self.launches
+        return speculative.finish_round(self.target_cache, self.draft_cache, self.result)

@@ -579,3 +579,51 @@ def attention_extend(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n
         out.data_ptr(), out.stride(0), out.stride(1), B, n_heads, P, D // n_heads, float(scale),
     )
     return out
+
+
+def argmax_rows(logits: Tensor, out: Tensor) -> Tensor:
+    """out[r] = the index of row r's largest logit, as ``torch.argmax(logits, dim=-1)`` (NaN counts as the largest
+    value, the lowest index wins a tie): logits a (rows, V) bf16 view with unit inner stride and a row stride that is a
+    multiple of 8 (the logits GEMM's rows of ceil8(V) columns), out a (rows,) int64 view of any stride (a column of the
+    (B, k+1) ids of a speculative round)."""
+    dev = _need_cuda(logits, out)
+    _need(logits, torch.bfloat16, "logits"), _need(out, torch.int64, "out")
+    if logits.dim() != 2 or logits.stride(1) != 1:
+        raise ValueError(f"logits must be a (rows, V) view with unit inner stride, got {tuple(logits.shape)} "
+                         f"strides {logits.stride()}")
+    rows, V = logits.shape
+    if out.dim() != 1 or out.shape[0] != rows:
+        raise ValueError(f"out must be a ({rows},) view, got {tuple(out.shape)}")
+    _call("b200enc_argmax_rows", dict(rows=rows, V=V), dev, logits.data_ptr(), logits.stride(0), rows, V,
+          out.data_ptr(), out.stride(0))
+    return out
+
+
+def speculative_accept(picks: Tensor, ids: Tensor, budget: Tensor, eos: int, target_length: Tensor,
+                       draft_length: Tensor, emitted: Tensor, n_emitted: Tensor) -> Tensor:
+    """The acceptance of a speculative round with k draft tokens (``b200enc_speculative_accept``): picks and ids
+    contiguous (B, k+1) int64 (the target's argmax of each verify row; the verify input [last, d_1 .. d_k], whose
+    column 0 becomes the next round's input), budget (B,) int32, the two caches' device lengths (1 element with B = 1,
+    else B), emitted a (B, k+1) int64 view and n_emitted a (B,) int64 view with the same row stride (two parts of one
+    buffer, read back with one copy). ``eos``: token id, or -1 for none."""
+    dev = _need_cuda(picks, ids, budget, target_length, draft_length, emitted, n_emitted)
+    for name, t in (("picks", picks), ("ids", ids), ("emitted", emitted), ("n_emitted", n_emitted)):
+        _need(t, torch.int64, name)
+    _need(budget, torch.int32, "budget")
+    _need(target_length, torch.int32, "target_length"), _need(draft_length, torch.int32, "draft_length")
+    if ids.dim() != 2 or not ids.is_contiguous() or picks.shape != ids.shape or not picks.is_contiguous():
+        raise ValueError(f"picks and ids must be contiguous (B, k+1) tensors, got {tuple(picks.shape)} and "
+                         f"{tuple(ids.shape)}")
+    B, k = ids.shape[0], ids.shape[1] - 1
+    if budget.shape != (B,) or not budget.is_contiguous():
+        raise ValueError(f"budget must be a contiguous ({B},) tensor, got {tuple(budget.shape)}")
+    if (emitted.shape != ids.shape or emitted.stride(1) != 1 or n_emitted.shape != (B,)
+            or n_emitted.stride(0) != emitted.stride(0)):
+        raise ValueError(f"emitted must be a ({B}, {k + 1}) view with unit inner stride and n_emitted a ({B},) view of "
+                         f"the same row stride, got {tuple(emitted.shape)} {emitted.stride()} and "
+                         f"{tuple(n_emitted.shape)} {n_emitted.stride()}")
+    _call("b200enc_speculative_accept", dict(B=B, k=k), dev, picks.data_ptr(), ids.data_ptr(), budget.data_ptr(),
+          int(eos), target_length.data_ptr(), int(_per_sequence(target_length, B, "target_length")),
+          draft_length.data_ptr(), int(_per_sequence(draft_length, B, "draft_length")), emitted.data_ptr(),
+          n_emitted.data_ptr(), emitted.stride(0), B, k)
+    return emitted

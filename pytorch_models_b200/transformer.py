@@ -791,6 +791,14 @@ class Decoder(nn.ModuleList):
         B, P, d = x3.shape
         cache.check_extend(B, P)
         lengths = cache.check_lengths(lengths, P)
+        out = self.extend_launches(x3, cache)
+        cache.extend_lengths(P, lengths)
+        return out
+
+    def extend_launches(self, x3: Tensor, cache: "KVCache") -> tuple[Tensor, Tensor | None]:
+        """The layer launches of `extend`, without its checks and without changing the cache's lengths (device or
+        host): the caller advances them, `extend` from the host, a speculative round on the device."""
+        B, P, d = x3.shape
         Lm = 0 if cache.memory3 is None else cache.memory3.shape[1]
         ws = self[0].workspace(B, P, x3.device, Lm)
         bufs = [torch.empty_like(x3), torch.empty_like(x3) if len(self) > 1 else None]
@@ -799,7 +807,6 @@ class Decoder(nn.ModuleList):
             out = bufs[i % 2].view(B * P, d)
             stats = layer.extend(cur, out, ws, cache, i, stats_in=stats, want_stats=True)
             cur = out
-        cache.extend_lengths(P, lengths)
         return cur.view(B, P, d), stats
 
 
@@ -906,14 +913,41 @@ class KVCache:
     def extend_lengths(self, P: int, lengths: list[int] | None) -> None:
         """After an extend of P tokens per row: sequence b grows by ``lengths[b]`` (or P), on the host mirror and on
         the device. The cache stays shared-length while every sequence has the same length, else it becomes ragged."""
-        new = [n + k for n, k in zip(self.seq_lengths, lengths or [P] * self.batch)]
+        self.store_lengths([n + k for n, k in zip(self.seq_lengths, lengths or [P] * self.batch)])
+
+    def store_lengths(self, new: list[int], device: bool = True) -> None:
+        """Sequence b now holds ``new[b]`` tokens: the host mirror, and with ``device`` the device lengths too
+        (``device=False``: they already hold ``new``, as after a speculative round's accept kernel). The cache keeps
+        one shared length while it has one and every sequence has the same length, else it holds one per sequence."""
         if not self.ragged and len(set(new)) == 1:
-            self.length.fill_(new[0])
+            if device:
+                self.length.fill_(new[0])
         else:
-            self.length = self.seq_length
-            self.length.copy_(torch.tensor(new, dtype=torch.int32))
+            if device:
+                self.length = self.seq_length
+                self.length.copy_(torch.tensor(new, dtype=torch.int32))
             self.pad = [max(new) - n for n in new]
         self.n = max(new)
+
+    def truncate(self, lengths) -> None:
+        """Keep the first ``lengths[b]`` tokens of sequence b (B host ints in [0, seq_lengths[b]], a list or a CPU
+        tensor): undo the last turn of a conversation, regenerate a reply, or roll back rejected draft tokens. The rows
+        past the new lengths are left as they are; the next step or extend overwrites them. A shared-length cache
+        truncated to unequal lengths becomes ragged."""
+        if isinstance(lengths, Tensor):
+            if lengths.is_cuda:
+                raise ValueError("lengths must be host ints (a list or a CPU tensor), not a CUDA tensor: the checks "
+                                 "and the host mirror of the cache need them without a device synchronisation")
+            lengths = lengths.reshape(-1).tolist()
+        lengths = [int(n) for n in lengths]
+        if len(lengths) != self.batch:
+            raise ValueError(f"lengths has {len(lengths)} entries for a batch of {self.batch}")
+        held = self.seq_lengths
+        bad = [b for b, n in enumerate(lengths) if not 0 <= n <= held[b]]
+        if bad:
+            b = bad[0]
+            raise ValueError(f"length {lengths[b]} of sequence {b} is outside [0, {held[b]}] (the tokens it holds)")
+        self.store_lengths(lengths)
 
     def check_extend(self, batch: int, P: int) -> None:
         if batch != self.batch:
@@ -1027,10 +1061,15 @@ class DecoderLM:
     tied token table, and cached decoding on top of it. Holds no parameters; the model defines ``token_embs``,
     ``pos_embs``, ``layers`` (the `Decoder`), ``_logits`` (a `TiedLogits`) and, except for GPT, the final ``norm``."""
 
+    def logits_bf16(self, h: Tensor, stats: Tensor | None) -> Tensor:
+        """bf16 tokens (B, L, d) -> bf16 logits (B, L, vocab), a view into rows of ceil8(vocab) columns (what the
+        greedy picks of a speculative round read); ``stats`` as in `_logits_as`."""
+        return self._logits(h, self.token_embs, getattr(self, "norm", None), stats)
+
     def _logits_as(self, h: Tensor, stats: Tensor | None, lead: tuple) -> Tensor:
         """bf16 tokens (B, L, d) -> logits (*lead, vocab) in the parameters' dtype; ``stats``: partial LayerNorm
         statistics of h's rows, if its producer wrote them."""
-        logits = self._logits(h, self.token_embs, getattr(self, "norm", None), stats)
+        logits = self.logits_bf16(h, stats)
         logits = logits.reshape(*lead, logits.shape[-1])
         out_dtype = self.token_embs.weight.dtype
         return logits if out_dtype == torch.bfloat16 else logits.to(out_dtype)
