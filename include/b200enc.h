@@ -332,6 +332,21 @@ int b200enc_speculative_accept(const long long* picks, long long* ids, int* budg
                                long long* n_emitted, long long out_stride, int B, int k, void* stream);
 
 /*
+ * Draft-free proposals: the k in [1, 15] drafts of a round by n-gram lookup in each sequence's own token history, in
+ * place of the draft model's steps. hist (B, capacity) int64 with row stride hist_stride holds n = len[b * len_stride]
+ * tokens of sequence b (len_stride as above); ids (B, k+1) int64 holds last in column 0. With s = hist[b][0, n)
+ * followed by last: for g = max_ngram down to min_ngram (1 <= min_ngram <= max_ngram <= 8, g <= n), the suffix
+ * s[n-g+1 .. n] is looked up at its latest earlier end e < n; the first g that occurs gives d_i = s'[e + i] for
+ * i = 1..k, s' being s followed by the drafts themselves (so a periodic history keeps its period), and no match gives
+ * d_i = last. Writes ids[b][1..k] = d, hist[b][n] = last, hist[b][n+1 .. n+k] = d and len += k + 1: the history then
+ * holds the rows the verify appends to the target cache, and b200enc_speculative_accept rolls both back alike. A
+ * length outside [0, capacity - k - 1] gets d_i = last and no history write, and still advances by k + 1. Rows at or
+ * past len are never read. One CTA per sequence.
+ */
+int b200enc_ngram_draft(long long* hist, long long hist_stride, int capacity, int* len, int len_stride, long long* ids,
+                        int B, int k, int max_ngram, int min_ngram, void* stream);
+
+/*
  * Launch plan: a recorded sequence of the entry points above, enqueued by ONE call.
  *
  * The reference's forward is a Python loop over modules (nn.Sequential at transformer.py:133-149, the layer body at

@@ -6,8 +6,9 @@ from .audio2text import Whisper, WhisperDecoder, WhisperEncoder, WhisperPreproce
 from .image import ViT
 from .text import BERT, GPT, GPT2
 from .graphs import GraphedStep, SpeculativeRound
+from .speculative import NGramDraft
 from .transformer import MHA, MLP, Decoder, DecoderLayer, Encoder, EncoderLayer, KVCache, invalidate_packed
 
 __all__ = ["MHA", "MLP", "Encoder", "EncoderLayer", "Decoder", "DecoderLayer", "ViT", "WhisperEncoder", "WhisperDecoder",
            "Whisper", "WhisperPreprocessor", "BERT", "GPT", "GPT2", "ops", "plans", "invalidate_packed", "_lib",
-           "KVCache", "GraphedStep", "SpeculativeRound"]
+           "KVCache", "GraphedStep", "SpeculativeRound", "NGramDraft"]

@@ -123,6 +123,8 @@ _SIGNATURES = {
     "b200enc_speculative_accept": (
         c_int, [c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p,
                 c_longlong, c_int, c_int, c_void_p]),
+    "b200enc_ngram_draft": (
+        c_int, [c_void_p, c_longlong, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -1,7 +1,7 @@
 // C-ABI entry points of incremental decoding (see include/b200enc.h): single-query attention over a KV cache, the
 // token + position embedding at the device-side cache length, the length update that ends a decode step, and the row
-// writer of an extend (its attention is b200enc_attention_extend in api_attention.cu), and the argmax and acceptance
-// kernels of a speculative-decoding round.
+// writer of an extend (its attention is b200enc_attention_extend in api_attention.cu), and the argmax, acceptance and
+// n-gram draft kernels of a speculative-decoding round.
 #include "../../include/b200enc.h"
 #include "attention_decode.cuh"
 #include "host_util.h"
@@ -272,4 +272,28 @@ extern "C" int b200enc_speculative_accept(const long long* picks, long long* ids
   return launch_pdl(speculative_accept_kernel, (B + 127) / 128, 128, static_cast<cudaStream_t>(stream), picks, ids,
                     budget, eos, len_target, target_len_stride, len_draft, draft_len_stride, emitted, n_emitted,
                     out_stride, B, k);
+}
+
+extern "C" int b200enc_ngram_draft(long long* hist, long long hist_stride, int capacity, int* len, int len_stride,
+                                   long long* ids, int B, int k, int max_ngram, int min_ngram, void* stream) {
+  const char* who = "b200enc_ngram_draft";
+  if (int rc0 = check_abort(who)) return rc0;
+  B200_CHECK_ARG(hist && len && ids, "%s: null pointer (hist=%p len=%p ids=%p)", who, static_cast<void*>(hist),
+                 static_cast<void*>(len), static_cast<void*>(ids));
+  B200_CHECK_ARG(B >= 1, "%s: B=%d must be >= 1", who, B);
+  B200_CHECK_ARG(k >= 1 && k <= 15, "%s: k=%d draft tokens, must be in [1, 15]", who, k);
+  B200_CHECK_ARG(min_ngram >= 1 && min_ngram <= max_ngram && max_ngram <= NGRAM_MAX,
+                 "%s: min_ngram=%d and max_ngram=%d must satisfy 1 <= min_ngram <= max_ngram <= %d", who, min_ngram,
+                 max_ngram, NGRAM_MAX);
+  B200_CHECK_ARG(len_stride == 1 || (len_stride == 0 && B == 1),
+                 "%s: len_stride=%d must be 1 (one length per sequence), or 0 (one length) with B=1 (B=%d)", who,
+                 len_stride, B);
+  B200_CHECK_ARG(capacity >= k + 1, "%s: capacity=%d cannot hold the k+1=%d rows of a round", who, capacity, k + 1);
+  B200_CHECK_ARG(hist_stride >= capacity || B == 1, "%s: hist_stride=%lld is smaller than capacity=%d", who,
+                 hist_stride, capacity);
+  B200_CHECK_ARG(((reinterpret_cast<uintptr_t>(hist) | reinterpret_cast<uintptr_t>(ids)) & 7u) == 0,
+                 "%s: hist=%p and ids=%p must be 8-byte aligned", who, static_cast<void*>(hist),
+                 static_cast<void*>(ids));
+  return launch_pdl(ngram_draft_kernel, B, NGRAM_THREADS, static_cast<cudaStream_t>(stream), hist, hist_stride,
+                    capacity, len, len_stride, ids, k, max_ngram, min_ngram);
 }

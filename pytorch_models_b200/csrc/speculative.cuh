@@ -1,6 +1,7 @@
-// The device half of a greedy speculative-decoding round (see DESIGN §3.2.5): the argmax of logits rows, and the
-// acceptance of draft tokens against the target's picks, which also rolls both KV caches back past the rejected rows.
-// Neither needs the host, so a whole round (draft steps, verify extend, picks, accept) replays as one CUDA graph.
+// The device half of a greedy speculative-decoding round (see DESIGN §3.2.5): the argmax of logits rows, the
+// acceptance of draft tokens against the target's picks, which also rolls both KV caches back past the rejected rows,
+// and the draft-free proposal of §3.2.6 by n-gram lookup in each sequence's own token history. None needs the host, so
+// a whole round (drafts, verify extend, picks, accept) replays as one CUDA graph.
 #pragma once
 
 #include <cuda_bf16.h>
@@ -125,6 +126,63 @@ __global__ void speculative_accept_kernel(const long long* __restrict__ picks, l
   len_t[b * stride_t] -= k + 1 - m;
   len_d[b * stride_d] -= k + 1 - m;
   if (m > 0) row[0] = em[m - 1];
+}
+
+constexpr int NGRAM_THREADS = 256;
+constexpr int NGRAM_MAX = 8;  // the longest n-gram matched
+
+// Step 1 of a draft-free round (DESIGN §3.2.6), one CTA per sequence b with n = len[b * len_stride] tokens in its
+// history row h = hist + b * ld and ids[b] = [last, ..]. With s = h[0, n) followed by last (T = n + 1 tokens):
+//   L(e)  = the number of leading j < max_ngram with j <= e and s[e - j] == s[n - j], for each end e < n;
+//   g*    = the largest min(L(e), max_ngram) over e, e* the largest e reaching it; no match when g* < min_ngram.
+//   This is "the longest g in [min_ngram, max_ngram] whose suffix occurs earlier, at its latest occurrence".
+//   d_i   = s'[e* + i] for i = 1..k, s' being s followed by the drafts (an overlapping copy keeps a period), or last
+//           for every i without a match.
+// Writes ids[b][1..k] = d, h[n] = last, h[n + 1 .. n + k] = d and len += k + 1, so that the history holds the rows
+// the verify appends to the target cache and speculative_accept rolls both back alike. A length outside
+// [0, capacity - k - 1] drafts last, writes no history row and still advances. Only rows below n are read.
+__global__ void __launch_bounds__(NGRAM_THREADS)
+ngram_draft_kernel(long long* __restrict__ hist, long long ld, int capacity, int* __restrict__ len, int len_stride,
+                   long long* __restrict__ ids, int k, int max_ngram, int min_ngram) {
+  griddep_wait();  // the previous round's accept wrote len and ids[b][0]
+  const int b = blockIdx.x;
+  long long* h = hist + b * ld;
+  long long* row = ids + (long long)b * (k + 1);
+  const int n = len[b * len_stride];
+  const long long last = row[0];
+  const bool ok = n >= 0 && n <= capacity - k - 1;
+  __shared__ long long suf[NGRAM_MAX];  // suf[j] = s[n - j]
+  __shared__ long long red[NGRAM_THREADS / 32];
+  if (ok && threadIdx.x < max_ngram && threadIdx.x <= n)
+    suf[threadIdx.x] = threadIdx.x == 0 ? last : h[n - threadIdx.x];
+  __syncthreads();
+  // key = (min(L(e), max_ngram) << 32) | e for the matches of at least min_ngram tokens, else -1; the largest wins
+  long long key = -1;
+  if (ok) {
+    for (int e = threadIdx.x; e < n; e += NGRAM_THREADS) {
+      int l = 0;
+      while (l < max_ngram && l <= e && h[e - l] == suf[l]) ++l;
+      if (l >= min_ngram) key = max(key, ((long long)l << 32) | e);
+    }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) key = max(key, __shfl_xor_sync(0xffffffffu, key, off));
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (lane == 0) red[warp] = key;
+  __syncthreads();  // also: every thread has read len[b] before thread 0 advances it
+  if (threadIdx.x != 0) return;
+  for (int w = 1; w < NGRAM_THREADS / 32; ++w) key = max(key, red[w]);
+  const int e = key < 0 ? -1 : int(key & 0xffffffffLL);
+  // s'[p] = s'[p - q] for p > n with q = n - e, so d_i = s[e + 1 + (i - 1) % q], a row below n or last
+  const int q = e < 0 ? 1 : n - e;
+  for (int i = 1; i <= k; ++i) {
+    const int p = e + 1 + (i - 1) % q;
+    const long long d = e < 0 || p == n ? last : h[p];
+    row[i] = d;
+    if (ok) h[n + i] = d;
+  }
+  if (ok) h[n] = last;
+  len[b * len_stride] = n + k + 1;
 }
 
 }  // namespace b200

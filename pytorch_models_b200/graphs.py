@@ -116,7 +116,8 @@ class GraphedStep:
 class SpeculativeRound:
     """``r = SpeculativeRound(target, target_cache, draft, draft_cache, k)``; ``r.start(last, budget)``; then each
     ``tokens = r()`` replays one captured greedy speculative round (`speculative.speculative_round`) with k draft
-    tokens and returns the tokens each sequence emitted, as host lists.
+    tokens and returns the tokens each sequence emitted, as host lists. ``draft`` may be a `speculative.NGramDraft`
+    with its token history (``draft.new_kv_cache``) as ``draft_cache``.
 
     Both caches hold the same tokens of every sequence and ``last`` (the newest token, in neither cache) lives on the
     device between rounds, so a replay needs no input from the host; `__call__` reads the result back with one small

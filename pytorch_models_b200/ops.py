@@ -627,3 +627,24 @@ def speculative_accept(picks: Tensor, ids: Tensor, budget: Tensor, eos: int, tar
           draft_length.data_ptr(), int(_per_sequence(draft_length, B, "draft_length")), emitted.data_ptr(),
           n_emitted.data_ptr(), emitted.stride(0), B, k)
     return emitted
+
+
+def ngram_draft(hist: Tensor, length: Tensor, ids: Tensor, k: int, max_ngram: int, min_ngram: int) -> Tensor:
+    """The k drafts of a draft-free speculative round (``b200enc_ngram_draft``): for each sequence, the tokens that
+    followed the latest earlier occurrence of the longest n-gram (max_ngram down to min_ngram tokens) that ends its
+    history ``hist[b, :length_b]`` followed by ``ids[b, 0]``, copied with overlap, or ``ids[b, 0]`` repeated without a
+    match. hist a (B, capacity) int64 view with unit inner stride, ``length`` int32 (1 element with B = 1, else B), ids
+    a contiguous (B, k+1) int64 tensor. Writes the drafts into ids[:, 1:] and [last, drafts] into the history rows at
+    each length, and advances the lengths by k + 1 on the device."""
+    dev = _need_cuda(hist, length, ids)
+    _need(hist, torch.int64, "hist"), _need(ids, torch.int64, "ids"), _need(length, torch.int32, "length")
+    if hist.dim() != 2 or hist.stride(1) != 1:
+        raise ValueError(f"hist must be a (B, capacity) view with unit inner stride, got {tuple(hist.shape)} strides "
+                         f"{hist.stride()}")
+    B, capacity = hist.shape
+    if ids.shape != (B, k + 1) or not ids.is_contiguous():
+        raise ValueError(f"ids must be a contiguous ({B}, {k + 1}) tensor, got {tuple(ids.shape)}")
+    _call("b200enc_ngram_draft", dict(B=B, k=k, capacity=capacity), dev, hist.data_ptr(), hist.stride(0), capacity,
+          length.data_ptr(), int(_per_sequence(length, B, "length")), ids.data_ptr(), B, int(k), int(max_ngram),
+          int(min_ngram))
+    return ids

@@ -60,7 +60,9 @@ class DecoderGenerator:
         ``draft``: a smaller model of the same vocabulary (``GPT2`` / ``GPT``) for greedy speculative decoding
         (``use_cache=True``, ``topk=1``): it proposes ``draft_tokens`` tokens per round, one extend of the model
         verifies them, and the accepted ones cost no step of the model (`graphs.SpeculativeRound`). The result is the
-        model's own greedy result, up to the near-ties above."""
+        model's own greedy result, up to the near-ties above. ``draft=NGramDraft()`` proposes without a second model:
+        the tokens that followed the latest earlier occurrence of the sequence's last few tokens in its own prompt and
+        output (`speculative.NGramDraft`)."""
         self._check_draft(draft, topk, use_cache)
         device = next(self.model.parameters()).device
         eos = self.tokenizer.eos_token_id

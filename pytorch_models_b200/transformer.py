@@ -810,24 +810,16 @@ class Decoder(nn.ModuleList):
         return cur.view(B, P, d), stats
 
 
-class KVCache:
-    """Keys and values of the tokens a `Decoder` has seen, for incremental decoding (`Decoder.new_kv_cache`).
+class CacheLengths:
+    """The length bookkeeping of a cache of B sequences of up to ``capacity`` rows, shared by `KVCache` and the token
+    history of a draft-free speculative round (`speculative.TokenHistory`).
 
-    Per layer: ``kv[i]`` (batch, capacity, 2·inner) bf16, the self-attention k|v rows of positions [0, n); with
-    cross-attention ``memory_kv[i]`` (batch, Lm, 2·inner), the projected memory. ``length`` is the device-side int32
-    length the decode kernels read and the step advances; ``n`` is its host mirror, used for the argument checks. Also
-    holds the step's scratch buffers and the fp32 workspace of the decode kernel.
+    ``length`` is the device-side int32 length the kernels read and advance, and ``n`` its host mirror, used for the
+    argument checks. It is the one ``shared_length`` of the batch until the cache is filled or cut to per-sequence
+    lengths: then it is the (batch,) ``seq_length`` tensor, ``n`` the longest sequence's length and ``pad[b]`` how
+    many tokens sequence b is shorter. `seq_lengths` reads the per-sequence lengths on the host."""
 
-    All sequences of a batch have the same length, unless the cache was filled by a ragged prefill (``lengths``): then
-    ``length`` is the cache's (batch,) int32 tensor of per-sequence lengths, which the step's launches read and advance
-    instead; ``n`` is the longest sequence's length and ``pad[b]`` how many tokens sequence b is shorter, fixed for the
-    whole fill. `seq_lengths` reads the per-sequence lengths on the host. A cache is valid for the weights it was
-    filled with: after changing the model's parameters, start a new cache (this is not detected)."""
-
-    def __init__(self, decoder: Decoder, batch: int, capacity: int, memory3: Tensor | None) -> None:
-        layers = list(decoder)
-        p = next(decoder.parameters())
-        dev = p.device
+    def __init__(self, batch: int, capacity: int, dev: torch.device) -> None:
         self.batch, self.capacity = batch, capacity
         self.n = 0
         self.pad = None
@@ -835,26 +827,6 @@ class KVCache:
         # allocated once, so that a step captured on a ragged fill keeps reading the same tensor after later fills
         self.seq_length = torch.zeros(batch, device=dev, dtype=torch.int32)
         self.length = self.shared_length
-        self.memory3 = memory3
-        e = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)  # noqa: E731
-        self.kv = [e(batch, capacity, 2 * layer.sa.n_heads * layer.sa.head_dim) for layer in layers]
-        self.memory_kv = None
-        ws_bytes = max(ops.decode_workspace_bytes(batch, layer.sa.n_heads, layer.sa.head_dim, capacity)
-                       for layer in layers)
-        if memory3 is not None:
-            Lm, d = memory3.shape[1], memory3.shape[2]
-            self.memory_kv = []
-            for layer in layers:
-                ca = layer.ca
-                ci = ca.n_heads * ca.head_dim
-                pkv = ca._pack("kv", [ca.k_proj, ca.v_proj])
-                mkv = e(batch, Lm, 2 * ci)
-                ops.linear(memory3.view(batch * Lm, d), pkv.w, pkv.bias, mkv.view(batch * Lm, 2 * ci))
-                self.memory_kv.append(mkv)
-                ws_bytes = max(ws_bytes, ops.decode_workspace_bytes(batch, ca.n_heads, ca.head_dim, Lm))
-        self.work = torch.empty((ws_bytes + 3) // 4, device=dev, dtype=torch.float32)
-        self.ws = layers[0].workspace(batch, 1, dev, 0)
-        self.bufs = [e(batch, decoder.d_model), e(batch, decoder.d_model)]
 
     def reset(self) -> None:
         """Empty the cache (for a new prefill); the buffers are kept."""
@@ -910,11 +882,6 @@ class KVCache:
         if not 1 <= P <= self.capacity:
             raise ValueError(f"prefill of {P} tokens into a cache of capacity {self.capacity}")
 
-    def extend_lengths(self, P: int, lengths: list[int] | None) -> None:
-        """After an extend of P tokens per row: sequence b grows by ``lengths[b]`` (or P), on the host mirror and on
-        the device. The cache stays shared-length while every sequence has the same length, else it becomes ragged."""
-        self.store_lengths([n + k for n, k in zip(self.seq_lengths, lengths or [P] * self.batch)])
-
     def store_lengths(self, new: list[int], device: bool = True) -> None:
         """Sequence b now holds ``new[b]`` tokens: the host mirror, and with ``device`` the device lengths too
         (``device=False``: they already hold ``new``, as after a speculative round's accept kernel). The cache keeps
@@ -948,6 +915,52 @@ class KVCache:
             b = bad[0]
             raise ValueError(f"length {lengths[b]} of sequence {b} is outside [0, {held[b]}] (the tokens it holds)")
         self.store_lengths(lengths)
+
+
+class KVCache(CacheLengths):
+    """Keys and values of the tokens a `Decoder` has seen, for incremental decoding (`Decoder.new_kv_cache`).
+
+    Per layer: ``kv[i]`` (batch, capacity, 2·inner) bf16, the self-attention k|v rows of positions [0, n); with
+    cross-attention ``memory_kv[i]`` (batch, Lm, 2·inner), the projected memory. ``length`` is the device-side int32
+    length the decode kernels read and the step advances; ``n`` is its host mirror, used for the argument checks. Also
+    holds the step's scratch buffers and the fp32 workspace of the decode kernel.
+
+    All sequences of a batch have the same length, unless the cache was filled by a ragged prefill (``lengths``): then
+    ``length`` is the cache's (batch,) int32 tensor of per-sequence lengths, which the step's launches read and advance
+    instead; ``n`` is the longest sequence's length and ``pad[b]`` how many tokens sequence b is shorter, fixed for the
+    whole fill. `seq_lengths` reads the per-sequence lengths on the host. A cache is valid for the weights it was
+    filled with: after changing the model's parameters, start a new cache (this is not detected)."""
+
+    def __init__(self, decoder: Decoder, batch: int, capacity: int, memory3: Tensor | None) -> None:
+        layers = list(decoder)
+        p = next(decoder.parameters())
+        dev = p.device
+        super().__init__(batch, capacity, dev)
+        self.memory3 = memory3
+        e = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)  # noqa: E731
+        self.kv = [e(batch, capacity, 2 * layer.sa.n_heads * layer.sa.head_dim) for layer in layers]
+        self.memory_kv = None
+        ws_bytes = max(ops.decode_workspace_bytes(batch, layer.sa.n_heads, layer.sa.head_dim, capacity)
+                       for layer in layers)
+        if memory3 is not None:
+            Lm, d = memory3.shape[1], memory3.shape[2]
+            self.memory_kv = []
+            for layer in layers:
+                ca = layer.ca
+                ci = ca.n_heads * ca.head_dim
+                pkv = ca._pack("kv", [ca.k_proj, ca.v_proj])
+                mkv = e(batch, Lm, 2 * ci)
+                ops.linear(memory3.view(batch * Lm, d), pkv.w, pkv.bias, mkv.view(batch * Lm, 2 * ci))
+                self.memory_kv.append(mkv)
+                ws_bytes = max(ws_bytes, ops.decode_workspace_bytes(batch, ca.n_heads, ca.head_dim, Lm))
+        self.work = torch.empty((ws_bytes + 3) // 4, device=dev, dtype=torch.float32)
+        self.ws = layers[0].workspace(batch, 1, dev, 0)
+        self.bufs = [e(batch, decoder.d_model), e(batch, decoder.d_model)]
+
+    def extend_lengths(self, P: int, lengths: list[int] | None) -> None:
+        """After an extend of P tokens per row: sequence b grows by ``lengths[b]`` (or P), on the host mirror and on
+        the device. The cache stays shared-length while every sequence has the same length, else it becomes ragged."""
+        self.store_lengths([n + k for n, k in zip(self.seq_lengths, lengths or [P] * self.batch)])
 
     def check_extend(self, batch: int, P: int) -> None:
         if batch != self.batch:
