@@ -1,6 +1,8 @@
 """Single-query attention over a KV cache (csrc/attention_decode.cuh) on the GPU, against fp32 SDPA on the same bf16
 inputs with the tolerance of test_gpu_head_dim.py: append mode (the new row comes from the fused q|k|v buffer and is
-written into the cache) and cross mode (read-only cache)."""
+written into the cache) and cross mode (read-only cache). The cache rows past the keys hold NaN (`_Case.poison`): a
+kernel that reads one of them gives NaN, however long the sequence. test_gpu_attention_exact.py checks the same kernel
+on inputs whose outputs are known exactly."""
 from __future__ import annotations
 
 import pytest
@@ -13,6 +15,11 @@ pytestmark = pytest.mark.gpu
 
 HEAD_DIMS = [64, 80, 96, 112, 128]
 GUARD = 8  # cache rows past the new one that must stay untouched
+
+
+def _same(a, b):
+    """Bit for bit, NaN included."""
+    return torch.equal(a.view(torch.int16), b.view(torch.int16))
 
 
 def _close(got, want, atol=0.02, rtol=0.02):
@@ -42,6 +49,12 @@ class _Case:
         self.length = torch.zeros(1, device="cuda", dtype=torch.int32)
         self.out = torch.full((B, W), float("nan"), device="cuda", dtype=torch.bfloat16)
 
+    def poison(self, lengths):
+        """NaN in every cache row past sequence b's new row (row lengths[b]), as after a rolled-back round."""
+        for b, n in enumerate(lengths):
+            if 0 <= n < self.capacity:
+                self.kv[b, n + 1:] = float("nan")
+
     def append(self, n):
         W = self.W
         self.length.fill_(n)
@@ -59,6 +72,7 @@ class _Case:
 def _check_append(B, H, hd, L, seed):
     """L keys: L - 1 cached rows plus the new one."""
     c = _Case(B, H, hd, L + GUARD, seed)
+    c.poison([L - 1] * B)
     before = c.kv.clone()
     want = c.want(L - 1)
     got = c.append(L - 1)
@@ -66,7 +80,7 @@ def _check_append(B, H, hd, L, seed):
     _close(got, want)
     assert torch.equal(c.kv[:, L - 1], c.qkv[:, c.W:]), "the new k|v row was not written bit for bit"
     assert torch.equal(c.kv[:, :L - 1], before[:, :L - 1]), "a cached row changed"
-    assert torch.equal(c.kv[:, L:], before[:, L:]), "the guard band past the new row changed"
+    assert _same(c.kv[:, L:], before[:, L:]), "the guard band past the new row changed"
 
 
 @pytest.mark.parametrize("hd", HEAD_DIMS)
@@ -89,11 +103,12 @@ def test_cross_matches_sdpa(hd, B, H):
     """Read-only cache of 1500 rows (Whisper's encoder memory); capacity larger than Lkv; the cache is not written."""
     Lkv = 1500
     c = _Case(B, H, hd, Lkv + GUARD, 99 + hd + B)
+    c.kv[:, Lkv:] = float("nan")
     before = c.kv.clone()
     W = c.W
     ops.attention_decode(c.qkv[:, :W], c.kv[:, :, :W], c.kv[:, :, W:], c.out, H, hd ** -0.5, c.work, Lkv=Lkv)
     _close(c.out, _sdpa1(c.qkv[:, :W], c.kv[:, :Lkv, :W], c.kv[:, :Lkv, W:], H, hd))
-    assert torch.equal(c.kv, before)
+    assert _same(c.kv, before)
 
 
 @pytest.mark.parametrize("hd", [64, 128])
@@ -118,6 +133,7 @@ def test_length_past_capacity_gives_nan_and_writes_nothing():
 @pytest.mark.parametrize("hd", [64, 112])
 def test_repeats_are_bit_identical(hd):
     c = _Case(16, 12, hd, 5000, 21 + hd)
+    c.poison([4000] * 16)
     first = c.append(4000).clone()
     for _ in range(3):
         assert torch.equal(c.append(4000), first)

@@ -16,22 +16,14 @@ import torch
 
 from conftest import build_model
 from oracle import oracle_torch
-from test_gpu_decode_attention import GUARD, HEAD_DIMS, _Case, _close, _sdpa1
+from attention_inputs import decode_chunk
+from test_gpu_decode_attention import GUARD, HEAD_DIMS, _Case, _close, _same, _sdpa1
 from test_gpu_kv_cache import MAX_ABS_12, _assert_logits
 
 import pytorch_models_b200 as pm
 from pytorch_models_b200 import ops
 
 pytestmark = pytest.mark.gpu
-
-
-def _kc(B, H, keys):
-    """Keys per work item of the decode kernel (decode_chunk in csrc/api_decode.cu)."""
-    bh = B * H
-    nch = 1 if bh >= 4096 else -(-4096 // bh)
-    kc = -(-keys // nch)
-    kc = -(-kc // 64) * 64
-    return min(max(kc, 64), 4096)
 
 
 class _Ragged(_Case):
@@ -50,7 +42,7 @@ class _Ragged(_Case):
 
 
 def _mixed_lengths(B, H, capacity):
-    kc = _kc(B, H, capacity)
+    kc = decode_chunk(B, H, capacity)
     base = [0, 1, kc - 1, kc, kc + 1, capacity - 1]
     return [base[i % len(base)] for i in range(B)]
 
@@ -62,6 +54,7 @@ def test_ragged_append_matches_sdpa(hd, B, H):
     capacity = 700
     c = _Ragged(B, H, hd, capacity, 11 * hd + B)
     lengths = _mixed_lengths(B, H, capacity)
+    c.poison(lengths)
     before = c.kv.clone()
     got = c.append_ragged(lengths).clone()
     torch.cuda.synchronize()
@@ -69,7 +62,7 @@ def test_ragged_append_matches_sdpa(hd, B, H):
         _close(got[b:b + 1], c.want_seq(b, n))
         assert torch.equal(c.kv[b, n], c.qkv[b, c.W:]), f"sequence {b}: the new k|v row was not written bit for bit"
         assert torch.equal(c.kv[b, :n], before[b, :n]), f"sequence {b}: a cached row changed"
-        assert torch.equal(c.kv[b, n + 1:], before[b, n + 1:]), f"sequence {b}: a row past the new one changed"
+        assert _same(c.kv[b, n + 1:], before[b, n + 1:]), f"sequence {b}: a row past the new one changed"
     for _ in range(2):
         assert torch.equal(c.append_ragged(lengths), got), "repeats differ"
 
@@ -78,6 +71,7 @@ def test_ragged_guard_band_and_long_lengths():
     """Lengths up to 4096 with a guard band of GUARD rows past the longest; one sequence of length 0."""
     lengths = [4095, 0, 1000, 63, 64, 2049, 129, 4000]
     c = _Ragged(len(lengths), 4, 128, 4096 + GUARD, 5)
+    c.poison(lengths)
     before = c.kv.clone()
     got = c.append_ragged(lengths).clone()
     for b, n in enumerate(lengths):
@@ -85,7 +79,7 @@ def test_ragged_guard_band_and_long_lengths():
         assert torch.equal(c.kv[b, n], c.qkv[b, c.W:])
         mask = torch.ones(c.capacity, dtype=torch.bool, device="cuda")
         mask[n] = False
-        assert torch.equal(c.kv[b, mask], before[b, mask]), f"sequence {b}: a row other than {n} changed"
+        assert _same(c.kv[b, mask], before[b, mask]), f"sequence {b}: a row other than {n} changed"
 
 
 @pytest.mark.parametrize("hd", [64, 112])
@@ -93,6 +87,7 @@ def test_ragged_length_at_capacity_gives_nan_for_that_sequence_only(hd):
     capacity = 300
     lengths = [5, capacity, 299, -1, 130]
     c = _Ragged(len(lengths), 3, hd, capacity, 3 + hd)
+    c.poison(lengths)
     before = c.kv.clone()
     got = c.append_ragged(lengths).clone()
     for b, n in enumerate(lengths):
@@ -101,7 +96,7 @@ def test_ragged_length_at_capacity_gives_nan_for_that_sequence_only(hd):
             assert torch.equal(c.kv[b, n], c.qkv[b, c.W:])
         else:
             assert bool(got[b].float().isnan().all()), f"sequence {b} (length {n}) is not NaN"
-            assert torch.equal(c.kv[b], before[b]), f"sequence {b} (length {n}) wrote to the cache"
+            assert _same(c.kv[b], before[b]), f"sequence {b} (length {n}) wrote to the cache"
 
 
 @pytest.mark.parametrize("hd", HEAD_DIMS)
