@@ -204,7 +204,17 @@ int b200enc_whisper_logmel(const float* audio, long long audio_stride, int N, in
                            float* out, int* sample_max, void* stream);
 
 /*
- * Incremental decoding: single-query attention over a KV cache (csrc/attention_decode.cuh).
+ * Incremental decoding.
+ *
+ * Device cache lengths: the lengths of a KV cache live in device int32 memory, so a step's arguments are the same at
+ * every position (CUDA-graph capture) and the host never reads them back. Every entry point below that reads them
+ * takes a pointer `lens` and a stride `len_stride`: sequence b reads lens[b * len_stride]. len_stride 0 gives the
+ * batch one shared length (lens holds 1 int), 1 gives each sequence its own (lens holds B ints: a ragged batch, the
+ * prompts of text/generator.py:11-39 run several at a time). Any other stride is refused (-1).
+ */
+
+/*
+ * Single-query attention over a KV cache (csrc/attention_decode.cuh).
  *
  *   out[b][hd*h + :] = softmax_j( q[b][hd*h + :] . k[b][j][hd*h + :] * scale ) v[b][j][hd*h + :]
  *
@@ -215,12 +225,14 @@ int b200enc_whisper_logmel(const float* audio, long long audio_stride, int N, in
  * elements). k_cache / v_cache: [B][capacity] rows of row stride ld_cache and batch stride cache_batch_stride (the K
  * and V halves of one k|v buffer are two pointers with the same strides).
  *
- *   append mode (len != NULL): the keys are cache rows [0, *len) plus the new row k_new / v_new (the step's output of
- *     the fused q|k|v projection, batch stride new_batch_stride). The new row is also written to cache row *len. *len
- *     is read on the device, so a step's arguments are the same at every position (CUDA-graph capture); the caller
- *     advances it (b200enc_decode_advance). A *len outside [0, capacity) gives NaN outputs and writes no cache row.
- *     Lkv is ignored.
- *   cross mode (len == NULL, k_new = v_new = NULL): the keys are cache rows [0, Lkv), Lkv <= capacity; read-only.
+ *   append mode (lens != NULL): with n_b = lens[b * len_stride] (the device cache lengths above), the keys of sequence
+ *     b are cache rows [0, n_b) plus the new row k_new / v_new (the step's output of the fused q|k|v projection, batch
+ *     stride new_batch_stride). The new row is also written to cache row n_b; the caller advances the lengths
+ *     (b200enc_decode_advance). An n_b outside [0, capacity) gives NaN outputs and writes no cache row for sequence b
+ *     only. Lkv is ignored. With per-sequence lengths, work items past a sequence's own length are skipped, so the K/V
+ *     bytes read follow the sum of the lengths; with equal lengths the outputs are bit-identical to len_stride 0.
+ *   cross mode (lens == NULL, k_new = v_new = NULL, len_stride 0): the keys are cache rows [0, Lkv), Lkv <= capacity;
+ *     read-only. Per-sequence lengths are append mode only.
  *
  * workspace: fp32 device scratch of at least b200enc_attention_decode_workspace_bytes(B, H, head_dim, keys) bytes with
  * keys = capacity (append mode) or Lkv (cross mode): per (sequence, head, chunk of keys) the partial softmax state.
@@ -228,43 +240,21 @@ int b200enc_whisper_logmel(const float* audio, long long audio_stride, int N, in
  */
 int b200enc_attention_decode(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
                              long long new_batch_stride, void* k_cache, void* v_cache, long long cache_batch_stride,
-                             int ld_cache, int capacity, const int* len, int Lkv, void* out, long long out_batch_stride,
-                             int B, int H, int head_dim, float scale, float* workspace, long long workspace_bytes,
-                             void* stream);
-
-/*
- * b200enc_attention_decode in append mode for a ragged batch: sequence b has its own device length lens[b] (B ints),
- * so the prompts of one batch can hold different numbers of tokens (text/generator.py:11-39 run on several prompts
- * at once). The keys of sequence b are cache rows [0, lens[b]) plus its new row, which is written to cache row
- * lens[b]. A lens[b] outside [0, capacity) gives NaN outputs for sequence b only and writes none of its rows. The
- * chunking, the grid and the workspace are those of b200enc_attention_decode with keys = capacity; work items past a
- * sequence's own length are skipped, so the K/V bytes read follow the sum of the lengths. With equal lengths the
- * outputs are bit-identical to b200enc_attention_decode. There is no cross mode: lens must not be NULL.
- */
-int b200enc_attention_decode_ragged(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
-                                    long long new_batch_stride, void* k_cache, void* v_cache,
-                                    long long cache_batch_stride, int ld_cache, int capacity, const int* lens,
-                                    void* out, long long out_batch_stride, int B, int H, int head_dim, float scale,
-                                    float* workspace, long long workspace_bytes, void* stream);
+                             int ld_cache, int capacity, const int* lens, int len_stride, int Lkv, void* out,
+                             long long out_batch_stride, int B, int H, int head_dim, float scale, float* workspace,
+                             long long workspace_bytes, void* stream);
 
 /* Workspace size in bytes of b200enc_attention_decode (0 for non-positive arguments). Host-only, no device needed. */
 long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys);
 
 /*
- * b200enc_embed_rows at a position held on the device: out[r][:] = bf16(tok[ids[r]][:] + pos[*pos0 + r % L][:]) for
- * r < rows. The embedding of a decode step (text/gpt2.py:22-23 at position L - 1 of the growing sequence), with *pos0
- * the cache length. pos has n_pos rows; a position outside [0, n_pos) or an id outside [0, vocab) gives a NaN row.
+ * b200enc_embed_rows at positions held on the device: out[r][:] = bf16(tok[ids[r]][:] + pos[p_s + r % L][:]) for
+ * r < rows, with s = r / L the sequence of row r and p_s = pos0[s * pos0_stride] (the device cache lengths above). The
+ * embedding of a decode step (text/gpt2.py:22-23 at position L - 1 of each growing sequence). pos has n_pos rows; a
+ * position outside [0, n_pos) or an id outside [0, vocab) gives a NaN row.
  */
 int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos, int n_pos,
-                          const int* pos0, int dtype, int vocab, int d, void* out, void* stream);
-
-/*
- * b200enc_embed_rows_at with one device position per sequence of L rows: out[r][:] = bf16(tok[ids[r]][:] +
- * pos[pos0[r / L] + r % L][:]), pos0 holding rows / L ints. The embedding of a decode step of a ragged batch
- * (text/gpt2.py:22-23 at each sequence's own position), with pos0 the per-sequence cache lengths.
- */
-int b200enc_embed_rows_at_ragged(const long long* ids, long long rows, int L, const void* tok, const void* pos,
-                                 int n_pos, const int* pos0, int dtype, int vocab, int d, void* out, void* stream);
+                          const int* pos0, int pos0_stride, int dtype, int vocab, int d, void* out, void* stream);
 
 /*
  * Extending a filled KV cache by P rows per sequence (multi-turn continuation, chunked prefill): causal attention whose
@@ -272,16 +262,16 @@ int b200enc_embed_rows_at_ragged(const long long* ids, long long rows, int L, co
  *
  *   out[b][i][hd*h + :] = softmax_{j <= n_b + i}( q[b][i][hd*h + :] . k[b][j][hd*h + :] * scale ) v[b][j][hd*h + :]
  *
- * with n_b = lens[b * len_stride] the device cache length of sequence b (len_stride 0: one length for the batch,
- * 1: one per sequence) and i < P. Replaces F.scaled_dot_product_attention at transformer.py:52 for the causal
- * self-attention of DecoderLayer (transformer.py:97) when the keys and values of the first n_b positions come from a
- * cache: the P query rows see the cached keys and the new ones up to their own position. The new rows' k|v must
- * already be in cache rows [n_b, n_b + P) (b200enc_kv_append), so every key is read from the cache. q, out: P rows
- * per sequence as in b200enc_attention; k_cache / v_cache: [B][capacity] rows of row stride ld_cache and batch stride
- * cache_batch_stride (the K and V halves of one k|v buffer). head_dim 64 or 80-128 (the streaming kernels of
- * b200enc_attention with the causal diagonal shifted by n_b). Only the K/V blocks below row n_b + P are read, so a
- * ragged batch costs what its own lengths cost. The lengths are read on the device; P <= capacity is checked here and
- * n_b + P <= capacity is the caller's (a sequence whose n_b is outside [0, capacity - P] gets NaN outputs).
+ * with n_b = lens[b * len_stride] the device cache length of sequence b (the device cache lengths above) and i < P.
+ * Replaces F.scaled_dot_product_attention at transformer.py:52 for the causal self-attention of DecoderLayer
+ * (transformer.py:97) when the keys and values of the first n_b positions come from a cache: the P query rows see the
+ * cached keys and the new ones up to their own position. The new rows' k|v must already be in cache rows [n_b, n_b + P)
+ * (b200enc_kv_append), so every key is read from the cache. q, out: P rows per sequence as in b200enc_attention;
+ * k_cache / v_cache: [B][capacity] rows of row stride ld_cache and batch stride cache_batch_stride (the K and V halves
+ * of one k|v buffer). head_dim 64 or 80-128 (the streaming kernels of b200enc_attention with the causal diagonal
+ * shifted by n_b). Only the K/V blocks below row n_b + P are read, so a ragged batch costs what its own lengths cost.
+ * The lengths are read on the device; P <= capacity is checked here and n_b + P <= capacity is the caller's (a sequence
+ * whose n_b is outside [0, capacity - P] gets NaN outputs).
  * With n_b = 0 the result is bit-identical to b200enc_attention with B200ENC_ATTN_CAUSAL on the same rows.
  */
 int b200enc_attention_extend(const void* q, long long q_batch_stride, int ldq, const void* k_cache, const void* v_cache,
@@ -290,20 +280,20 @@ int b200enc_attention_extend(const void* q, long long q_batch_stride, int ldq, c
                              float scale, void* stream);
 
 /*
- * cache[b][n_b + r][:width] = src[b][r][:width] for r < P, n_b = lens[b * len_stride] on the device: writes the k|v
- * rows of the fused q|k|v projection (transformer.py:47-49) into a KV cache at each sequence's length, ahead of
- * b200enc_attention_extend. bf16, strides in elements, rows 16-byte aligned, width % 8 == 0. A row that would land
- * outside [0, capacity) is not written; the lengths are not changed.
+ * cache[b][n_b + r][:width] = src[b][r][:width] for r < P, n_b = lens[b * len_stride] (the device cache lengths
+ * above): writes the k|v rows of the fused q|k|v projection (transformer.py:47-49) into a KV cache at each sequence's
+ * length, ahead of b200enc_attention_extend. bf16, strides in elements, rows 16-byte aligned, width % 8 == 0. A row
+ * that would land outside [0, capacity) is not written; the lengths are not changed.
  */
 int b200enc_kv_append(const void* src, long long src_batch_stride, int ld_src, void* cache, long long cache_batch_stride,
                       int ld_cache, int capacity, const int* lens, int len_stride, int B, int P, int width,
                       void* stream);
 
-/* *len += delta on the device: the last launch of a decode step, so that the captured step can be replayed. */
-int b200enc_decode_advance(int* len, int delta, void* stream);
-
-/* lens[i] += delta for i < n on the device: b200enc_decode_advance for the per-sequence lengths of a ragged batch. */
-int b200enc_decode_advance_ragged(int* lens, int n, int delta, void* stream);
+/*
+ * lens[i] += delta for i < n on the device cache lengths above (n = 1: the shared length, n = B: one per sequence):
+ * the last launch of a decode step, so that the captured step can be replayed.
+ */
+int b200enc_decode_advance(int* lens, int n, int delta, void* stream);
 
 /*
  * Greedy speculative decoding: the picks and the acceptance of one round (draft steps, one verify extend of the last
@@ -325,7 +315,8 @@ int b200enc_argmax_rows(const void* logits, long long ld, int rows, int V, long 
  * Writes emitted[b * out_stride + i] = the kept tokens for i < m and -1 up to i = k, n_emitted[b * out_stride] = m,
  * budget[b] -= m (0 after an EOS), len[b * len_stride] -= k + 1 - m in both caches (the target's extend and the
  * draft's k + 1 steps each added k + 1 rows; the kept ones are last and the accepted drafts), and ids[b][0] = the last
- * kept token when m > 0, the next round's input. len_stride 1: one length per sequence; 0: one length, with B = 1.
+ * kept token when m > 0, the next round's input. The lengths are the device cache lengths above, with a shared length
+ * (stride 0) accepted only when B = 1.
  */
 int b200enc_speculative_accept(const long long* picks, long long* ids, int* budget, long long eos, int* len_target,
                                int target_len_stride, int* len_draft, int draft_len_stride, long long* emitted,
@@ -334,7 +325,7 @@ int b200enc_speculative_accept(const long long* picks, long long* ids, int* budg
 /*
  * Draft-free proposals: the k in [1, 15] drafts of a round by n-gram lookup in each sequence's own token history, in
  * place of the draft model's steps. hist (B, capacity) int64 with row stride hist_stride holds n = len[b * len_stride]
- * tokens of sequence b (len_stride as above); ids (B, k+1) int64 holds last in column 0. With s = hist[b][0, n)
+ * tokens of sequence b (len_stride as in b200enc_speculative_accept); ids (B, k+1) int64 holds last in column 0. With s = hist[b][0, n)
  * followed by last: for g = max_ngram down to min_ngram (1 <= min_ngram <= max_ngram <= 8, g <= n), the suffix
  * s[n-g+1 .. n] is looked up at its latest earlier end e < n; the first g that occurs gives d_i = s'[e + i] for
  * i = 1..k, s' being s followed by the drafts themselves (so a periodic history keeps its period), and no match gives

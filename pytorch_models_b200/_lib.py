@@ -97,20 +97,14 @@ _SIGNATURES = {
     "b200enc_attention_decode": (
         c_int,
         [c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p,
-         c_int, c_void_p, c_longlong, c_int, c_int, c_int, c_float, c_void_p, c_longlong, c_void_p],
+         c_int, c_int, c_void_p, c_longlong, c_int, c_int, c_int, c_float, c_void_p, c_longlong, c_void_p],
     ),
     "b200enc_attention_decode_workspace_bytes": (c_longlong, [c_int, c_int, c_int, c_int]),
     "b200enc_embed_rows_at": (
-        c_int, [c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
-    "b200enc_decode_advance": (c_int, [c_void_p, c_int, c_void_p]),
-    "b200enc_attention_decode_ragged": (
         c_int,
-        [c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p,
-         c_void_p, c_longlong, c_int, c_int, c_int, c_float, c_void_p, c_longlong, c_void_p],
+        [c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     ),
-    "b200enc_embed_rows_at_ragged": (
-        c_int, [c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
-    "b200enc_decode_advance_ragged": (c_int, [c_void_p, c_int, c_int, c_void_p]),
+    "b200enc_decode_advance": (c_int, [c_void_p, c_int, c_int, c_void_p]),
     "b200enc_attention_extend": (
         c_int,
         [c_void_p, c_longlong, c_int, c_void_p, c_void_p, c_longlong, c_int, c_int, c_void_p, c_int, c_void_p,

@@ -1,7 +1,9 @@
 // C-ABI entry points of incremental decoding (see include/b200enc.h): single-query attention over a KV cache, the
 // token + position embedding at the device-side cache length, the length update that ends a decode step, and the row
 // writer of an extend (its attention is b200enc_attention_extend in api_attention.cu), and the argmax, acceptance and
-// n-gram draft kernels of a speculative-decoding round.
+// n-gram draft kernels of a speculative-decoding round. Every entry point that reads the device lengths takes them as
+// (lens, len_stride): sequence b reads lens[b * len_stride], so one function serves a shared length (stride 0) and
+// per-sequence lengths (stride 1).
 #include "../../include/b200enc.h"
 #include "attention_decode.cuh"
 #include "host_util.h"
@@ -43,19 +45,30 @@ int launch_pdl(Kern kern, int grid, int threads, cudaStream_t s, Args... args) {
 }
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+}  // namespace
 
-// b200enc_attention_decode (len_stride 0) and b200enc_attention_decode_ragged (len_stride 1, append mode only)
-int attention_decode(const char* who, const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
-                     long long new_batch_stride, void* k_cache, void* v_cache, long long cache_batch_stride,
-                     int ld_cache, int capacity, const int* len, int len_stride, int Lkv, void* out,
-                     long long out_batch_stride, int B, int H, int head_dim, float scale, float* workspace,
-                     long long workspace_bytes, void* stream) {
+extern "C" long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys) {
+  if (B < 1 || H < 1 || head_dim < 1 || keys < 1) return 0;
+  return decode_ws_bytes(B, H, head_dim, keys);
+}
+
+extern "C" int b200enc_attention_decode(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
+                                        long long new_batch_stride, void* k_cache, void* v_cache,
+                                        long long cache_batch_stride, int ld_cache, int capacity, const int* lens,
+                                        int len_stride, int Lkv, void* out, long long out_batch_stride, int B, int H,
+                                        int head_dim, float scale, float* workspace, long long workspace_bytes,
+                                        void* stream) {
+  const char* who = "b200enc_attention_decode";
   if (int rc0 = check_abort(who)) return rc0;
   B200_CHECK_ARG(q && k_cache && v_cache && out && workspace, "%s: null pointer (q=%p k_cache=%p v_cache=%p out=%p "
                  "workspace=%p)", who, q, k_cache, v_cache, out, static_cast<void*>(workspace));
-  const bool append = len != nullptr;
-  B200_CHECK_ARG(!append || (k_new && v_new), "%s: append mode (len != NULL) needs k_new and v_new", who);
-  B200_CHECK_ARG(append || (!k_new && !v_new), "%s: cross mode (len == NULL) takes no k_new / v_new", who);
+  B200_CHECK_ARG(len_stride == 0 || len_stride == 1, "%s: len_stride=%d must be 0 (one length) or 1 (one per sequence)",
+                 who, len_stride);
+  const bool append = lens != nullptr;
+  B200_CHECK_ARG(append || len_stride == 0, "%s: lens=(nil) with len_stride=%d: per-sequence lengths are append mode "
+                 "only", who, len_stride);
+  B200_CHECK_ARG(!append || (k_new && v_new), "%s: append mode (lens != NULL) needs k_new and v_new", who);
+  B200_CHECK_ARG(append || (!k_new && !v_new), "%s: cross mode (lens == NULL) takes no k_new / v_new", who);
   B200_CHECK_ARG(head_dim >= 64 && head_dim <= 128 && head_dim % 16 == 0,
                  "%s: head_dim=%d is not supported (64, 80, 96, 112 or 128)", who, head_dim);
   B200_CHECK_ARG(B >= 1 && H >= 1, "%s: bad shape B=%d H=%d", who, B, H);
@@ -98,7 +111,7 @@ int attention_decode(const char* who, const void* q, long long q_batch_stride, c
   p.cache_bs = cache_batch_stride;
   p.ld_cache = ld_cache;
   p.capacity = capacity;
-  p.len = len;
+  p.len = lens;
   p.len_stride = len_stride;
   p.Lkv = append ? 0 : Lkv;
   p.out = static_cast<__nv_bfloat16*>(out);
@@ -121,9 +134,13 @@ int attention_decode(const char* who, const void* q, long long q_batch_stride, c
   return launch_pdl(decode_combine_kernel, B * H, 128, s, p);
 }
 
-int embed_rows_at(const char* who, const long long* ids, long long rows, int L, const void* tok, const void* pos,
-                  int n_pos, const int* pos0, int pos0_stride, int dtype, int vocab, int d, void* out, void* stream) {
+extern "C" int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos,
+                                     int n_pos, const int* pos0, int pos0_stride, int dtype, int vocab, int d,
+                                     void* out, void* stream) {
+  const char* who = "b200enc_embed_rows_at";
   B200_CHECK_ARG(ids && tok && pos && pos0 && out, "%s: null pointer", who);
+  B200_CHECK_ARG(pos0_stride == 0 || pos0_stride == 1,
+                 "%s: pos0_stride=%d must be 0 (one length) or 1 (one per sequence)", who, pos0_stride);
   B200_CHECK_ARG(rows >= 1 && L >= 1 && rows % L == 0, "%s: rows=%lld must be a positive multiple of L=%d", who, rows,
                  L);
   B200_CHECK_ARG(vocab >= 1 && n_pos >= 1, "%s: vocab=%d and n_pos=%d must be >= 1", who, vocab, n_pos);
@@ -145,54 +162,6 @@ int embed_rows_at(const char* who, const long long* ids, long long rows, int L, 
     return set_error(-1, "%s: unsupported dtype %d", who, dtype);
   B200_CUDA(cudaGetLastError());
   return 0;
-}
-
-int decode_advance(const char* who, int* len, int n, int delta, void* stream) {
-  B200_CHECK_ARG(len != nullptr, "%s: null len", who);
-  B200_CHECK_ARG(n >= 1, "%s: n=%d must be >= 1", who, n);
-  const int threads = n < 256 ? n : 256;
-  return launch_pdl(decode_advance_kernel, 1, threads, static_cast<cudaStream_t>(stream), len, n, delta);
-}
-}  // namespace
-
-extern "C" long long b200enc_attention_decode_workspace_bytes(int B, int H, int head_dim, int keys) {
-  if (B < 1 || H < 1 || head_dim < 1 || keys < 1) return 0;
-  return decode_ws_bytes(B, H, head_dim, keys);
-}
-
-extern "C" int b200enc_attention_decode(const void* q, long long q_batch_stride, const void* k_new, const void* v_new,
-                                        long long new_batch_stride, void* k_cache, void* v_cache,
-                                        long long cache_batch_stride, int ld_cache, int capacity, const int* len,
-                                        int Lkv, void* out, long long out_batch_stride, int B, int H, int head_dim,
-                                        float scale, float* workspace, long long workspace_bytes, void* stream) {
-  return attention_decode("b200enc_attention_decode", q, q_batch_stride, k_new, v_new, new_batch_stride, k_cache,
-                          v_cache, cache_batch_stride, ld_cache, capacity, len, 0, Lkv, out, out_batch_stride, B, H,
-                          head_dim, scale, workspace, workspace_bytes, stream);
-}
-
-extern "C" int b200enc_attention_decode_ragged(const void* q, long long q_batch_stride, const void* k_new,
-                                               const void* v_new, long long new_batch_stride, void* k_cache,
-                                               void* v_cache, long long cache_batch_stride, int ld_cache, int capacity,
-                                               const int* lens, void* out, long long out_batch_stride, int B, int H,
-                                               int head_dim, float scale, float* workspace, long long workspace_bytes,
-                                               void* stream) {
-  const char* who = "b200enc_attention_decode_ragged";
-  B200_CHECK_ARG(lens != nullptr, "%s: lens=(nil): per-sequence lengths are append mode only", who);
-  return attention_decode(who, q, q_batch_stride, k_new, v_new, new_batch_stride, k_cache, v_cache,
-                          cache_batch_stride, ld_cache, capacity, lens, 1, 0, out, out_batch_stride, B, H, head_dim,
-                          scale, workspace, workspace_bytes, stream);
-}
-
-extern "C" int b200enc_embed_rows_at(const long long* ids, long long rows, int L, const void* tok, const void* pos,
-                                     int n_pos, const int* pos0, int dtype, int vocab, int d, void* out, void* stream) {
-  return embed_rows_at("b200enc_embed_rows_at", ids, rows, L, tok, pos, n_pos, pos0, 0, dtype, vocab, d, out, stream);
-}
-
-extern "C" int b200enc_embed_rows_at_ragged(const long long* ids, long long rows, int L, const void* tok,
-                                            const void* pos, int n_pos, const int* pos0, int dtype, int vocab, int d,
-                                            void* out, void* stream) {
-  return embed_rows_at("b200enc_embed_rows_at_ragged", ids, rows, L, tok, pos, n_pos, pos0, 1, dtype, vocab, d, out,
-                       stream);
 }
 
 extern "C" int b200enc_kv_append(const void* src, long long src_batch_stride, int ld_src, void* cache,
@@ -224,12 +193,12 @@ extern "C" int b200enc_kv_append(const void* src, long long src_batch_stride, in
                     width);
 }
 
-extern "C" int b200enc_decode_advance(int* len, int delta, void* stream) {
-  return decode_advance("b200enc_decode_advance", len, 1, delta, stream);
-}
-
-extern "C" int b200enc_decode_advance_ragged(int* lens, int n, int delta, void* stream) {
-  return decode_advance("b200enc_decode_advance_ragged", lens, n, delta, stream);
+extern "C" int b200enc_decode_advance(int* lens, int n, int delta, void* stream) {
+  const char* who = "b200enc_decode_advance";
+  B200_CHECK_ARG(lens != nullptr, "%s: null lens", who);
+  B200_CHECK_ARG(n >= 1, "%s: n=%d must be >= 1", who, n);
+  const int threads = n < 256 ? n : 256;
+  return launch_pdl(decode_advance_kernel, 1, threads, static_cast<cudaStream_t>(stream), lens, n, delta);
 }
 
 extern "C" int b200enc_argmax_rows(const void* logits, long long ld, int rows, int V, long long* out,

@@ -435,7 +435,8 @@ def whisper_logmel(audio: Tensor, filters_t: Tensor, out: Tensor) -> Tensor:
 
 def _per_sequence(length: Tensor | None, B: int, name: str) -> bool:
     """True if a device length tensor holds one length per sequence (B > 1 elements), False if it holds one shared
-    length; anything else is refused."""
+    length; anything else is refused. As an int it is the ``len_stride`` of the C-ABI: sequence b reads
+    length[b * stride]."""
     if length is None or length.numel() == 1:
         return False
     if length.dim() != 1 or length.numel() != B or not length.is_contiguous():
@@ -457,8 +458,8 @@ def attention_decode(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n
     workspace: fp32, at least `decode_workspace_bytes` bytes.
     Append mode (``length`` = int32 device tensor of one element): attends over cache rows [0, length) plus the new row
     ``k_new`` / ``v_new`` ((B, H*hd) views) and writes the new row into cache row ``length``; ``length`` itself is not
-    changed (`decode_advance`). A ``length`` of B elements gives each sequence its own length (a ragged batch,
-    ``b200enc_attention_decode_ragged``). Cross mode (``length`` None): attends over cache rows [0, Lkv)."""
+    changed (`decode_advance`). A ``length`` of B elements gives each sequence its own length (a ragged batch).
+    Cross mode (``length`` None): attends over cache rows [0, Lkv)."""
     dev = _need_cuda(q, k_cache, v_cache, out, workspace, k_new, v_new, length)
     for name, t in (("q", q), ("k_cache", k_cache), ("v_cache", v_cache), ("out", out), ("k_new", k_new),
                     ("v_new", v_new)):
@@ -482,20 +483,12 @@ def attention_decode(q: Tensor, k_cache: Tensor, v_cache: Tensor, out: Tensor, n
         new_bs = k_new.stride(0)
     if not workspace.is_contiguous():
         raise ValueError("workspace must be contiguous")
-    if _per_sequence(length, B, "length"):
-        _call(
-            "b200enc_attention_decode_ragged", dict(B=B, H=n_heads, keys=k_cache.shape[1], append=True), dev,
-            q.data_ptr(), q.stride(0), k_new.data_ptr(), v_new.data_ptr(), new_bs, k_cache.data_ptr(),
-            v_cache.data_ptr(), k_cache.stride(0), k_cache.stride(1), k_cache.shape[1], length.data_ptr(),
-            out.data_ptr(), out.stride(0), B, n_heads, D // n_heads, float(scale), workspace.data_ptr(),
-            workspace.numel() * 4,
-        )
-        return out
     _call(
         "b200enc_attention_decode", dict(B=B, H=n_heads, keys=k_cache.shape[1], append=length is not None), dev,
         q.data_ptr(), q.stride(0), _ptr(k_new), _ptr(v_new), new_bs, k_cache.data_ptr(), v_cache.data_ptr(),
-        k_cache.stride(0), k_cache.stride(1), k_cache.shape[1], _ptr(length), int(Lkv), out.data_ptr(), out.stride(0),
-        B, n_heads, D // n_heads, float(scale), workspace.data_ptr(), workspace.numel() * 4,
+        k_cache.stride(0), k_cache.stride(1), k_cache.shape[1], _ptr(length), int(_per_sequence(length, B, "length")),
+        int(Lkv), out.data_ptr(), out.stride(0), B, n_heads, D // n_heads, float(scale), workspace.data_ptr(),
+        workspace.numel() * 4,
     )
     return out
 
@@ -509,11 +502,10 @@ def embed_rows_at(ids: Tensor, tok: Tensor, pos: Tensor, pos0: Tensor, out: Tens
     dt = _embed_args("embed_rows_at", ids, tok, pos, out)
     B, L = ids.shape
     vocab, d = tok.shape
-    name = "b200enc_embed_rows_at_ragged" if _per_sequence(pos0, B, "pos0") else "b200enc_embed_rows_at"
     _call(
-        name, dict(rows=B * L, d=d), dev,
-        ids.data_ptr(), B * L, L, tok.data_ptr(), pos.data_ptr(), pos.shape[0], pos0.data_ptr(), dt, vocab, d,
-        out.data_ptr(),
+        "b200enc_embed_rows_at", dict(rows=B * L, d=d), dev,
+        ids.data_ptr(), B * L, L, tok.data_ptr(), pos.data_ptr(), pos.shape[0], pos0.data_ptr(),
+        int(_per_sequence(pos0, B, "pos0")), dt, vocab, d, out.data_ptr(),
     )
     return out
 
@@ -523,11 +515,8 @@ def decode_advance(length: Tensor, delta: int = 1) -> Tensor:
     a decode step's decoder stack."""
     dev = _need_cuda(length)
     _need(length, torch.int32, "length")
-    n = length.numel()
-    if _per_sequence(length, n, "length"):
-        _call("b200enc_decode_advance_ragged", dict(n=n, delta=delta), dev, length.data_ptr(), n, int(delta))
-    else:
-        _call("b200enc_decode_advance", dict(delta=delta), dev, length.data_ptr(), int(delta))
+    n = length.numel() if _per_sequence(length, length.numel(), "length") else 1
+    _call("b200enc_decode_advance", dict(n=n, delta=delta), dev, length.data_ptr(), n, int(delta))
     return length
 
 

@@ -1,9 +1,9 @@
 """Ragged incremental decoding on the GPU: one batch of sequences of different lengths, each with its own device-side
 cache length.
 
-Kernel: b200enc_attention_decode_ragged against fp32 SDPA per sequence (tolerance of test_gpu_decode_attention.py), its
-cache writes, its repeats, its NaN for an out-of-range length, bit-identity with the shared-length launch at equal
-lengths; the per-sequence embedding and length update against torch.
+Kernel: b200enc_attention_decode with per-sequence lengths against fp32 SDPA per sequence (tolerance of
+test_gpu_decode_attention.py), its cache writes, its repeats, its NaN for an out-of-range length, bit-identity with the
+shared-length launch at equal lengths; the per-sequence embedding and length update against torch.
 Models: ragged prefill + teacher-forced steps of GPT-2, GPT and the Whisper decoder against each sequence's own
 unpadded forward and the reference's logits (bound of test_gpu_kv_cache.py), a 12-layer d 768 GPT-2 against the fp32
 oracle, equal-length ragged fills against uniform fills, graphed against eager steps, and `generate_batch` against

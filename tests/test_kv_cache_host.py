@@ -14,14 +14,15 @@ A = 0x10000  # a 16-byte aligned fake device address: every call below fails its
 
 
 def _decode(**over):
-    """b200enc_attention_decode in append mode with valid arguments except for ``over``; returns (rc, message)."""
+    """b200enc_attention_decode in append mode with one shared length (len_stride 0) and valid arguments except for
+    ``over``; returns (rc, message)."""
     B, H, hd, cap = 2, 3, 64, 100
     W = H * hd
     lib = _lib.load()
     ws = lib.b200enc_attention_decode_workspace_bytes(B, H, hd, cap)
     a = dict(q=A, q_bs=3 * W, k_new=A, v_new=A, new_bs=3 * W, k_cache=A, v_cache=A, cache_bs=cap * 2 * W,
-             ld_cache=2 * W, capacity=cap, len=A, Lkv=0, out=A, out_bs=W, B=B, H=H, head_dim=hd, scale=0.125,
-             ws=A, ws_bytes=ws)
+             ld_cache=2 * W, capacity=cap, lens=A, len_stride=0, Lkv=0, out=A, out_bs=W, B=B, H=H, head_dim=hd,
+             scale=0.125, ws=A, ws_bytes=ws)
     a.update(over)
     rc = lib.b200enc_attention_decode(*a.values(), None)
     return rc, lib.b200enc_last_error().decode()
@@ -40,12 +41,12 @@ def test_workspace_size_is_positive_and_grows_with_capacity():
     (dict(out=None), "out=(nil)"),
     (dict(ws=None), "workspace=(nil)"),
     (dict(k_new=None), "needs k_new and v_new"),
-    (dict(len=None, Lkv=50), "takes no k_new"),
+    (dict(lens=None, Lkv=50), "takes no k_new"),
     (dict(head_dim=32), "head_dim=32"),
     (dict(head_dim=72), "head_dim=72"),
     (dict(B=0), "B=0"),
     (dict(capacity=0), "capacity=0"),
-    (dict(len=None, k_new=None, v_new=None, Lkv=101), "Lkv=101"),
+    (dict(lens=None, k_new=None, v_new=None, Lkv=101), "Lkv=101"),
     (dict(ld_cache=100), "ld_cache=100"),
     (dict(cache_bs=1000), "cache_batch_stride=1000"),
     (dict(q_bs=8), "q_batch_stride=8"),
@@ -54,15 +55,18 @@ def test_workspace_size_is_positive_and_grows_with_capacity():
     (dict(q=A + 8), "16-byte aligned"),
     (dict(out_bs=196), "out 196"),
     (dict(ws_bytes=16), "workspace_bytes=16"),
+    (dict(len_stride=2), "len_stride=2 must be 0 (one length) or 1 (one per sequence)"),
+    (dict(len_stride=-1), "len_stride=-1 must be 0 (one length) or 1 (one per sequence)"),
+    (dict(lens=None, k_new=None, v_new=None, Lkv=50, len_stride=1), "append mode only"),
 ])
-def test_decode_argument_checks(over, needle):
+def test_decode_shared_length_argument_checks(over, needle):
     rc, msg = _decode(**over)
     assert rc == -1 and needle in msg, msg
 
 
 def _embed_at(**over):
     lib = _lib.load()
-    a = dict(ids=A, rows=4, L=1, tok=A, pos=A, n_pos=10, pos0=A, dtype=0, vocab=50, d=64, out=A)
+    a = dict(ids=A, rows=4, L=1, tok=A, pos=A, n_pos=10, pos0=A, pos0_stride=0, dtype=0, vocab=50, d=64, out=A)
     a.update(over)
     rc = lib.b200enc_embed_rows_at(*a.values(), None)
     return rc, lib.b200enc_last_error().decode()
@@ -76,15 +80,17 @@ def _embed_at(**over):
     (dict(d=60), "d=60"),
     (dict(out=A + 4), "16-byte aligned"),
     (dict(dtype=7), "dtype 7"),
+    (dict(pos0_stride=2), "pos0_stride=2 must be 0 (one length) or 1 (one per sequence)"),
+    (dict(pos0_stride=-1), "pos0_stride=-1 must be 0 (one length) or 1 (one per sequence)"),
 ])
-def test_embed_rows_at_argument_checks(over, needle):
+def test_embed_rows_at_shared_length_argument_checks(over, needle):
     rc, msg = _embed_at(**over)
     assert rc == -1 and needle in msg, msg
 
 
-def test_decode_advance_refuses_null():
+def test_decode_advance_refuses_null_lens():
     lib = _lib.load()
-    assert lib.b200enc_decode_advance(None, 1, None) == -1
+    assert lib.b200enc_decode_advance(None, 1, 1, None) == -1
     assert b"null len" in lib.b200enc_last_error()
 
 

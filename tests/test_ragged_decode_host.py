@@ -1,6 +1,6 @@
 """Host-side checks of ragged incremental decoding, sequences of different lengths in one batch (no GPU needed): the
-argument checks of the per-sequence entry points, the refusals of a ragged prefill, and that a ragged decode step
-issues the same launches as a shared-length one."""
+argument checks of the entry points called with per-sequence lengths (len_stride 1), the refusals of a ragged prefill,
+and that a ragged decode step issues the same launches as a shared-length one."""
 from __future__ import annotations
 
 import pytest
@@ -13,17 +13,18 @@ from pytorch_models_b200.transformer import KVCache
 A = 0x10000  # a 16-byte aligned fake device address: every call below fails its checks before touching it
 
 
-def _decode_ragged(**over):
-    """b200enc_attention_decode_ragged with valid arguments except for ``over``; returns (rc, message)."""
+def _decode_per_sequence(**over):
+    """b200enc_attention_decode with per-sequence lengths and valid arguments except for ``over``; returns (rc,
+    message)."""
     B, H, hd, cap = 2, 3, 64, 100
     W = H * hd
     lib = _lib.load()
     ws = lib.b200enc_attention_decode_workspace_bytes(B, H, hd, cap)
     a = dict(q=A, q_bs=3 * W, k_new=A, v_new=A, new_bs=3 * W, k_cache=A, v_cache=A, cache_bs=cap * 2 * W,
-             ld_cache=2 * W, capacity=cap, lens=A, out=A, out_bs=W, B=B, H=H, head_dim=hd, scale=0.125,
-             ws=A, ws_bytes=ws)
+             ld_cache=2 * W, capacity=cap, lens=A, len_stride=1, Lkv=0, out=A, out_bs=W, B=B, H=H, head_dim=hd,
+             scale=0.125, ws=A, ws_bytes=ws)
     a.update(over)
-    rc = lib.b200enc_attention_decode_ragged(*a.values(), None)
+    rc = lib.b200enc_attention_decode(*a.values(), None)
     return rc, lib.b200enc_last_error().decode()
 
 
@@ -44,17 +45,17 @@ def _decode_ragged(**over):
     (dict(out_bs=196), "out 196"),
     (dict(ws_bytes=16), "workspace_bytes=16"),
 ])
-def test_decode_ragged_argument_checks(over, needle):
-    rc, msg = _decode_ragged(**over)
+def test_decode_per_sequence_argument_checks(over, needle):
+    rc, msg = _decode_per_sequence(**over)
     assert rc == -1 and needle in msg, msg
-    assert msg.startswith("b200enc_attention_decode_ragged:"), msg
+    assert msg.startswith("b200enc_attention_decode:"), msg
 
 
-def _embed_at_ragged(**over):
+def _embed_at_per_sequence(**over):
     lib = _lib.load()
-    a = dict(ids=A, rows=4, L=1, tok=A, pos=A, n_pos=10, pos0=A, dtype=0, vocab=50, d=64, out=A)
+    a = dict(ids=A, rows=4, L=1, tok=A, pos=A, n_pos=10, pos0=A, pos0_stride=1, dtype=0, vocab=50, d=64, out=A)
     a.update(over)
-    rc = lib.b200enc_embed_rows_at_ragged(*a.values(), None)
+    rc = lib.b200enc_embed_rows_at(*a.values(), None)
     return rc, lib.b200enc_last_error().decode()
 
 
@@ -67,16 +68,16 @@ def _embed_at_ragged(**over):
     (dict(out=A + 4), "16-byte aligned"),
     (dict(dtype=7), "dtype 7"),
 ])
-def test_embed_rows_at_ragged_argument_checks(over, needle):
-    rc, msg = _embed_at_ragged(**over)
-    assert rc == -1 and needle in msg and msg.startswith("b200enc_embed_rows_at_ragged:"), msg
+def test_embed_rows_at_per_sequence_argument_checks(over, needle):
+    rc, msg = _embed_at_per_sequence(**over)
+    assert rc == -1 and needle in msg and msg.startswith("b200enc_embed_rows_at:"), msg
 
 
-def test_decode_advance_ragged_checks():
+def test_decode_advance_per_sequence_checks():
     lib = _lib.load()
-    assert lib.b200enc_decode_advance_ragged(None, 4, 1, None) == -1
+    assert lib.b200enc_decode_advance(None, 4, 1, None) == -1
     assert b"null len" in lib.b200enc_last_error()
-    assert lib.b200enc_decode_advance_ragged(A, 0, 1, None) == -1
+    assert lib.b200enc_decode_advance(A, 0, 1, None) == -1
     assert b"n=0" in lib.b200enc_last_error()
 
 

@@ -3,7 +3,7 @@
 after warm-up, medians of `--rounds` interleaved rounds; the device name, power limit and SM clocks are queried
 (nothing is changed) and stored beside the numbers.
 
-1. b200enc_attention_decode_ragged with lengths drawn uniformly from [1, capacity], against the shared-length launch
+1. b200enc_attention_decode with per-sequence lengths drawn uniformly from [1, capacity], against the shared-length launch
    at the mean length and at the longest length (what padding every sequence to the longest would cost). The K/V
    caches are rotated over enough copies that every launch reads its rows from HBM, not from the 126 MB L2.
 2. The shared-length launch of this build against a parent build of libb200enc.so (`--parent-lib`, loaded next to
@@ -68,8 +68,8 @@ class Caches:
                                         length=length)
         rc = lib.b200enc_attention_decode(
             q.data_ptr(), q.stride(0), kn.data_ptr(), vn.data_ptr(), kn.stride(0), k.data_ptr(), v.data_ptr(),
-            k.stride(0), k.stride(1), k.shape[1], length.data_ptr(), 0, self.out.data_ptr(), self.out.stride(0), self.B,
-            self.H, self.hd, self.hd ** -0.5, self.work.data_ptr(), self.work.numel() * 4,
+            k.stride(0), k.stride(1), k.shape[1], length.data_ptr(), 0, 0, self.out.data_ptr(), self.out.stride(0),
+            self.B, self.H, self.hd, self.hd ** -0.5, self.work.data_ptr(), self.work.numel() * 4,
             torch.cuda.current_stream().cuda_stream)
         assert rc == 0, lib.b200enc_last_error()
         return self.out
